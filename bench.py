@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the memento hot path: genes tested/sec for ht_1d_moments (num_boot=10k).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1], "IFN-beta PBMC-shaped"): 25 000 cells x 10 000 genes synthetic
 negative-binomial counts, q = 0.07, stim vs ctrl x 8 cell types = 16 groups, covariate = cell-type
@@ -115,7 +115,35 @@ def parse():
                     help="c2 (default): the headline metric's configuration; the others time the whole API "
                          "pipeline of a larger BASELINE shape, gene-sharded over the ranks (strong scaling)")
     ap.add_argument("--genes-total", type=int, default=0, help="workload runs: genes over ALL ranks (0 = the shape's)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result arrays of the last timed ht_1d_moments call as DIR/<name>.npy (float64)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs records the GPU path's results; --impl reference tests a timing-dependent gene sample")
+    return a
+
+
+DUMP_KEYS = ("mean_coef", "mean_se", "mean_asl", "var_coef", "var_se", "var_asl")
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(directory, mem):
+    """``--dump-outputs``: the six flat result arrays a caller of ht_1d_moments receives (all ranks' genes when
+    gene-sharded), so that two builds can be compared output for output on the same seeded inputs.  Above 64 MB in
+    all, every array keeps the same fixed, seeded sample of test positions, stored as sample_index.npy."""
+    ht = mem.get("1d_ht_all") or mem["1d_ht"]
+    arrays = {k: np.asarray(ht[k], dtype=np.float64) for k in DUMP_KEYS}
+    n = arrays[DUMP_KEYS[0]].size
+    per_test = 8 * (len(arrays) + 1)
+    if n * 8 * len(arrays) > DUMP_LIMIT:
+        keep = np.sort(np.random.default_rng(0).choice(n, size=DUMP_LIMIT // per_test, replace=False))
+        arrays = {k: v[keep] for k, v in arrays.items()}
+        arrays["sample_index"] = keep.astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(directory, k + ".npy"), v)
 
 
 def config_dict(a, n_groups, n_tested, extra=None):
@@ -532,6 +560,8 @@ def run_ours(a):
     launches += _lib.launch_count()
     barrier()
     gc.enable()
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, mem)       # before the end-to-end steps below overwrite the results
     gpu_ht = {k: np.array(v) for k, v in mem["1d_ht"].items() if k.endswith(("_coef", "_se", "_asl"))}
     ms_total = e0.elapsed_time(e1)
     clk = clocks.stop() if clocks else None
@@ -778,6 +808,8 @@ def run_workload(a):
     for i in range(a.steps):
         timed("ht_1d_moments", lambda: memento.ht_1d_moments(ad, cov, tr, seed=100 + i, **kw))
     launches = _lib.launch_count() - l0
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, mem)
     clk = clocks.stop() if clocks else None
     stage_ms = {k: v / a.steps for k, v in st.timer.collect().items()}
     G = ad.shape[1]
