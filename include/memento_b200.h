@@ -28,8 +28,10 @@ int mm_version(void);
 /* Number of kernels this library has launched in the process so far (every launch site is counted): the bench line's
  * "gpu_launches" is the difference of two readings around the timed region. */
 int64_t mm_launch_count(void);
-/* The MM_* tuning / A-B environment variables are read once, when the library is loaded; this re-reads them (tests and
- * tuning scripts only; not safe against calls running on other threads). */
+/* Test hook: MM_MOMENTS_KERNEL = tile | stream | stream_l1 in the environment forces the kernel mm_seg_moments uses on
+ * its streamed path (otherwise chosen from the input), so that tests can run every kernel on every segment structure.
+ * The variable is read once, when the library is loaded; this re-reads it (tests only; not safe against calls running
+ * on other threads). */
 int mm_reload_tuning(void);
 const char* mm_last_error(void);
 
@@ -102,19 +104,6 @@ int mm_relayout_fill(int device, void* stream, const int64_t* indptr, const int3
 int mm_seg_moments(int device, void* stream, const float* vals, const int32_t* rows,
                    const int64_t* seg_ptr, int64_t n_seg, int64_t nnz, const double* inv_sf,
                    int64_t n_cells, double* out, int32_t* big_list, const int32_t* chunk_seg, double* edge);
-
-/* The same five sums by the row-window kernel (csrc/moments.cu): rows [0, n_cells) are cut into n_win windows,
- * win_lo [n_win + 1], none crossing a group boundary (win_group [n_win]; group_win_lo [R + 1] = the windows of every
- * group, consecutive) and none longer than max_window_rows (its 1/size-factor slice lives in shared memory, 8 bytes
- * per row, <= 226 KB).  win_parts [n_win] <= parts_max: CTAs that share the genes of a window.  partial
- * [n_win][n_genes][5] is needed when a group has several windows (n_win > R).  For segments long enough that a warp
- * per (gene, window) piece is efficient; same results as mm_seg_moments up to summation order.
- * Replaces: memento/estimator.py:175-185 per group (main.py:190-194) and over all cells (main.py:62, :86). */
-int mm_seg_moments_windows(int device, void* stream, const float* vals, const int32_t* rows,
-                           const int64_t* seg_ptr, int32_t n_genes, int32_t R, int32_t n_win,
-                           const int32_t* win_lo, const int32_t* win_group, const int32_t* win_parts,
-                           int32_t parts_max, int32_t max_window_rows, const int32_t* group_win_lo,
-                           const double* inv_sf, double* out, double* partial);
 
 /* Dense gene block on the tensor cores, step 1: the fp16 operand panels of one group.  For every listed gene i
  * (gene_idx[i], n_genes of them) and every cell c of group `group` (renumbered rows row0 .. row0 + n_cells - 1),
@@ -192,12 +181,6 @@ int mm_block_cross_batch(int device, void* stream, const float* vals, const int3
                          const int32_t* gene_b, int32_t nb, const double* center_b, const double* inv_scale_b,
                          const double* scale_b, void* panel_a, void* panel_b, int32_t k_cap, int32_t n_bufs,
                          const uint64_t* b_panels, const int32_t* cell_w, double* out, int64_t ldo, int64_t group_stride);
-
-/* Diagnostics of mm_block_gemm (host call, synchronises the device): with MM_BLOCK_DEBUG=9 in the environment the
- * kernel adds up the cycles its roles spend waiting; out8[0..7] = producer on empty ring slots, MMA thread on full
- * slots, MMA thread on drained accumulators, one epilogue warp on finished accumulators, its TMEM loads + float64
- * adds, its stores, whole kernel (per CTA), number of CTAs.  The counters are reset by the call. */
-int mm_block_debug_counters(int device, uint64_t* out8);
 
 /* Covariance sums of gene pairs within every group: for pair k and group r,
  *   out[k*R + r] = sum over cells of the group of x_{c,i} * x_{c,j} / sf_c^2

@@ -1,7 +1,6 @@
 """Moment / ingest kernels timed on the BASELINE shapes (one GPU's gene shard of the large ones):
     python scripts/bench_moments_shapes.py [c2 northstar c5] > profiles/rNN_moments_shapes.json
-Per shape: mm_seg_moments by the size-chosen kernel ("legacy": span / tile kernels) and by the row-window kernel, on
-the grouped matrix and on the all-cells matrix; mm_csr_row_sums; the re-layout (count + fill) -- CUDA-event times over
+Per shape: mm_seg_moments (the size-chosen span / tile kernel) on the grouped matrix and on the all-cells matrix; mm_csr_row_sums; the re-layout (count + fill) -- CUDA-event times over
 10 launches after 3 warm-ups, algorithmic bytes as in DESIGN.md section 4, fraction of the measured HBM peak."""
 import json, os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -53,24 +52,13 @@ for name in (sys.argv[1:] or ["c2", "northstar", "c5"]):
     relayout_bytes = csr.nnz * (4 + 4 + 4 + 4 + 4)
     res["relayout_all_cells"] = entry(timed(lambda: dev_mod.SegMatrix.from_csr_grouped(csr), reps=3), relayout_bytes)
     inv_all = torch.ones(w["cells"], dtype=torch.float64, device="cuda")
-    for kern in ("legacy", "windows"):
-        dev_mod.MOMENTS_KERNEL = kern
-        res["seg_moments_all_cells_" + kern] = entry(timed(lambda: seg_all.moments(inv_all)), seg_all.moments_bytes())
-    dev_mod.MOMENTS_KERNEL = "auto"
+    res["seg_moments_all_cells"] = entry(timed(lambda: seg_all.moments(inv_all)), seg_all.moments_bytes())
     memento.create_groups(ad, w["labels"])
     memento.compute_1d_moments(ad, min_perc_group=0.7, filter_genes=False)
     seg = st.seg
     res["groups"] = seg.R
     res["mean_segment"] = seg.nnz / max(1, seg.n_seg)
-    plan = seg.window_plan()
-    res["windows"] = None if plan is None else {"n_win": plan["n_win"], "max_rows": plan["max_rows"], "parts_max": plan["parts_max"]}
-    for kern in ("legacy", "windows"):
-        dev_mod.MOMENTS_KERNEL = kern
-        if kern == "windows" and plan is None:
-            continue
-        res["seg_moments_grouped_" + kern] = entry(timed(lambda: seg.moments(st.inv_sf_sorted)), seg.moments_bytes())
-    dev_mod.MOMENTS_KERNEL = "auto"
-    res["seg_moments_grouped_auto_uses_windows"] = bool(seg.use_windows())
+    res["seg_moments_grouped"] = entry(timed(lambda: seg.moments(st.inv_sf_sorted)), seg.moments_bytes())
     res["relayout_grouped_ms_from_timer"] = st.timer.collect().get("relayout")
     out["shapes"][name] = res
     del ad, st, seg, seg_all, csr

@@ -28,9 +28,9 @@
 //              128 columns), float64 accumulation over the chunks in registers (the tensor core's fp32
 //              accumulation truncates, see block_gemm_kernel), rescale, transposition of 8-column slices through
 //              2 KB of shared memory per warp, coalesced stores of the float64 block.
-// What bounds it (MM_BLOCK_DEBUG=9 wait counters, scripts/diag_block_waits.py, configs[2] block): not the operand
-// traffic (the 2 x 2 cluster variant with multicast halves is no faster; no reloads at all: 4 % faster), not the
-// MMA count (one product of three: 19 % faster) -- the epilogue warps: per tile 17 k cycles of TMEM loads and
+// What bounds it (per-role wait counters and timing experiments, since removed, on the configs[2] block; see
+// DESIGN.md): not the operand traffic (a 2 x 2 cluster variant with multicast halves was no faster; no reloads at
+// all: 4 % faster), not the MMA count (one product of three: 19 % faster) -- the epilogue warps: per tile 17 k cycles of TMEM loads and
 // float64 adds and 15 k cycles in which all SMs store their 128 KB of float64 results at once, against 21 k cycles
 // of MMAs.  Round 2: 182 -> 119 us per group (8 -> 16 epilogue warps, staged stores instead of 16-byte stores into
 // 32 rows per instruction: 27 k -> 15 k cycles per tile).
@@ -121,14 +121,6 @@ block_panels_kernel(const float* __restrict__ vals, const int* __restrict__ rows
     }
 }
 
-// MM_BLOCK_DEBUG=9: cycles the roles of block_gemm_kernel spend waiting, summed over the CTAs (read and reset with
-// mm_block_debug_counters): [0] producer on empty slots, [1] MMA thread on full slots, [2] MMA thread on drained
-// accumulators, [3] epilogue warp 2 on finished accumulators, [4] its TMEM loads + float64 adds, [5] its stores,
-// [6] whole kernel (thread 0), [7] CTAs
-__device__ unsigned long long g_blk_dbg[8];
-#define MM_DBG_T0(var) long long var = 0; if (debug == 9) var = clock64();
-#define MM_DBG_ADD(slot, var) if (debug == 9) atomicAdd(&g_blk_dbg[slot], (unsigned long long)(clock64() - var));
-
 // ------------------------------------------------------------------ tcgen05 helpers
 __device__ __forceinline__ uint64_t umma_desc(uint32_t smem_addr) {
     // K-major operand tile, 128-byte swizzle: 8-row groups 1024 bytes apart; descriptor version 1 (sm_100)
@@ -153,30 +145,11 @@ __device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, u
         "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
         ::"r"(smem_u32(dst)), "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1) : "memory");
 }
-__device__ __forceinline__ void tma_load_2d_mc(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, uint16_t cta_mask) {
-    // the tile lands at the same shared-memory offset, and signals the barrier at the same offset, in every CTA of cta_mask
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;"
-        ::"r"(smem_u32(dst)), "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(cta_mask) : "memory");
-}
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t cta_mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-                 ::"r"(smem_u32(bar)), "h"(cta_mask) : "memory");
-}
 // TMA store of a shared-memory box into the output tensor (rows / columns outside the tensor are clipped by the unit)
 __device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, const void* src, int c0, int c1) {
     asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
                  ::"l"(map), "r"(smem_u32(src)), "r"(c0), "r"(c1) : "memory");
     asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
 __device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&r)[8]) {
     asm volatile(
@@ -198,20 +171,11 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
 // kChunkBlocks k-blocks (256 cells, error <= ~4e-6 of the chunk); the epilogue warps add the chunks up in
 // float64 registers while the MMA warp already fills the other accumulator pair (TMEM is double buffered:
 // 2 x (128 + 128) columns = all 512).
-//
-// kCl == 2: the launch groups the tiles into 2 x 2 thread-block clusters.  The two CTAs of a cluster row work on the
-// same 128 rows of A, the two of a cluster column on the same 128 rows of B: every CTA fetches HALF of its A tile
-// and half of its B tile (64 rows each, tensor maps with 64-row boxes) and TMA-multicasts them to the peer that
-// needs the same rows, so a k-block costs 32 KB of L2 reads per CTA instead of 64 KB.  A ring slot may be refilled
-// once this CTA AND the two peers its loads write into have read it: the MMA warp's tcgen05.commit arrives on the
-// empty barrier of all three.  Measured on the configs[2] block: no faster than the single-CTA kernel (the operand
-// traffic is not what limits it), so the launch uses it only on request (MM_BLOCK_CLUSTER=2).
-template <int kCl>
 __global__ void __launch_bounds__(kGemmThreads, 1)
 block_gemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_constant__ CUtensorMap map_a_lo,
                   const __grid_constant__ CUtensorMap map_b_hi, const __grid_constant__ CUtensorMap map_b_lo,
                   const __grid_constant__ CUtensorMap map_out, int k_blocks, int M, int N, const double* __restrict__ scale_a, const double* __restrict__ scale_b,
-                  double* __restrict__ out, long long ldo, int vec_ok, int tiles_n, int tiles_m, int debug) {
+                  double* __restrict__ out, long long ldo, int tma_out, int tiles_n, int tiles_m) {
     extern __shared__ unsigned char smem_raw[];
     // 128-byte-swizzled operand tiles need a 1024-byte aligned base (the launch adds 1 KB of slack)
     unsigned char* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -219,19 +183,14 @@ block_gemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_con
     __shared__ uint32_t tmem_base_smem;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int n_chunks = (k_blocks + kChunkBlocks - 1) / kChunkBlocks;
-    // PERSISTENT: the grid is one CTA (kCl == 2: one cluster of four) per SM (group); a CTA walks the units
-    // unit0, unit0 + stride, ...  A unit is one 128 x 128 tile (kCl == 2: a 2 x 2 group of tiles, this CTA's tile is
-    // (2 bx + cx, 2 by + cy)).  The ring-slot and accumulator-buffer counters run on across tiles, so the producer
-    // and the MMA warp are already in the next tile while the epilogue warps scale and store the previous one.
-    constexpr int kCtasPerUnit = kCl == 2 ? 4 : 1;
-    const int units_n = tiles_n / kCl, n_units = units_n * (tiles_m / kCl);
-    const int unit0 = blockIdx.x / kCtasPerUnit, unit_stride = gridDim.x / kCtasPerUnit;
+    // PERSISTENT: the grid is one CTA per SM; a CTA walks the 128 x 128 tiles unit0, unit0 + stride, ...  The
+    // ring-slot and accumulator-buffer counters run on across tiles, so the producer and the MMA warp are already in
+    // the next tile while the epilogue warps scale and store the previous one.
+    const int n_units = tiles_n * tiles_m;
+    const int unit0 = blockIdx.x, unit_stride = gridDim.x;
 
-    uint32_t rank = 0;
-    if constexpr (kCl == 2) rank = cluster_ctarank();       // cx + 2 cy: position inside the 2 x 2 group of tiles
-    const int cx = rank & 1, cy = rank >> 1;
     if (threadIdx.x == 0) {
-        for (int s = 0; s < kGemmStages; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], kCl == 2 ? 3 : 1); }
+        for (int s = 0; s < kGemmStages; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
         for (int b = 0; b < 2; ++b) { mbar_init(&tmem_full[b], 1); mbar_init(&tmem_empty[b], kEpiWarps); }
         mbar_init_fence();
     }
@@ -241,37 +200,23 @@ block_gemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_con
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
-    if constexpr (kCl == 2) cluster_sync_all();             // the peers' barriers exist before anything is sent to them
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t tmem_base = tmem_base_smem;
-    MM_DBG_T0(t_kernel)
 
     if (warp == 0) {
         if (lane == 0) {
             uint32_t it = 0;                                  // k-blocks issued so far, over all tiles
             for (int u = unit0; u < n_units; u += unit_stride) {
-                const int n_blk = (u % units_n) * kCl + cx, m_blk = (u / units_n) * kCl + cy;
+                const int n_blk = u % tiles_n, m_blk = u / tiles_n;
                 for (int kb = 0; kb < k_blocks; ++kb, ++it) {
                     const int s = it % kGemmStages;
-                    MM_DBG_T0(t0)
                     if (it >= kGemmStages) mbar_wait(&empty_bar[s], ((it / kGemmStages) & 1) ^ 1);
-                    MM_DBG_ADD(0, t0)
                     unsigned char* st = smem + (size_t)s * kStageBytes;
-                    if (debug == 2 && it >= kGemmStages) { mbar_arrive(&full_bar[s]); continue; }     // timing experiment: no reloads
-                    mbar_arrive_expect_tx(&full_bar[s], kStageBytes);     // own halves + the peers' halves
-                    if constexpr (kCl == 2) {
-                        constexpr int kHalf = kOperandBytes / 2;           // 64 rows x 128 bytes
-                        const uint16_t mask_a = (uint16_t)(0x3u << (2 * cy)), mask_b = (uint16_t)(0x5u << cx);
-                        tma_load_2d_mc(st + cx * kHalf, &map_a_hi, &full_bar[s], kb * kBK, m_blk * kBM + cx * (kBM / 2), mask_a);
-                        tma_load_2d_mc(st + kOperandBytes + cx * kHalf, &map_a_lo, &full_bar[s], kb * kBK, m_blk * kBM + cx * (kBM / 2), mask_a);
-                        tma_load_2d_mc(st + 2 * kOperandBytes + cy * kHalf, &map_b_hi, &full_bar[s], kb * kBK, n_blk * kBN + cy * (kBN / 2), mask_b);
-                        tma_load_2d_mc(st + 3 * kOperandBytes + cy * kHalf, &map_b_lo, &full_bar[s], kb * kBK, n_blk * kBN + cy * (kBN / 2), mask_b);
-                    } else {
-                        tma_load_2d(st, &map_a_hi, &full_bar[s], kb * kBK, m_blk * kBM);
-                        tma_load_2d(st + kOperandBytes, &map_a_lo, &full_bar[s], kb * kBK, m_blk * kBM);
-                        tma_load_2d(st + 2 * kOperandBytes, &map_b_hi, &full_bar[s], kb * kBK, n_blk * kBN);
-                        tma_load_2d(st + 3 * kOperandBytes, &map_b_lo, &full_bar[s], kb * kBK, n_blk * kBN);
-                    }
+                    mbar_arrive_expect_tx(&full_bar[s], kStageBytes);
+                    tma_load_2d(st, &map_a_hi, &full_bar[s], kb * kBK, m_blk * kBM);
+                    tma_load_2d(st + kOperandBytes, &map_a_lo, &full_bar[s], kb * kBK, m_blk * kBM);
+                    tma_load_2d(st + 2 * kOperandBytes, &map_b_hi, &full_bar[s], kb * kBK, n_blk * kBN);
+                    tma_load_2d(st + 3 * kOperandBytes, &map_b_lo, &full_bar[s], kb * kBK, n_blk * kBN);
                 }
             }
         }
@@ -283,17 +228,13 @@ block_gemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_con
             for (int u = unit0; u < n_units; u += unit_stride) {
                 for (int c = 0; c < n_chunks; ++c, ++ch) {
                     const int buf = ch & 1;
-                    MM_DBG_T0(t2)
                     if (ch >= 2) mbar_wait(&tmem_empty[buf], ((ch >> 1) & 1) ^ 1);    // the epilogue has drained this pair
-                    MM_DBG_ADD(2, t2)
                     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                     const uint32_t acc0 = tmem_base + buf * (2 * kBN), acc1 = acc0 + kBN;
                     const int kb_end = min(k_blocks, (c + 1) * kChunkBlocks);
                     for (int kb = c * kChunkBlocks; kb < kb_end; ++kb, ++it) {
                         const int s = it % kGemmStages;
-                        MM_DBG_T0(t1)
                         mbar_wait(&full_bar[s], (it / kGemmStages) & 1);
-                        MM_DBG_ADD(1, t1)
                         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                         const uint32_t base = smem_u32(smem + (size_t)s * kStageBytes);
 #pragma unroll
@@ -303,13 +244,10 @@ block_gemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_con
                             const uint64_t b_hi = umma_desc(base + 2 * kOperandBytes + koff), b_lo = umma_desc(base + 3 * kOperandBytes + koff);
                             const uint32_t acc = (kb > c * kChunkBlocks || k > 0) ? 1u : 0u;
                             umma_f16(acc0, a_hi, b_hi, idesc, acc);               // acc0 (+)= hi hi
-                            if (debug == 1) continue;                             // timing experiment: one product only
                             umma_f16(acc1, a_hi, b_lo, idesc, acc);               // acc1 (+)= hi lo
                             umma_f16(acc1, a_lo, b_hi, idesc, 1u);                // acc1 += lo hi
                         }
-                        // the ring slot is free once these MMAs have read it (cluster: tell the peers that write into it too)
-                        if constexpr (kCl == 2) umma_commit_mc(&empty_bar[s], (uint16_t)((1u << rank) | (1u << (rank ^ 1)) | (1u << (rank ^ 2))));
-                        else umma_commit(&empty_bar[s]);
+                        umma_commit(&empty_bar[s]);            // the ring slot is free once these MMAs have read it
                     }
                     umma_commit(&tmem_full[buf]);          // this accumulator pair is complete
                 }
@@ -321,17 +259,14 @@ block_gemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_con
         const int q = warp & 3, part = (warp - 2) >> 2;        // lane quarter (fixed by the warp id) and column part
         uint32_t ch = 0;                                      // chunks drained so far, over all tiles
         for (int u = unit0; u < n_units; u += unit_stride) {
-            const int n_blk = (u % units_n) * kCl + cx, m_blk = (u / units_n) * kCl + cy;
+            const int n_blk = u % tiles_n, m_blk = u / tiles_n;
             const int m = m_blk * kBM + q * 32 + lane;
             double acc[kEpiCols];
 #pragma unroll
             for (int j = 0; j < kEpiCols; ++j) acc[j] = 0.0;
             for (int c = 0; c < n_chunks; ++c, ++ch) {
                 const int buf = ch & 1;
-                MM_DBG_T0(t3)
                 mbar_wait(&tmem_full[buf], (ch >> 1) & 1);
-                if (warp == 2 && lane == 0) { MM_DBG_ADD(3, t3) }
-                MM_DBG_T0(t4)
                 asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                 const uint32_t trow = tmem_base + ((uint32_t)(q * 32) << 16) + buf * (2 * kBN) + part * kEpiCols;
 #pragma unroll
@@ -340,7 +275,6 @@ block_gemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_con
                     tmem_ld8(trow + c0, r0);
                     tmem_ld8(trow + kBN + c0, r1);
                     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-                    if (debug == 3) continue;                 // timing experiment: loads only
 #pragma unroll
                     for (int j = 0; j < 8; ++j)      // hi hi + 2^-11 (hi lo + lo hi) in fp32 (24 bits are enough for one chunk), then float64
                         acc[c0 + j] += (double)fmaf(__uint_as_float(r1[j]), (float)(1.0 / kLoScale), __uint_as_float(r0[j]));
@@ -348,9 +282,7 @@ block_gemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_con
                 asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&tmem_empty[buf]);
-                if (warp == 2 && lane == 0) { MM_DBG_ADD(4, t4) }
             }
-            MM_DBG_T0(t5)
             // ---- scale and store.  A thread holds 32 columns of ONE row, so storing from the registers writes 16 bytes
             // into 32 different rows per instruction (measured: 27 k cycles per tile, 44 % of the kernel).  Instead
             // the warp transposes 8-column slices through its own 2 KB of shared memory (16-byte chunks XOR-swizzled
@@ -363,9 +295,9 @@ block_gemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_con
                 const int m_base = m_blk * kBM + q * 32;
 #pragma unroll
                 for (int c0 = 0; c0 < kEpiCols; c0 += 8) {
-                    // vec_ok == 2: the slice leaves through the TMA unit (one bulk tensor store per slice; the staging
+                    // tma_out: the slice leaves through the TMA unit (one bulk tensor store per slice; the staging
                     // layout is the unit's 64-byte swizzle): wait until the previous store has READ the buffer
-                    if (vec_ok == 2) {
+                    if (tma_out) {
                         if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
                         __syncwarp();
                     }
@@ -376,7 +308,7 @@ block_gemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_con
                         const double v1 = n + 1 < N ? acc[c0 + 2 * k + 1] * sa * __ldg(scale_b + n + 1) : 0.0;
                         *reinterpret_cast<double2*>(stage + lane * 64 + ((k ^ ((lane >> 1) & 3)) << 4)) = make_double2(v0, v1);
                     }
-                    if (vec_ok == 2) {
+                    if (tma_out) {
                         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
                         __syncwarp();
                         if (lane == 0) tma_store_2d(&map_out, stage, n_base + c0, m_base);
@@ -390,24 +322,18 @@ block_gemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_con
                         const int mm_ = m_base + row, n = n_base + c0 + 2 * k;
                         if (mm_ < M) {
                             double* dst = out + (long long)mm_ * ldo + n;
-                            if (vec_ok && n + 1 < N) *reinterpret_cast<double2*>(dst) = v;
-                            else {
-                                if (n < N) dst[0] = v.x;
-                                if (n + 1 < N) dst[1] = v.y;
-                            }
+                            if (n < N) dst[0] = v.x;
+                            if (n + 1 < N) dst[1] = v.y;
                         }
                     }
                     __syncwarp();
                 }
             }
-            if (warp == 2 && lane == 0) { MM_DBG_ADD(5, t5) }
         }
-        if (vec_ok == 2 && lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+        if (tma_out && lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
-    if (threadIdx.x == 0) { MM_DBG_ADD(6, t_kernel) if (debug == 9) atomicAdd(&g_blk_dbg[7], 1ull); }
-    if constexpr (kCl == 2) cluster_sync_all();             // nobody leaves while a peer's commit may still arrive here
     if (warp == 1) {
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTmemCols) : "memory");
@@ -428,12 +354,12 @@ static PFN_cuTensorMapEncodeTiled_v12000 encode_fn() {
 }
 
 // fp16 matrix [rows][k_pad], k contiguous; box = 64 x 128 with the 128-byte swizzle
-static int make_map(CUtensorMap* map, const void* ptr, int rows, int k_pad, int box_rows) {
+static int make_map(CUtensorMap* map, const void* ptr, int rows, int k_pad) {
     auto fn = encode_fn();
     if (!fn) { set_error("cuTensorMapEncodeTiled is not available from the driver"); return 2; }
     cuuint64_t dims[2] = {(cuuint64_t)k_pad, (cuuint64_t)rows};
     cuuint64_t strides[1] = {(cuuint64_t)k_pad * 2};
-    cuuint32_t box[2] = {(cuuint32_t)kBK, (cuuint32_t)box_rows};
+    cuuint32_t box[2] = {(cuuint32_t)kBK, (cuuint32_t)kBM};
     cuuint32_t estr[2] = {1, 1};
     CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(ptr), dims, strides, box, estr,
                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
@@ -476,16 +402,6 @@ MM_EXPORT int mm_block_panels(int device, void* stream, const float* vals, const
     return check_launch("mm_block_panels");
 }
 
-MM_EXPORT int mm_block_debug_counters(int device, uint64_t* out8) {
-    if (int s = enter(device)) return s;
-    MM_REQUIRE(out8, "null pointer");
-    MM_CUDA(cudaDeviceSynchronize());
-    MM_CUDA(cudaMemcpyFromSymbol(out8, g_blk_dbg, sizeof(unsigned long long) * 8));
-    unsigned long long zero[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    MM_CUDA(cudaMemcpyToSymbol(g_blk_dbg, zero, sizeof(zero)));
-    return 0;
-}
-
 static int block_gemm_launch(int device, cudaStream_t stream, const void* a_hi, const void* a_lo, int32_t m, const void* b_hi,
                              const void* b_lo, int32_t n, int32_t k_pad, const double* scale_a, const double* scale_b,
                              double* out, int64_t ldo) {
@@ -494,25 +410,19 @@ static int block_gemm_launch(int device, cudaStream_t stream, const void* a_hi, 
     MM_REQUIRE(a_hi && a_lo && b_hi && b_lo && scale_a && scale_b && out, "null pointer");
     MM_REQUIRE((((uintptr_t)a_hi | (uintptr_t)a_lo | (uintptr_t)b_hi | (uintptr_t)b_lo) & 15) == 0,
                "operand panels must be 16-byte aligned");
-    // 0: scalar stores; 1: 128-bit stores (16-byte aligned rows); 2: TMA tensor stores (the same alignment is what the
-    // tensor map needs; MM_BLOCK_DEBUG=4 keeps the 128-bit stores for A/B)
-    int vec_ok = (((uintptr_t)out & 15) == 0 && (ldo & 1) == 0) ? 1 : 0;
+    // TMA tensor stores where the rows are 16-byte aligned (what the tensor map needs), scalar stores otherwise
+    const int tma_out = (((uintptr_t)out & 15) == 0 && (ldo & 1) == 0) ? 1 : 0;
     CUtensorMap m_out;
     memset(&m_out, 0, sizeof(m_out));
-    if (vec_ok && tuning().block_debug != 4) {
+    if (tma_out) {
         if (int s = make_out_map(&m_out, out, m, n, ldo)) return s;
-        vec_ok = 2;
     }
-    // MM_BLOCK_CLUSTER=2: 2 x 2 clusters with multicast operand halves (needs at least two tiles each way); default:
-    // the single-CTA persistent kernel, which measured faster
     const int tiles_n = (n + kBN - 1) / kBN, tiles_m = (m + kBM - 1) / kBM;
-    const bool clustered = tuning().block_cluster == 2 && tiles_n >= 2 && tiles_m >= 2;
-    const int box_rows = clustered ? kBM / 2 : kBM;
     CUtensorMap ma_hi, ma_lo, mb_hi, mb_lo;
-    if (int s = make_map(&ma_hi, a_hi, m, k_pad, box_rows)) return s;
-    if (int s = make_map(&ma_lo, a_lo, m, k_pad, box_rows)) return s;
-    if (int s = make_map(&mb_hi, b_hi, n, k_pad, box_rows)) return s;
-    if (int s = make_map(&mb_lo, b_lo, n, k_pad, box_rows)) return s;
+    if (int s = make_map(&ma_hi, a_hi, m, k_pad)) return s;
+    if (int s = make_map(&ma_lo, a_lo, m, k_pad)) return s;
+    if (int s = make_map(&mb_hi, b_hi, n, k_pad)) return s;
+    if (int s = make_map(&mb_lo, b_lo, n, k_pad)) return s;
     // operand ring + the epilogue warps' store staging + slack for the 1024-byte alignment
     const size_t smem = (size_t)kGemmStages * kStageBytes + (size_t)kEpiWarps * kStoreStageBytes + 1024;
     static int n_sm_cached[64] = {0};
@@ -521,35 +431,10 @@ static int block_gemm_launch(int device, cudaStream_t stream, const void* a_hi, 
         if (cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, device) != cudaSuccess || n_sm <= 0) n_sm = 148;
         if (device >= 0 && device < 64) n_sm_cached[device] = n_sm;
     }
-    const int debug = tuning().block_debug;
-    if (clustered) {
-        const int tn = (tiles_n + 1) / 2 * 2, tm = (tiles_m + 1) / 2 * 2;      // whole 2 x 2 groups (padding tiles store nothing)
-        const int n_units = (tn / 2) * (tm / 2);
-        MM_CUDA(cudaFuncSetAttribute(block_gemm_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        cudaLaunchConfig_t cfg = {};
-        cfg.blockDim = dim3(kGemmThreads);
-        cfg.dynamicSmemBytes = smem;
-        cfg.stream = stream;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = 4; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = 1;
-        cfg.gridDim = dim3(4);
-        int max_clusters = 0;
-        if (cudaOccupancyMaxActiveClusters(&max_clusters, block_gemm_kernel<2>, &cfg) != cudaSuccess || max_clusters <= 0) {
-            cudaGetLastError();
-            max_clusters = n_sm / 4;
-        }
-        cfg.gridDim = dim3((unsigned)(4 * (n_units < max_clusters ? n_units : max_clusters)));
-        MM_CUDA(cudaLaunchKernelEx(&cfg, block_gemm_kernel<2>, ma_hi, ma_lo, mb_hi, mb_lo, m_out, (int)(k_pad / kBK), (int)m, (int)n,
-                                   scale_a, scale_b, out, (long long)ldo, vec_ok, tn, tm, debug));
-    } else {
-        MM_CUDA(cudaFuncSetAttribute(block_gemm_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        const int n_units = tiles_n * tiles_m;
-        block_gemm_kernel<1><<<(unsigned)(n_units < n_sm ? n_units : n_sm), kGemmThreads, smem, stream>>>(
-            ma_hi, ma_lo, mb_hi, mb_lo, m_out, k_pad / kBK, m, n, scale_a, scale_b, out, ldo, vec_ok, tiles_n, tiles_m, debug);
-    }
+    MM_CUDA(cudaFuncSetAttribute(block_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const int n_units = tiles_n * tiles_m;
+    block_gemm_kernel<<<(unsigned)(n_units < n_sm ? n_units : n_sm), kGemmThreads, smem, stream>>>(
+        ma_hi, ma_lo, mb_hi, mb_lo, m_out, k_pad / kBK, m, n, scale_a, scale_b, out, ldo, tma_out, tiles_n, tiles_m);
     return check_launch("mm_block_gemm");
 }
 

@@ -205,7 +205,6 @@ struct PrepParams {
     uint32_t* acc_pool;          // [n_genes_tile * acc_stride]
     SegInfo* info;               // [n_seg]
     float min_accept;            // fall back to the chain / direct resampling below this expected acceptance rate
-    int allow_direct;            // 0: chain only
 };
 
 // One warp per segment: choose the remainder category, decide the sampler, rewrite the entries'
@@ -279,7 +278,7 @@ boot_prepare_kernel(PrepParams P) {
     if (exp(-best) < (double)P.min_accept) {
         // flat, dense gene: if its nonzero cells fit the direct kernel's shared-memory table and the table is not
         // much shorter than the group (chain ~ 90 U instructions per replicate, direct ~ 14 N), resample cells
-        if (P.allow_direct && mass <= kDirectMaxCells && (long long)N <= 6LL * U) { si.mode = 2; si.s_lo = (int)mass; }
+        if (mass <= kDirectMaxCells && (long long)N <= 6LL * U) { si.mode = 2; si.s_lo = (int)mass; }
         publish();
         return;
     }
@@ -416,13 +415,12 @@ bootstrap_1d_kernel(BootParams P) {
     for (int i = blockIdx.y; i < n_list; i += gridDim.y) chain_segment(P, lists.chain[i], b);
 }
 
-// One finished replicate: kFast && log_rows writes log(mean) and log(residual variance) straight into the regression's
-// rows (table-driven log, no division, log rv = log var - trend(log mean)); otherwise the library-math path.
-template <bool kFast>
+// One finished replicate: with log_rows, log(mean) and log(residual variance) go straight into the regression's rows
+// (table-driven log, no division, log rv = log var - trend(log mean)); otherwise the library-math path.
 __device__ __forceinline__ void emit_replicate(const BootParams& P, long long seg_rel, int b, double m1, double m2,
                                                int N, double inv_n, const double* __restrict__ fit,
                                                const double2* s_log) {
-    if (kFast && P.log_rows) {
+    if (P.log_rows) {
         double mean, var;
         if (P.estimator == 0) { mean = m1 * inv_n; var = m2 * inv_n - mean * mean; }
         else { mean = m1 * inv_n + 1.0; var = 10.0; }
@@ -449,29 +447,24 @@ __device__ __forceinline__ void emit_replicate(const BootParams& P, long long se
 // ---------------------------------------------------------------- Poissonised sampler
 // Block = kBootThreads lanes, each looping over its own replicates of one segment (see header).
 //
-// kFast (default) trims the three non-essential costs of the loop, measured in the SASS of the plain variant
-// (107 instructions per 4 draws, 40 of them Philox; ~490 per replicate outside the loop):
-//   * Philox4x32-7 instead of -10 (see Philox::rounds): 28 instead of 40 instructions per 4 draws;
-//   * count -> float64 by the 2^52 trick (one DADD on the FP64 pipe instead of I2F.F64 on the quarter-rate XU pipe);
-//   * log rows written directly: log(mean) and log(var) by the table-driven log_pos (no fp64 division, no
-//     exp / log round trip for the residual variance: log rv = log var - poly(log mean)).
-// The plain variant is kept for A/B measurements (MM_BOOT_PLAIN=1) and for raw (non-log) output rows.
-__device__ __forceinline__ double count_to_double(int k) {        // k >= 0
-    return __hiloint2double(0x43300000, k) - 4503599627370496.0;
-}
-
-// kSlots > 1: every lane runs kSlots replicates in lockstep over the same categories, so the warp-uniform 32-byte
-// category record is loaded once per kSlots draws.  ncu on the one-slot kernel: L1 data-pipe wavefronts are its most
-// loaded unit (67 %), and 8 of the 10 wavefronts of a draw are the record (32 lanes x 32 B written back to registers,
+// Against a plain loop (Philox4x32-10, library log / exp for the log rows: 107 instructions per 4 draws, 40 of them
+// Philox; ~490 per replicate outside the loop) this kernel uses Philox4x32-7 (see Philox::rounds: 28 instead of 40
+// instructions per 4 draws) and writes log(mean) and log(var) by the table-driven log_pos (no fp64 division, no
+// exp / log round trip for the residual variance: log rv = log var - poly(log mean)).
+//
+// Every lane runs kBootSlots replicates in lockstep over the same categories, so the warp-uniform 32-byte category
+// record is loaded once per kBootSlots draws.  ncu on a one-slot kernel: L1 data-pipe wavefronts are its most loaded
+// unit (67 %), and 8 of the 10 wavefronts of a draw are the record (32 lanes x 32 B written back to registers,
 // uniform address or not) -- two slots cut that to 6 per draw and amortise the record unpacking and loop overhead
 // (25 -> 19 instructions per draw).  A pass over one segment has the same length for every replicate, so slots never
 // wait for each other: an accepted slot claims the next replicate, a rejected one repeats its own.  The random numbers
-// of a replicate depend on (seed, replicate, segment, attempt) only, so every kSlots gives bit-identical rows.
-template <int kVariant, int kSlots>      // kVariant 0: plain, 1: Philox-7 + direct log rows, 2: 1 + 2^52 conversion
-__global__ void __launch_bounds__(kBootThreads, kVariant ? (kSlots == 1 ? 8 : kSlots == 2 ? 6 : kSlots == 3 ? 5 : 4) : 0)
+// of a replicate depend on (seed, replicate, segment, attempt) only, so neither the slot count nor the replicates per
+// block change the rows.
+constexpr int kBootSlots = 2;
+
+__global__ void __launch_bounds__(kBootThreads, 6)
 bootstrap_1d_poisson_kernel(BootParams P) {
-    constexpr bool kFast = kVariant > 0;
-    constexpr int kR = kFast ? 7 : 10;
+    constexpr int kR = 7;
     // block rows are dispatched in order: with seg_order = segments by decreasing table length the long blocks (a
     // dense gene's block runs 10 x the average) start first instead of leaving a tail of a few busy SMs
     const long long seg_rel = P.seg_order ? P.seg_order[blockIdx.y] : blockIdx.y;
@@ -488,31 +481,31 @@ bootstrap_1d_poisson_kernel(BootParams P) {
     const double* fit = P.mv_fit + 3 * r;
     const int b_end = min(P.B, (int)(blockIdx.x + 1) * P.reps_per_block);
     __shared__ int s_next;
-    __shared__ double2 s_log[kFast ? 128 : 1];
+    __shared__ double2 s_log[128];
     static_assert(kBootThreads >= 128, "one log-table entry per thread");
-    if (kFast && threadIdx.x < 128) log_tab_fill(s_log, threadIdx.x);
-    if (threadIdx.x == 0) s_next = blockIdx.x * P.reps_per_block + kSlots * kBootThreads;
+    if (threadIdx.x < 128) log_tab_fill(s_log, threadIdx.x);
+    if (threadIdx.x == 0) s_next = blockIdx.x * P.reps_per_block + kBootSlots * kBootThreads;
     __syncthreads();
     const double inv_n = 1.0 / (double)N;
     // Philox counter = (replicate, segment lo, block number, segment hi ^ tag); the block number runs on over the
     // attempts of one replicate and restarts with a new replicate
     const uint32_t key0 = (uint32_t)P.seed, key1 = (uint32_t)(P.seed >> 32);
     const uint32_t c1 = (uint32_t)sid, c3 = (uint32_t)(sid >> 32) ^ 0x9015u;
-    int b[kSlots];
-    uint32_t blk[kSlots];
+    int b[kBootSlots];
+    uint32_t blk[kBootSlots];
 #pragma unroll
-    for (int j = 0; j < kSlots; ++j) { b[j] = blockIdx.x * P.reps_per_block + j * kBootThreads + threadIdx.x; blk[j] = 0; }
+    for (int j = 0; j < kBootSlots; ++j) { b[j] = blockIdx.x * P.reps_per_block + j * kBootThreads + threadIdx.x; blk[j] = 0; }
     auto live = [&]() {
         bool any = false;
 #pragma unroll
-        for (int j = 0; j < kSlots; ++j) any |= b[j] < b_end;
+        for (int j = 0; j < kBootSlots; ++j) any |= b[j] < b_end;
         return any;
     };
     while (live()) {
-        int S[kSlots];
-        double M1[kSlots], M2[kSlots];
+        int S[kBootSlots];
+        double M1[kBootSlots], M2[kBootSlots];
 #pragma unroll
-        for (int j = 0; j < kSlots; ++j) { S[j] = 0; M1[j] = 0.0; M2[j] = 0.0; }
+        for (int j = 0; j < kBootSlots; ++j) { S[j] = 0; M1[j] = 0.0; M2[j] = 0.0; }
         auto fresh4 = [&](int j) {
             return Philox::rounds<kR>(make_uint4((uint32_t)b[j], c1, blk[j]++, c3), key0, key1);
         };
@@ -520,7 +513,7 @@ bootstrap_1d_poisson_kernel(BootParams P) {
         auto draw = [&](int j, const int4& lo4, const int4& hi4, uint32_t rnd) {
             const int k = alias_draw(P.tab_pool, (unsigned)hi4.x, (unsigned)hi4.y, hi4.w, rnd);
             S[j] += k;
-            const double kd = kVariant == 2 ? count_to_double(k) : (double)k;
+            const double kd = (double)k;
             M1[j] = fma(__hiloint2double(lo4.y, lo4.x), kd, M1[j]);
             M2[j] = fma(__hiloint2double(lo4.w, lo4.z), kd, M2[j]);
         };
@@ -533,38 +526,38 @@ bootstrap_1d_poisson_kernel(BootParams P) {
                 hi4[c] = __ldg(reinterpret_cast<const int4*>(tab + u + c) + 1);
             }
 #pragma unroll
-            for (int j = 0; j < kSlots; ++j) {
+            for (int j = 0; j < kBootSlots; ++j) {
                 const uint4 r4 = fresh4(j);
                 draw(j, lo4[0], hi4[0], r4.x); draw(j, lo4[1], hi4[1], r4.y);
                 draw(j, lo4[2], hi4[2], r4.z); draw(j, lo4[3], hi4[3], r4.w);
             }
         }
-        uint4 r4[kSlots];
+        uint4 r4[kBootSlots];
 #pragma unroll
-        for (int j = 0; j < kSlots; ++j) r4[j] = fresh4(j);
+        for (int j = 0; j < kBootSlots; ++j) r4[j] = fresh4(j);
         if (u < U) {
             const int4 lo4 = __ldg(reinterpret_cast<const int4*>(tab + u)), hi4 = __ldg(reinterpret_cast<const int4*>(tab + u) + 1);
 #pragma unroll
-            for (int j = 0; j < kSlots; ++j) draw(j, lo4, hi4, r4[j].x);
+            for (int j = 0; j < kBootSlots; ++j) draw(j, lo4, hi4, r4[j].x);
         }
         if (u + 1 < U) {
             const int4 lo4 = __ldg(reinterpret_cast<const int4*>(tab + u + 1)), hi4 = __ldg(reinterpret_cast<const int4*>(tab + u + 1) + 1);
 #pragma unroll
-            for (int j = 0; j < kSlots; ++j) draw(j, lo4, hi4, r4[j].y);
+            for (int j = 0; j < kBootSlots; ++j) draw(j, lo4, hi4, r4[j].y);
         }
         if (u + 2 < U) {
             const int4 lo4 = __ldg(reinterpret_cast<const int4*>(tab + u + 2)), hi4 = __ldg(reinterpret_cast<const int4*>(tab + u + 2) + 1);
 #pragma unroll
-            for (int j = 0; j < kSlots; ++j) draw(j, lo4, hi4, r4[j].z);
+            for (int j = 0; j < kBootSlots; ++j) draw(j, lo4, hi4, r4[j].z);
         }
         if (si.zero_off >= 0) {
 #pragma unroll
-            for (int j = 0; j < kSlots; ++j)
+            for (int j = 0; j < kBootSlots; ++j)
                 S[j] += alias_draw(P.tab_pool, (unsigned)si.zero_off, (unsigned)(si.zero_kl & 0xFFFF),
                                    (si.zero_kl >> 16) - si.zero_off, r4[j].w);
         }
 #pragma unroll
-        for (int j = 0; j < kSlots; ++j) {
+        for (int j = 0; j < kBootSlots; ++j) {
             const uint4 ra = fresh4(j);
             const int i = S[j] - si.s_lo;
             bool ok = (i >= 0) && (i < si.acc_len) && (b[j] < b_end);
@@ -572,7 +565,7 @@ bootstrap_1d_poisson_kernel(BootParams P) {
             if (ok) {
                 const double w = (double)(N - S[j]);            // the remainder category takes the rest
                 const double m1 = fma(si.rem_a, w, M1[j]), m2 = fma(si.rem_b, w, M2[j]);
-                emit_replicate<kFast>(P, seg_rel, b[j], m1, m2, N, inv_n, fit, s_log);
+                emit_replicate(P, seg_rel, b[j], m1, m2, N, inv_n, fit, s_log);
                 b[j] = atomicAdd(&s_next, 1);                // results depend on (seed, replicate) only, not on the lane
                 blk[j] = 0;
             }
@@ -648,7 +641,7 @@ bootstrap_1d_direct_kernel(BootParams P) {
                 if (i + 1 < N) draw(r4.y, M1b, M2b);
                 if (i + 2 < N) draw(r4.z, M1, M2);
             }
-            emit_replicate<true>(P, seg_rel, b, M1 + M1b, M2 + M2b, N, inv_n, fit, s_log);
+            emit_replicate(P, seg_rel, b, M1 + M1b, M2 + M2b, N, inv_n, fit, s_log);
         }
     }
 }
@@ -742,7 +735,6 @@ MM_EXPORT int mm_boot_prepare(int device, void* stream, void* entries, const int
     P.R = R; P.seg_U = seg_U; P.group_ncells = group_ncells; P.n_table_max = n_table_max; P.tab_off = tab_off;
     P.acc_slot = (const long long*)acc_slot; P.acc_stride = acc_stride; P.acc_pool = acc_pool;
     P.info = (SegInfo*)seg_info; P.min_accept = min_accept;
-    P.allow_direct = tuning().boot_direct != 0;      // A/B hook
     long long blocks = (n_seg + 7) / 8;
     MM_REQUIRE(blocks < 2147483647LL, "too many segments");
     MM_CUDA(cudaMemsetAsync(seg_lists(seg_info, n_seg).count, 0, 4 * sizeof(int), (cudaStream_t)stream));
@@ -771,19 +763,14 @@ MM_EXPORT int mm_bootstrap_1d(int device, void* stream, const void* entries, con
     P.log_rows = log_rows; P.n_invalid = n_invalid; P.seg_order = seg_order;
     MM_REQUIRE(!log_rows || n_invalid, "log_rows needs the n_invalid counters (zero-initialised)");
     P.info = (const SegInfo*)seg_info; P.tab_pool = (const uint2*)tab_pool; P.acc_pool = acc_pool;
-    const Tuning& tune = tuning();
-    const int variant = tune.boot_variant >= 0 ? tune.boot_variant : 1;     // A/B hooks
-    const int slots = tune.boot_slots >= 0 ? tune.boot_slots : 2;
-    const int n_slots = (variant == 0 || slots <= 1) ? 1 : (slots >= 4 ? 4 : slots);
     // replicates per block: lanes claim replicates from the block's counter, so only the block's last pass has idle
     // lanes -- one block per segment when there are enough segments to fill the GPU (C2: 40 passes 165 ms, 20 passes
     // 173 ms, 10 passes 189 ms), more blocks per segment otherwise
     const long long want_blocks = (148 * 6 * 2 + n_seg - 1) / n_seg;
-    int passes = (int)((num_boot + (long long)kBootThreads * n_slots * want_blocks - 1) / ((long long)kBootThreads * n_slots * want_blocks));
+    int passes = (int)((num_boot + (long long)kBootThreads * kBootSlots * want_blocks - 1) / ((long long)kBootThreads * kBootSlots * want_blocks));
     if (passes > 40) passes = 40;
-    if (tune.boot_passes >= 0) passes = tune.boot_passes;      // A/B hook
     if (passes < 1) passes = 1;
-    P.reps_per_block = kBootThreads * passes * n_slots;
+    P.reps_per_block = kBootThreads * passes * kBootSlots;
     MM_REQUIRE(!seg_info || (tab_pool && acc_pool), "seg_info needs tab_pool and acc_pool");
     // with a sampler choice the chain kernel walks the chain list (modes 0 / -1: usually a handful of segments)
     dim3 grid((num_boot + kBootThreads - 1) / kBootThreads, (unsigned)(seg_info ? (n_seg < 512 ? n_seg : 512) : n_seg));
@@ -792,13 +779,7 @@ MM_EXPORT int mm_bootstrap_1d(int device, void* stream, const void* entries, con
     if (seg_info) {
         dim3 grid2((num_boot + P.reps_per_block - 1) / P.reps_per_block, (unsigned)n_seg);
         cudaStream_t st = (cudaStream_t)stream;
-        if (variant == 0) bootstrap_1d_poisson_kernel<0, 1><<<grid2, kBootThreads, 0, st>>>(P);
-        else if (variant == 2 && n_slots == 1) bootstrap_1d_poisson_kernel<2, 1><<<grid2, kBootThreads, 0, st>>>(P);
-        else if (variant == 2 && n_slots == 2) bootstrap_1d_poisson_kernel<2, 2><<<grid2, kBootThreads, 0, st>>>(P);
-        else if (n_slots == 1) bootstrap_1d_poisson_kernel<1, 1><<<grid2, kBootThreads, 0, st>>>(P);
-        else if (n_slots == 3) bootstrap_1d_poisson_kernel<1, 3><<<grid2, kBootThreads, 0, st>>>(P);
-        else if (n_slots == 4) bootstrap_1d_poisson_kernel<1, 4><<<grid2, kBootThreads, 0, st>>>(P);
-        else bootstrap_1d_poisson_kernel<1, 2><<<grid2, kBootThreads, 0, st>>>(P);
+        bootstrap_1d_poisson_kernel<<<grid2, kBootThreads, 0, st>>>(P);
         if (int s = check_launch("mm_bootstrap_1d (Poissonised)")) return s;
         // dense segments boot_prepare marked for direct cell resampling (blocks of other segments exit at once)
         const size_t smem = (size_t)kDirectMaxCells * sizeof(double2);

@@ -16,26 +16,11 @@ void set_error(const char* fmt, ...);
 int check_launch(const char* what);      // cudaGetLastError -> status
 int enter(int device);                   // cudaSetDevice + clear error; returns status
 
-// A/B and tuning switches (MM_* environment variables), read ONCE per process at the first C-ABI call -- never on
-// the per-call path.  -1 / 0 = "not set" (the built-in choice applies).
+// Test hook, read ONCE per process when the library is loaded (and again by mm_reload_tuning) -- never on the
+// per-call path.  MM_MOMENTS_KERNEL = tile | stream | stream_l1 forces one of the three kernels mm_seg_moments
+// otherwise picks from the input, so that tests can run every kernel on every segment structure.
 struct Tuning {
-    int moments_notile;     // MM_MOMENTS_NOTILE: set -> generic W-lane kernels
-    int moments_kernel;     // MM_MOMENTS_KERNEL: 0 auto, 1 tile, 2 stream, 3 stream_l1
-    int moments_threads;    // MM_MOMENTS_THREADS (stream kernel): 512 / 640 / 768 / 896
-    int moments_prefetch;   // MM_MOMENTS_PREFETCH: -1 unset
-    int moments_chunk;      // MM_MOMENTS_CHUNK: spans per chunk, 1 / 4 / 8
-    int block_cluster;      // MM_BLOCK_CLUSTER (dense-block GEMM): 2 = 2 x 2 clusters with multicast operand halves (default: single-CTA kernel)
-    int block_debug;        // MM_BLOCK_DEBUG (timing experiments, wrong results): 1 = one MMA of three, 2 = no TMA reloads, 3 = no float64 accumulation
-    int relayout_scan_threads;   // MM_RELAYOUT_SCAN_THREADS (row scan of the tiled re-layout): 256 / 512 / 1024
-    int relayout_cfg;       // MM_RELAYOUT_CFG (tiled fill pass): -1 unset, 0..4 tile shapes
-    int moments_cfg;        // MM_MOMENTS_CFG (tile kernel): -1 unset
-    int moments_regime;     // MM_MOMENTS_REGIME
-    int moments_w;          // MM_MOMENTS_W: lanes per segment of the generic kernel
-    int boot_direct;        // MM_BOOT_DIRECT: -1 unset, 0 = no direct sampler
-    int boot_variant;       // MM_BOOT_VARIANT: -1 unset
-    int boot_slots;         // MM_BOOT_SLOTS: -1 unset
-    int boot_passes;        // MM_BOOT_PASSES: -1 unset
-    int pair_slots;         // MM_PAIR_SLOTS: -1 unset
+    int moments_kernel;     // 0 auto, 1 tile, 2 stream, 3 stream_l1
 };
 const Tuning& tuning();
 

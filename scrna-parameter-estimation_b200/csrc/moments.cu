@@ -415,12 +415,14 @@ __device__ __forceinline__ void consume_pieces(MomStage& st, int n, long long t_
     }
 }
 
-template <int kStages, int kMinBlocks>
-__global__ void __launch_bounds__(kTileThreads, kMinBlocks)
+constexpr int kStages = 2;             // tiles in flight per CTA
+constexpr int kTileBlocksPerSm = 3;
+
+__global__ void __launch_bounds__(kTileThreads, kTileBlocksPerSm)
 seg_moments_tile_kernel(const float* __restrict__ vals, const int* __restrict__ rows,
                         const long long* __restrict__ seg_ptr, long long n_seg, long long nnz,
                         const int* __restrict__ chunk_seg, const double* __restrict__ inv_sf,
-                        double* __restrict__ out, double* __restrict__ edge, int regime) {
+                        double* __restrict__ out, double* __restrict__ edge) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     MomStage* stages = reinterpret_cast<MomStage*>(smem_raw);
     __shared__ uint64_t full_bar[kStages], empty_bar[kStages];
@@ -464,7 +466,7 @@ seg_moments_tile_kernel(const float* __restrict__ vals, const int* __restrict__ 
             }
             __syncwarp();
             int n_long = 0;
-            if (npieces > kSpanMaxPieces || regime != 0) {       // the span regime does not use the list
+            if (npieces > kSpanMaxPieces) {       // the span regime does not use the list
                 for (int k0 = 0; k0 < nb - 1; k0 += 32) {
                     const int k = k0 + lane;
                     bool lg = false;
@@ -505,7 +507,7 @@ seg_moments_tile_kernel(const float* __restrict__ vals, const int* __restrict__ 
         const long long np_ll = s1 - s0 + 1;
         const int npieces = np_ll > 2147483647LL ? 2147483647 : (int)np_ll;
         mbar_wait(&full_bar[s], (it / kStages) & 1);
-        if (npieces <= kSpanMaxPieces && regime == 0)
+        if (npieces <= kSpanMaxPieces)
             consume_spans(st, n, s0, npieces, tile, n_seg, inv_sf, out, edge, warp, lane);
         else if ((long long)n >= (long long)kLaneMaxLen * npieces)
             consume_pieces<8, 4>(st, n, t_lo, s0, npieces, tile, n_seg, it, seg_ptr, inv_sf, out, edge, warp, lane);
@@ -548,7 +550,11 @@ __device__ __forceinline__ double warp_sum4(double sx, double s1, double s2, dou
     return keep;      // lanes 0-7: sum sx, 8-15: sum s1, 16-23: sum s2, 24-31: sum s3
 }
 
-template <bool kSmemTable, int kStreamThreads, bool kPrefetch, int kC, int kQ>
+constexpr int kStreamThreads = 640;
+constexpr int kC = 4;                  // spans per chunk
+constexpr int kQ = 4;                  // quad rows (of 128 nonzeros) per span
+
+template <bool kSmemTable>
 __global__ void __launch_bounds__(kStreamThreads, 1)
 seg_moments_stream_kernel(const float* __restrict__ vals, const int* __restrict__ rows,
                           const long long* __restrict__ seg_ptr, long long n_seg, long long nnz,
@@ -646,7 +652,7 @@ seg_moments_stream_kernel(const float* __restrict__ vals, const int* __restrict_
         if (sp_lo >= n) break;
         // ---- the next span (of this chunk, or the first of the warp's next chunk) goes to L2 now (one 128-byte
         // line per lane and array): a register-free second buffer, so that its loads are L2 hits
-        if (kPrefetch && (sp_lo & 1023) == 0) {              // one prefetch covers 32 lanes x 32 elements = 1024 nonzeros
+        if ((sp_lo & 1023) == 0) {              // one prefetch covers 32 lanes x 32 elements = 1024 nonzeros
             const long long p_lo = (sp_lo + 1024 < kChunkElems ? t_lo + sp_lo + 1024 : (span + warps_total) * kChunkElems) + 32 * lane;
             if (p_lo + 32 <= nnz) { prefetch_l2(vals + p_lo); prefetch_l2(rows + p_lo); }
         }
@@ -810,118 +816,6 @@ pair_products_kernel(const float* __restrict__ vals, const int* __restrict__ row
     if (lane == 0) out[item] = acc;
 }
 
-// ------------------------------------------------------------------ row-window kernel
-// The group-sorted layout gives every segment (gene, group) a CONTIGUOUS range of row ids -- the group's cells.  A CTA
-// that only ever touches segments of one group therefore needs just that group's slice of the 1/size-factor table,
-// and the slice fits shared memory where the whole table does not (1 M cells: 8 MB table, 25 k cells per group).
-// Rows are cut into windows that never cross a group boundary (a group larger than the shared-memory budget is cut
-// into several; rows ascend inside a segment, so a window's share of a segment is a contiguous piece found by a
-// binary search).  grid = (parts, windows): the CTAs of a window split the genes; a warp reduces one piece with
-// 128-bit streaming loads, no boundary bookkeeping and no edge pass.  Pieces of a multi-window group go to
-// `partial` and are combined in window order (deterministic).
-struct WinParams {
-    const float* vals; const int* rows; const long long* seg_ptr;
-    int n_genes, R, n_win;
-    const int* win_lo;          // [n_win + 1] first row of every window (windows tile [0, n_cells))
-    const int* win_group;       // [n_win]
-    const int* win_parts;       // [n_win] CTAs working on the window (<= gridDim.x)
-    const int* group_win_lo;    // [R + 1] windows of every group
-    const double* inv_sf;
-    double* out;                // [5][n_genes * R]
-    double* partial;            // [n_win][n_genes][5] (only read / written for groups with several windows)
-};
-
-__device__ __forceinline__ long long lower_bound_row(const int* __restrict__ rows, long long lo, long long hi, int key) {
-    while (lo < hi) {
-        const long long mid = (lo + hi) >> 1;
-        if (__ldg(rows + mid) < key) lo = mid + 1; else hi = mid;
-    }
-    return lo;
-}
-
-template <int kThreads>
-__global__ void __launch_bounds__(kThreads)
-seg_moments_window_kernel(WinParams P) {
-    extern __shared__ __align__(16) double s_tab[];
-    const int w = blockIdx.y;
-    const int parts = P.win_parts[w];
-    if ((int)blockIdx.x >= parts) return;
-    const int row_lo = P.win_lo[w], row_hi = P.win_lo[w + 1];
-    const int r = P.win_group[w];
-    const bool whole = P.group_win_lo[r + 1] - P.group_win_lo[r] == 1;      // the window is the group
-    for (int i = threadIdx.x; i < row_hi - row_lo; i += kThreads) s_tab[i] = P.inv_sf[row_lo + i];
-    __syncthreads();
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int g_lo = (int)((long long)P.n_genes * blockIdx.x / parts);
-    const int g_hi = (int)((long long)P.n_genes * (blockIdx.x + 1) / parts);
-    const long long n_seg = (long long)P.n_genes * P.R;
-    const float4* __restrict__ v4 = reinterpret_cast<const float4*>(P.vals);
-    const int4* __restrict__ r4 = reinterpret_cast<const int4*>(P.rows);
-    const double* tab = s_tab - row_lo;
-    for (int g = g_lo + warp; g < g_hi; g += kThreads / 32) {
-        const long long seg = (long long)g * P.R + r;
-        long long a = __ldg(P.seg_ptr + seg), b = __ldg(P.seg_ptr + seg + 1);
-        if (!whole) {
-            const long long a0 = a;
-            a = lower_bound_row(P.rows, a0, b, row_lo);
-            b = lower_bound_row(P.rows, a, b, row_hi);
-        }
-        Mom m;
-        long long a4 = (a + 3) & ~3LL;
-        if (a4 > b) a4 = b;
-        if (lane < a4 - a) m.add(ld_stream(P.vals + a + lane), tab[ld_stream(P.rows + a + lane)]);
-        const long long b4 = (b & ~3LL) > a4 ? (b & ~3LL) : a4;
-        long long q = a4 / 4 + lane;
-        const long long qe = b4 / 4;
-        auto quad = [&](const float4& v, const int4& rr) {
-            m.add(v.x, tab[rr.x]); m.add(v.y, tab[rr.y]); m.add(v.z, tab[rr.z]); m.add(v.w, tab[rr.w]);
-        };
-        for (; q + 96 < qe; q += 128) {         // four quads per lane in flight
-            const float4 va = ld_stream4(v4 + q), vb = ld_stream4(v4 + q + 32), vc = ld_stream4(v4 + q + 64), vd = ld_stream4(v4 + q + 96);
-            const int4 ra = ld_stream4(r4 + q), rb = ld_stream4(r4 + q + 32), rc = ld_stream4(r4 + q + 64), rd = ld_stream4(r4 + q + 96);
-            quad(va, ra); quad(vb, rb); quad(vc, rc); quad(vd, rd);
-        }
-        {   // up to four more, issued together
-            float4 vv[4];
-            int4 rr[4];
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                if (q + 32 * u < qe) { vv[u] = ld_stream4(v4 + q + 32 * u); rr[u] = ld_stream4(r4 + q + 32 * u); }
-            }
-#pragma unroll
-            for (int u = 0; u < 4; ++u) if (q + 32 * u < qe) quad(vv[u], rr[u]);
-        }
-        if (lane < b - b4) m.add(ld_stream(P.vals + b4 + lane), tab[ld_stream(P.rows + b4 + lane)]);
-        const double red = warp_sum4(m.sx, m.s1, m.s2, m.s3, lane);       // lanes 0 / 8 / 16 / 24 hold sx / s1 / s2 / s3
-        const float mx = warp_max(m.mx);
-        if (whole) {
-            if ((lane & 7) == 0) P.out[(long long)(lane == 0 ? 0 : lane == 8 ? 2 : lane == 16 ? 3 : 4) * n_seg + seg] = red;
-            if (lane == 1) P.out[n_seg + seg] = (double)mx;
-        } else {
-            double* pp = P.partial + ((long long)w * P.n_genes + g) * 5;
-            if ((lane & 7) == 0) pp[lane == 0 ? 0 : lane == 8 ? 2 : lane == 16 ? 3 : 4] = red;
-            if (lane == 1) pp[1] = (double)mx;
-        }
-    }
-}
-
-// groups cut into several windows: add their pieces up in window order
-__global__ void seg_moments_window_combine_kernel(WinParams P) {
-    const long long n_seg = (long long)P.n_genes * P.R;
-    const long long seg = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (seg >= n_seg) return;
-    const int g = (int)(seg / P.R), r = (int)(seg % P.R);
-    const int w0 = P.group_win_lo[r], w1 = P.group_win_lo[r + 1];
-    if (w1 - w0 == 1) return;
-    double acc[5] = {0, 0, 0, 0, 0};
-    for (int w = w0; w < w1; ++w) {
-        const double* pp = P.partial + ((long long)w * P.n_genes + g) * 5;
-        acc[0] += pp[0]; acc[1] = fmax(acc[1], pp[1]); acc[2] += pp[2]; acc[3] += pp[3]; acc[4] += pp[4];
-    }
-#pragma unroll
-    for (int k = 0; k < 5; ++k) P.out[(long long)k * n_seg + seg] = acc[k];
-}
-
 // ------------------------------------------------------------------ host-side error state
 static thread_local char g_err[512] = "";
 void set_error(const char* fmt, ...) {
@@ -952,30 +846,10 @@ int enter(int device) {
 const char* last_error() { return g_err; }
 long long launch_count() { return g_launches.load(std::memory_order_relaxed); }
 
-static int env_int(const char* name, int unset) {
-    const char* v = getenv(name);
-    return v ? atoi(v) : unset;
-}
 static Tuning read_tuning() {
     Tuning u;
-    u.moments_notile = getenv("MM_MOMENTS_NOTILE") ? 1 : 0;
     const char* k = getenv("MM_MOMENTS_KERNEL");
     u.moments_kernel = !k ? 0 : !strcmp(k, "tile") ? 1 : !strcmp(k, "stream") ? 2 : !strcmp(k, "stream_l1") ? 3 : 0;
-    u.moments_threads = env_int("MM_MOMENTS_THREADS", 0);
-    u.moments_prefetch = env_int("MM_MOMENTS_PREFETCH", -1);
-    u.moments_chunk = env_int("MM_MOMENTS_CHUNK", 0);
-    u.relayout_cfg = env_int("MM_RELAYOUT_CFG", -1);
-    u.relayout_scan_threads = env_int("MM_RELAYOUT_SCAN_THREADS", 0);
-    u.block_cluster = env_int("MM_BLOCK_CLUSTER", -1);
-    u.block_debug = env_int("MM_BLOCK_DEBUG", 0);
-    u.moments_cfg = env_int("MM_MOMENTS_CFG", -1);
-    u.moments_regime = env_int("MM_MOMENTS_REGIME", 0);
-    u.moments_w = env_int("MM_MOMENTS_W", 0);
-    u.boot_direct = env_int("MM_BOOT_DIRECT", -1);
-    u.boot_variant = env_int("MM_BOOT_VARIANT", -1);
-    u.boot_slots = env_int("MM_BOOT_SLOTS", -1);
-    u.boot_passes = env_int("MM_BOOT_PASSES", -1);
-    u.pair_slots = env_int("MM_PAIR_SLOTS", -1);
     return u;
 }
 static Tuning g_tuning = read_tuning();      // once, when the library is loaded
@@ -987,7 +861,7 @@ void reload_tuning() { g_tuning = read_tuning(); }
 using namespace mm;
 
 MM_EXPORT const char* mm_last_error(void) { return mm::last_error(); }
-MM_EXPORT int mm_version(void) { return 101; }
+MM_EXPORT int mm_version(void) { return 102; }
 namespace mm { long long launch_count(); void reload_tuning(); }
 MM_EXPORT int mm_reload_tuning(void) { mm::reload_tuning(); return 0; }
 MM_EXPORT int64_t mm_launch_count(void) { return (int64_t)mm::launch_count(); }
@@ -1033,22 +907,20 @@ static int launch_edge(cudaStream_t st, long long n_chunks, const long long* sp,
     return check_launch("seg_moments_edge");
 }
 
-template <int S, int kBlocksPerSm>
-static int launch_tile(cudaStream_t st, int n_sm, int regime, const float* vals, const int32_t* rows,
+static int launch_tile(cudaStream_t st, int n_sm, const float* vals, const int32_t* rows,
                        const long long* sp, long long n_seg, long long nnz, const int32_t* chunk_seg,
                        const double* inv_sf, double* out, double* edge) {
-    const size_t smem = sizeof(MomStage) * S;
-    MM_CUDA(cudaFuncSetAttribute(seg_moments_tile_kernel<S, kBlocksPerSm>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const size_t smem = sizeof(MomStage) * kStages;
+    MM_CUDA(cudaFuncSetAttribute(seg_moments_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const long long n_tiles = (nnz + kTile - 1) / kTile;
-    long long grid = (long long)n_sm * kBlocksPerSm;
+    long long grid = (long long)n_sm * kTileBlocksPerSm;
     if (grid > n_tiles) grid = n_tiles;
-    seg_moments_tile_kernel<S, kBlocksPerSm><<<(unsigned)grid, kTileThreads, smem, st>>>(vals, rows, sp, n_seg, nnz, chunk_seg,
-                                                                                       inv_sf, out, edge, regime);
+    seg_moments_tile_kernel<<<(unsigned)grid, kTileThreads, smem, st>>>(vals, rows, sp, n_seg, nnz, chunk_seg,
+                                                                      inv_sf, out, edge);
     if (int s = check_launch("seg_moments_tile")) return s;
     return launch_edge<kTile>(st, n_tiles, sp, n_seg, nnz, chunk_seg, edge, out);
 }
 
-template <int kThreads, bool kPrefetch, int kC, int kQ>
 static int launch_stream(cudaStream_t st, int n_sm, const float* vals, const int32_t* rows, const long long* sp,
                          long long n_seg, long long nnz, const int32_t* chunk_seg, const double* inv_sf,
                          long long n_cells, double* out, double* edge, bool smem_table) {
@@ -1056,55 +928,19 @@ static int launch_stream(cudaStream_t st, int n_sm, const float* vals, const int
     static_assert(kChunk % kSpanElems == 0, "chunks must be whole multiples of the chunk_seg granularity");
     const long long n_spans = (nnz + kChunk - 1) / kChunk;      // chunks of kC spans
     long long grid = n_sm;
-    const long long need = (n_spans + kThreads / 32 - 1) / (kThreads / 32);
+    const long long need = (n_spans + kStreamThreads / 32 - 1) / (kStreamThreads / 32);
     if (grid > need) grid = need;
     if (smem_table) {
         const size_t smem = (size_t)n_cells * sizeof(double);
-        MM_CUDA(cudaFuncSetAttribute(seg_moments_stream_kernel<true, kThreads, kPrefetch, kC, kQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        seg_moments_stream_kernel<true, kThreads, kPrefetch, kC, kQ><<<(unsigned)grid, kThreads, smem, st>>>(vals, rows, sp, n_seg, nnz, chunk_seg,
-                                                                                        inv_sf, (int)n_cells, out, edge);
+        MM_CUDA(cudaFuncSetAttribute(seg_moments_stream_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        seg_moments_stream_kernel<true><<<(unsigned)grid, kStreamThreads, smem, st>>>(vals, rows, sp, n_seg, nnz, chunk_seg,
+                                                                                inv_sf, (int)n_cells, out, edge);
     } else {
-        seg_moments_stream_kernel<false, kThreads, kPrefetch, kC, kQ><<<(unsigned)grid, kThreads, 0, st>>>(vals, rows, sp, n_seg, nnz, chunk_seg,
-                                                                                      inv_sf, (int)n_cells, out, edge);
+        seg_moments_stream_kernel<false><<<(unsigned)grid, kStreamThreads, 0, st>>>(vals, rows, sp, n_seg, nnz, chunk_seg,
+                                                                              inv_sf, (int)n_cells, out, edge);
     }
     if (int s = check_launch("seg_moments_stream")) return s;
     return launch_edge<kChunk>(st, n_spans, sp, n_seg, nnz, chunk_seg, edge, out);
-}
-
-MM_EXPORT int mm_seg_moments_windows(int device, void* stream, const float* vals, const int32_t* rows,
-                                     const int64_t* seg_ptr, int32_t n_genes, int32_t R, int32_t n_win,
-                                     const int32_t* win_lo, const int32_t* win_group, const int32_t* win_parts,
-                                     int32_t parts_max, int32_t max_window_rows, const int32_t* group_win_lo,
-                                     const double* inv_sf, double* out, double* partial) {
-    if (int s = enter(device)) return s;
-    MM_REQUIRE(n_genes >= 0 && R > 0 && n_win >= R && parts_max > 0 && parts_max <= 65535 * 16, "n_genes/R/n_win/parts_max");
-    MM_REQUIRE(n_win <= 65535, "at most 65535 row windows");
-    if (n_genes == 0) return 0;
-    MM_REQUIRE(vals && rows && seg_ptr && win_lo && win_group && win_parts && group_win_lo && inv_sf && out, "null pointer");
-    MM_REQUIRE(n_win == R || partial, "groups cut into several windows need the partial buffer");
-    MM_REQUIRE((((uintptr_t)vals | (uintptr_t)rows) & 15) == 0, "vals / rows must be 16-byte aligned");
-    const size_t smem = (size_t)max_window_rows * sizeof(double);
-    MM_REQUIRE(max_window_rows > 0 && smem <= 226 * 1024, "window too large for shared memory");
-    WinParams P;
-    P.vals = vals; P.rows = rows; P.seg_ptr = (const long long*)seg_ptr; P.n_genes = n_genes; P.R = R; P.n_win = n_win;
-    P.win_lo = win_lo; P.win_group = win_group; P.win_parts = win_parts; P.group_win_lo = group_win_lo;
-    P.inv_sf = inv_sf; P.out = out; P.partial = partial;
-    cudaStream_t st = (cudaStream_t)stream;
-    const dim3 grid((unsigned)parts_max, (unsigned)n_win);
-    if (smem > 100 * 1024) {        // one CTA per SM: as many warps as a CTA can have
-        MM_CUDA(cudaFuncSetAttribute(seg_moments_window_kernel<768>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        seg_moments_window_kernel<768><<<grid, 768, smem, st>>>(P);
-    } else {
-        MM_CUDA(cudaFuncSetAttribute(seg_moments_window_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        seg_moments_window_kernel<512><<<grid, 512, smem, st>>>(P);
-    }
-    if (int s = check_launch("seg_moments_window")) return s;
-    if (n_win > R) {
-        const long long n_seg = (long long)n_genes * R;
-        seg_moments_window_combine_kernel<<<(unsigned)((n_seg + 255) / 256), 256, 0, st>>>(P);
-        return check_launch("seg_moments_window_combine");
-    }
-    return 0;
 }
 
 MM_EXPORT int mm_seg_moments(int device, void* stream, const float* vals, const int32_t* rows,
@@ -1124,40 +960,19 @@ MM_EXPORT int mm_seg_moments(int device, void* stream, const float* vals, const 
     const long long* sp = (const long long*)seg_ptr;
     const long long mean_len = nnz / n_seg;
     const bool aligned = (((uintptr_t)vals | (uintptr_t)rows | (uintptr_t)inv_sf) & 15) == 0;
-    const Tuning& tune = tuning();
-    if (chunk_seg && edge && aligned && n_seg < 2147483647LL && !tune.moments_notile) {
+    if (chunk_seg && edge && aligned && n_seg < 2147483647LL) {
         const int n_sm = sm_count(device);
-        // Tuning hooks: MM_MOMENTS_KERNEL = stream | stream_l1 | tile overrides the choice below;
-        // MM_MOMENTS_CFG (tile kernel) 0 = 3 stages x 2 CTAs/SM, 1 = 2 stages x 3 CTAs/SM, 2 = 4 stages x 1 CTA/SM.
         bool use_stream = mean_len >= kStreamMinMean;
         bool smem_table = n_cells > 0 && n_cells * 8 <= 227 * 1024 - 1024;
-        if (tune.moments_kernel == 1) use_stream = false;
-        else if (tune.moments_kernel == 2) use_stream = true;
-        else if (tune.moments_kernel == 3) { use_stream = true; smem_table = false; }
-        if (use_stream) {
-            int threads = 640;
-            bool pf = true;
-            if (tune.moments_threads) threads = tune.moments_threads;      // tuning hooks
-            if (tune.moments_prefetch >= 0) pf = tune.moments_prefetch != 0;
-            const int chunk_spans = (tune.moments_chunk == 1 || tune.moments_chunk == 8) ? tune.moments_chunk : 4;   // 8: 256-nonzero spans
-#define MM_STREAM(T, PF) (chunk_spans == 1 ? launch_stream<T, PF, 1, 4>(st, n_sm, vals, rows, sp, n_seg, nnz, chunk_seg, inv_sf, n_cells, out, edge, smem_table) \
-                        : chunk_spans == 8 ? launch_stream<T, PF, 8, 2>(st, n_sm, vals, rows, sp, n_seg, nnz, chunk_seg, inv_sf, n_cells, out, edge, smem_table) \
-                                           : launch_stream<T, PF, 4, 4>(st, n_sm, vals, rows, sp, n_seg, nnz, chunk_seg, inv_sf, n_cells, out, edge, smem_table))
-            if (threads == 896) return pf ? MM_STREAM(896, true) : MM_STREAM(896, false);
-            if (threads == 768) return pf ? MM_STREAM(768, true) : MM_STREAM(768, false);
-            if (threads == 512) return pf ? MM_STREAM(512, true) : MM_STREAM(512, false);
-            return pf ? MM_STREAM(640, true) : MM_STREAM(640, false);
-#undef MM_STREAM
-        }
-        int cfg = 1, regime = 0;
-        if (tune.moments_cfg >= 0) cfg = tune.moments_cfg;
-        regime = tune.moments_regime;
-        if (cfg == 0) return launch_tile<3, 2>(st, n_sm, regime, vals, rows, sp, n_seg, nnz, chunk_seg, inv_sf, out, edge);
-        if (cfg == 2) return launch_tile<4, 1>(st, n_sm, regime, vals, rows, sp, n_seg, nnz, chunk_seg, inv_sf, out, edge);
-        return launch_tile<2, 3>(st, n_sm, regime, vals, rows, sp, n_seg, nnz, chunk_seg, inv_sf, out, edge);
+        const int forced = tuning().moments_kernel;      // test hook MM_MOMENTS_KERNEL (common.cuh)
+        if (forced == 1) use_stream = false;
+        else if (forced == 2) use_stream = true;
+        else if (forced == 3) { use_stream = true; smem_table = false; }
+        if (use_stream)
+            return launch_stream(st, n_sm, vals, rows, sp, n_seg, nnz, chunk_seg, inv_sf, n_cells, out, edge, smem_table);
+        return launch_tile(st, n_sm, vals, rows, sp, n_seg, nnz, chunk_seg, inv_sf, out, edge);
     }
-    int W = mean_len < 48 ? 8 : (mean_len < 1024 ? 16 : 32);
-    if (tune.moments_w == 8 || tune.moments_w == 16 || tune.moments_w == 32) W = tune.moments_w;   // tuning hook
+    const int W = mean_len < 48 ? 8 : (mean_len < 1024 ? 16 : 32);
     // Without the tile index (or with unaligned arrays): W lanes per segment straight from global memory;
     // segments far above the mean are deferred to the CTA kernel through big_list.
     MM_REQUIRE(big_list, "null pointer (big_list)");

@@ -318,10 +318,12 @@ struct PairBootParams {
     const int* item_order;      // [n_items] nullable: item handled by block row y (longest tables first)
 };
 
-// kSlots replicates per lane run in lockstep over the same categories (see bootstrap_1d_poisson_kernel): the
-// warp-uniform 64-byte category record is loaded once per kSlots draws.  Philox4x32-7; the random numbers of a
-// replicate depend on (seed, replicate, item, attempt) only, so every kSlots gives bit-identical rows.
-template <int kSlots>
+// kPairSlots replicates per lane run in lockstep over the same categories (see bootstrap_1d_poisson_kernel): the
+// warp-uniform 64-byte category record is loaded once per kPairSlots draws.  Philox4x32-7; the random numbers of a
+// replicate depend on (seed, replicate, item, attempt) only, so neither the slot count nor the replicates per block
+// change the rows.
+constexpr int kPairSlots = 2;
+
 __global__ void __launch_bounds__(kPairThreads)
 pair_bootstrap_kernel(PairBootParams P) {
     constexpr int kR = 7;
@@ -350,25 +352,25 @@ pair_bootstrap_kernel(PairBootParams P) {
     const uint32_t* acc = P.acc_pool + pi.acc_off;
     const long long sid = P.item_id ? P.item_id[item] : item;
     __shared__ int s_next;
-    if (threadIdx.x == 0) s_next = b_lo + kSlots * kPairThreads;
+    if (threadIdx.x == 0) s_next = b_lo + kPairSlots * kPairThreads;
     __syncthreads();
     const uint32_t key0 = (uint32_t)P.seed, key1 = (uint32_t)(P.seed >> 32);
     const uint32_t c1 = (uint32_t)sid, c3 = (uint32_t)(sid >> 32) ^ 0x2D2Du;
-    int b[kSlots];
-    uint32_t blk[kSlots];
+    int b[kPairSlots];
+    uint32_t blk[kPairSlots];
 #pragma unroll
-    for (int j = 0; j < kSlots; ++j) { b[j] = b_lo + j * kPairThreads + threadIdx.x; blk[j] = 0; }
+    for (int j = 0; j < kPairSlots; ++j) { b[j] = b_lo + j * kPairThreads + threadIdx.x; blk[j] = 0; }
     auto live = [&]() {
         bool any = false;
 #pragma unroll
-        for (int j = 0; j < kSlots; ++j) any |= b[j] < b_end;
+        for (int j = 0; j < kPairSlots; ++j) any |= b[j] < b_end;
         return any;
     };
     while (live()) {
-        int S[kSlots];
-        double acc5[kSlots][5];
+        int S[kPairSlots];
+        double acc5[kPairSlots][5];
 #pragma unroll
-        for (int j = 0; j < kSlots; ++j) {
+        for (int j = 0; j < kPairSlots; ++j) {
             S[j] = 0;
 #pragma unroll
             for (int c = 0; c < 5; ++c) acc5[j][c] = 0.0;
@@ -384,57 +386,57 @@ pair_bootstrap_kernel(PairBootParams P) {
             acc5[j][2] = fma(e.cx, kd, acc5[j][2]); acc5[j][3] = fma(e.v1, kd, acc5[j][3]);
             acc5[j][4] = fma(e.v2, kd, acc5[j][4]);
         };
-        uint4 r4[kSlots];
+        uint4 r4[kPairSlots];
         int u = 0;
         for (; u + 4 <= pi.U; u += 4) {     // four categories per Philox block and slot; one record live at a time
 #pragma unroll
-            for (int j = 0; j < kSlots; ++j) r4[j] = fresh4(j);
+            for (int j = 0; j < kPairSlots; ++j) r4[j] = fresh4(j);
             {
                 const PairEntry e = tab[u];
 #pragma unroll
-                for (int j = 0; j < kSlots; ++j) draw(j, e, r4[j].x);
+                for (int j = 0; j < kPairSlots; ++j) draw(j, e, r4[j].x);
             }
             {
                 const PairEntry e = tab[u + 1];
 #pragma unroll
-                for (int j = 0; j < kSlots; ++j) draw(j, e, r4[j].y);
+                for (int j = 0; j < kPairSlots; ++j) draw(j, e, r4[j].y);
             }
             {
                 const PairEntry e = tab[u + 2];
 #pragma unroll
-                for (int j = 0; j < kSlots; ++j) draw(j, e, r4[j].z);
+                for (int j = 0; j < kPairSlots; ++j) draw(j, e, r4[j].z);
             }
             {
                 const PairEntry e = tab[u + 3];
 #pragma unroll
-                for (int j = 0; j < kSlots; ++j) draw(j, e, r4[j].w);
+                for (int j = 0; j < kPairSlots; ++j) draw(j, e, r4[j].w);
             }
         }
 #pragma unroll
-        for (int j = 0; j < kSlots; ++j) r4[j] = fresh4(j);
+        for (int j = 0; j < kPairSlots; ++j) r4[j] = fresh4(j);
         if (u < pi.U) {
             const PairEntry e = tab[u];
 #pragma unroll
-            for (int j = 0; j < kSlots; ++j) draw(j, e, r4[j].x);
+            for (int j = 0; j < kPairSlots; ++j) draw(j, e, r4[j].x);
         }
         if (u + 1 < pi.U) {
             const PairEntry e = tab[u + 1];
 #pragma unroll
-            for (int j = 0; j < kSlots; ++j) draw(j, e, r4[j].y);
+            for (int j = 0; j < kPairSlots; ++j) draw(j, e, r4[j].y);
         }
         if (u + 2 < pi.U) {
             const PairEntry e = tab[u + 2];
 #pragma unroll
-            for (int j = 0; j < kSlots; ++j) draw(j, e, r4[j].z);
+            for (int j = 0; j < kPairSlots; ++j) draw(j, e, r4[j].z);
         }
         if (pi.zero_off >= 0) {
 #pragma unroll
-            for (int j = 0; j < kSlots; ++j)
+            for (int j = 0; j < kPairSlots; ++j)
                 S[j] += alias_draw(P.tab_pool, (unsigned)pi.zero_off, (unsigned)(pi.zero_kl & 0xFFFF),
                                    (pi.zero_kl >> 16) - pi.zero_off, r4[j].w);
         }
 #pragma unroll
-        for (int j = 0; j < kSlots; ++j) {
+        for (int j = 0; j < kPairSlots; ++j) {
             const uint4 ra = fresh4(j);
             const int i = S[j] - pi.s_lo;
             bool ok = (i >= 0) && (i < pi.acc_len) && (b[j] < b_end);
@@ -547,20 +549,14 @@ MM_EXPORT int mm_pair_bootstrap(int device, void* stream, const void* entries, c
     P.entries = (const PairEntry*)entries; P.item_ptr = (const long long*)item_ptr; P.n_items = n_items; P.R = R;
     P.info = (const PairInfo*)info; P.group_ncells = group_ncells; P.true_corr = true_corr;
     P.tab_pool = (const uint2*)tab_pool; P.acc_pool = acc_pool; P.B = num_boot; P.seed = seed;
-    const Tuning& tune = tuning();
-    const int slots = tune.pair_slots >= 0 ? tune.pair_slots : 2;      // A/B hook
-    const int n_slots = slots <= 1 ? 1 : (slots >= 3 ? 3 : 2);
     const long long want_blocks = (148 * 4 * 2 + n_items - 1) / n_items;     // see mm_bootstrap_1d
-    int passes = (int)((num_boot + (long long)kPairThreads * n_slots * want_blocks - 1) / ((long long)kPairThreads * n_slots * want_blocks));
+    int passes = (int)((num_boot + (long long)kPairThreads * kPairSlots * want_blocks - 1) / ((long long)kPairThreads * kPairSlots * want_blocks));
     if (passes > 40) passes = 40;
-    if (tune.boot_passes >= 0) passes = tune.boot_passes;      // A/B hook
     if (passes < 1) passes = 1;
-    P.item_id = (const long long*)item_id; P.reps_per_block = kPairThreads * passes * n_slots;
+    P.item_id = (const long long*)item_id; P.reps_per_block = kPairThreads * passes * kPairSlots;
     P.boot_corr = boot_corr; P.item_good = item_good; P.item_order = item_order;
     dim3 grid((num_boot + P.reps_per_block - 1) / P.reps_per_block, (unsigned)n_items);
-    if (n_slots == 1) pair_bootstrap_kernel<1><<<grid, kPairThreads, 0, (cudaStream_t)stream>>>(P);
-    else if (n_slots == 3) pair_bootstrap_kernel<3><<<grid, kPairThreads, 0, (cudaStream_t)stream>>>(P);
-    else pair_bootstrap_kernel<2><<<grid, kPairThreads, 0, (cudaStream_t)stream>>>(P);
+    pair_bootstrap_kernel<<<grid, kPairThreads, 0, (cudaStream_t)stream>>>(P);
     return check_launch("mm_pair_bootstrap");
 }
 

@@ -29,8 +29,8 @@
 //       rank of an element inside its gene's run = popcount of the lower rows' bits -- so the tile's nonzeros are
 //       placed in a staging buffer sorted by (gene, row) with no ordering constraint between warps, and go out as one
 //       coalesced run per gene (chunk rows x density elements: ~240 B on the 25k x 10k matrix).
-// Bit-identical to the generic path and to the stable sort (tests/test_gpu_relayout.py).  Measured (scripts/
-// ab_relayout.py, B200): 25k x 10k, 61 M nonzeros: 0.20 + 0.55 ms (round 2's thread-per-row tiles: 0.24 + 1.34 ms);
+// Bit-identical to the generic path and to the stable sort (tests/test_gpu_relayout.py).  Measured (B200,
+// profiles/r02_relayout_tiles.json): 25k x 10k, 61 M nonzeros: 0.20 + 0.55 ms (round 2's thread-per-row tiles: 0.24 + 1.34 ms);
 // 1 M x 2500, 599 M nonzeros: 2.3 + 4.5 ms (was 14.1 ms).
 #include "common.cuh"
 #include <cooperative_groups.h>
@@ -117,13 +117,26 @@ relayout_fill_kernel(RelayoutParams P, const long long* __restrict__ seg_ptr, fl
 constexpr int kTileRows = 256;       // rows per chunk (bit-matrix height); chunks may be shorter
 constexpr int kScanLoads = 8;        // pass A: 32-index loads in flight per warp
 constexpr int kMaxTiledGenes = 100000;   // pass A keeps 16-bit counters of all genes in shared memory (<= 200 KB)
+// Warps per CTA of pass A: a warp walks its rows one after the other (order -> indptr -> row loads is a chain of
+// dependent loads per row), so more warps = fewer rows per warp; measured on C2 with 256 / 512 / 1024 threads:
+// 0.20 / 0.21 / 0.26 ms.
+constexpr int kScanThreads = 256;
+// Pass C's tile shape: genes per block / staged nonzeros per pass / threads / CTAs per SM (measured against 128-gene
+// tiles and other staging sizes: 256-gene tiles, two 512-thread CTAs per SM).  Pass A writes the block starts at
+// the same granularity (kTileShift).
+constexpr int kTileGenes = 256;
+constexpr int kTileShift = 8;
+static_assert((1 << kTileShift) == kTileGenes, "pass A's block shift is pass C's tile width");
+constexpr int kStageCap = 16384;
+constexpr int kFillThreads = 512;
+constexpr int kFillBlocksPerSm = 2;
 
 // grid = n_chunks x S CTAs, a thread-block CLUSTER of S CTAs per chunk (S = 1, 2, 4 or 8: a matrix of 25k cells has
 // only 98 chunks).  The cluster's warps share the chunk's rows (a warp per row, 8 x 32 indices in flight): strict-
 // ascent check, block starts, counts.  Counters are 16-bit halves of 32-bit words (a chunk has at most 256 rows, so a
 // count fits) in each CTA's own shared memory, updated with 32-bit shared-memory atomics; at the end every CTA adds
 // up its slice of the genes over the cluster's S counter arrays through distributed shared memory.
-template <bool kPacked, int kScanThreads>
+template <bool kPacked>
 __global__ void __launch_bounds__(kScanThreads)
 relayout_rowscan_kernel(RelayoutParams P, int* __restrict__ bnd, long long n_rows_total, int tile_shift) {
     namespace cg = cooperative_groups;
@@ -219,17 +232,16 @@ relayout_rowscan_kernel(RelayoutParams P, int* __restrict__ bnd, long long n_row
     cluster.sync();                                               // nobody leaves while its counters are being read
 }
 
-template <int kGenes, int kCap>
 struct FillSmem {
-    unsigned mask[kTileRows / 32][kGenes];              // bit (row & 31) of word [row >> 5][gene]
-    int rank0[kTileRows / 32][kGenes];                  // staging slot of the gene's first nonzero in this row word
-    int off[kGenes + 1];                                // exclusive scan of the block's per-gene counts
-    long long gdelta[kGenes];                           // output position of staging slot s of gene j = gdelta[j] + s
-    int wsum[kGenes / 32];
+    unsigned mask[kTileRows / 32][kTileGenes];          // bit (row & 31) of word [row >> 5][gene]
+    int rank0[kTileRows / 32][kTileGenes];              // staging slot of the gene's first nonzero in this row word
+    int off[kTileGenes + 1];                            // exclusive scan of the block's per-gene counts
+    long long gdelta[kTileGenes];                       // output position of staging slot s of gene j = gdelta[j] + s
+    int wsum[kTileGenes / 32];
     long long run_lo[kTileRows];                        // first element of the row's run in the block
     int run_len[kTileRows];
-    float sval[kCap];                                   // staged nonzeros of one pass; a denser tile takes several
-    unsigned char srow[kCap];                           // row inside the chunk
+    float sval[kStageCap];                              // staged nonzeros of one pass; a denser tile takes several
+    unsigned char srow[kStageCap];                      // row inside the chunk
 };
 
 // Visits every nonzero of the tile: f(row t, k-th element of the run, position in the arrays).  A warp takes four
@@ -270,13 +282,12 @@ __device__ __forceinline__ void for_each_run(const Smem& S, int n_rows, int warp
 // incidence goes into a 256 x 256 bit matrix in shared memory, the rank of an element inside its gene's run is the
 // popcount of the lower rows' bits, so the tile's nonzeros are placed in a staging buffer sorted by (gene, row) with
 // no ordering constraint between warps, and go out as one coalesced run per gene.
-template <int kTileGenes, int kStageCap, int kFillThreads, int kMinBlocks>
-__global__ void __launch_bounds__(kFillThreads, kMinBlocks)
+__global__ void __launch_bounds__(kFillThreads, kFillBlocksPerSm)
 relayout_tile_fill_kernel(RelayoutParams P, const int* __restrict__ bnd, long long n_rows_total, int blocks_per_cta,
                           const long long* __restrict__ seg_ptr, float* __restrict__ vals_out,
                           int* __restrict__ rows_out) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    using Smem = FillSmem<kTileGenes, kStageCap>;
+    using Smem = FillSmem;
     constexpr int kFillWarps = kFillThreads / 32;
     Smem& S = *reinterpret_cast<Smem*>(smem_raw);
     if (P.err && *P.err) return;                    // pass A found an unsorted row: bnd is not usable
@@ -549,14 +560,6 @@ MM_EXPORT int mm_csr_check_sorted(int device, void* stream, const int64_t* indpt
     return check_launch("mm_csr_check_sorted");
 }
 
-// Tile shapes of the fill pass (MM_RELAYOUT_CFG, read once at load): genes per block / staged nonzeros per pass / threads /
-// CTAs per SM.  The count pass writes the block starts at the same granularity, so both calls read the same setting.
-static int tile_cfg() {
-    const int c = tuning().relayout_cfg;
-    return (c >= 0 && c <= 4) ? c : 2;      // measured: 256-gene tiles, two 512-thread CTAs per SM (scripts/ab_relayout.py)
-}
-static int tile_genes_of(int cfg) { return (cfg == 2 || cfg == 3) ? 256 : 128; }
-
 static int tile_launch_shape(int n_chunks, int n_genes, int tile_genes, int* blocks_per_cta, dim3* grid) {
     const int n_blocks = (n_genes + tile_genes - 1) / tile_genes;
     // enough CTAs for a few waves of 2-3 per SM; a CTA walks at least one gene block
@@ -569,17 +572,14 @@ static int tile_launch_shape(int n_chunks, int n_genes, int tile_genes, int* blo
     return 0;
 }
 
-template <int kGenes, int kCap, int kThreads, int kMinBlocks>
 static int launch_tile_fill(cudaStream_t st, const RelayoutParams& P, const int* bnd, long long n_rows,
                             const long long* seg_ptr, float* vals_out, int* rows_out) {
-    static_assert(kThreads >= kTileRows && kThreads >= kGenes, "a thread per row and per gene of the tile");
+    static_assert(kFillThreads >= kTileRows && kFillThreads >= kTileGenes, "a thread per row and per gene of the tile");
     int per; dim3 grid;
-    tile_launch_shape(P.n_chunks, P.n_genes, kGenes, &per, &grid);
-    const size_t smem = sizeof(FillSmem<kGenes, kCap>);
-    MM_CUDA(cudaFuncSetAttribute(relayout_tile_fill_kernel<kGenes, kCap, kThreads, kMinBlocks>,
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    relayout_tile_fill_kernel<kGenes, kCap, kThreads, kMinBlocks><<<grid, kThreads, smem, st>>>(
-        P, bnd, n_rows, per, seg_ptr, vals_out, rows_out);
+    tile_launch_shape(P.n_chunks, P.n_genes, kTileGenes, &per, &grid);
+    const size_t smem = sizeof(FillSmem);
+    MM_CUDA(cudaFuncSetAttribute(relayout_tile_fill_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    relayout_tile_fill_kernel<<<grid, kFillThreads, smem, st>>>(P, bnd, n_rows, per, seg_ptr, vals_out, rows_out);
     return check_launch("relayout_tile_fill");
 }
 
@@ -615,18 +615,13 @@ MM_EXPORT int mm_relayout_count(int device, void* stream, const int64_t* indptr,
         // 32-bit counters up to 24k genes (96 KB: two CTAs per SM), 16-bit halves above
         const bool packed = n_genes > 24576;
         const size_t smem = sizeof(unsigned) * (size_t)(packed ? (n_genes + 1) / 2 : n_genes);
-        // warps per CTA: a warp walks its rows one after the other (order -> indptr -> row loads is a chain of dependent
-        // loads per row), so more warps = fewer rows per warp (MM_RELAYOUT_SCAN_THREADS: 256 / 512 / 1024; measured on C2:
-        // 0.20 / 0.21 / 0.26 ms, so 256 stays)
-        const int scan_threads = tuning().relayout_scan_threads == 512 ? 512 : tuning().relayout_scan_threads == 1024 ? 1024 : 256;
-        auto kern = packed ? (scan_threads == 256 ? relayout_rowscan_kernel<true, 256> : scan_threads == 512 ? relayout_rowscan_kernel<true, 512> : relayout_rowscan_kernel<true, 1024>)
-                           : (scan_threads == 256 ? relayout_rowscan_kernel<false, 256> : scan_threads == 512 ? relayout_rowscan_kernel<false, 512> : relayout_rowscan_kernel<false, 1024>);
+        auto kern = packed ? relayout_rowscan_kernel<true> : relayout_rowscan_kernel<false>;
         MM_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         int S = 1;                              // CTAs per chunk (cluster size): at least ~4 CTAs per SM when possible
         while (S < 8 && (long long)n_chunks * S < 148 * 4) S *= 2;
         cudaLaunchConfig_t cfg = {};
         cfg.gridDim = dim3((unsigned)n_chunks * S);
-        cfg.blockDim = dim3(scan_threads);
+        cfg.blockDim = dim3(kScanThreads);
         cfg.dynamicSmemBytes = smem;
         cfg.stream = st;
         cudaLaunchAttribute attr[1];
@@ -634,8 +629,7 @@ MM_EXPORT int mm_relayout_count(int device, void* stream, const int64_t* indptr,
         attr[0].val.clusterDim.x = (unsigned)S; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
         cfg.attrs = attr;
         cfg.numAttrs = 1;
-        MM_CUDA(cudaLaunchKernelEx(&cfg, kern, P, (int*)row_block_ptr, (long long)n_rows,
-                                   tile_genes_of(tile_cfg()) == 256 ? 8 : 7));
+        MM_CUDA(cudaLaunchKernelEx(&cfg, kern, P, (int*)row_block_ptr, (long long)n_rows, kTileShift));
         if (int s = check_launch("relayout_rowscan")) return s;
     } else if (n_chunks > 0) {
         MM_REQUIRE(indices, "null pointer");
@@ -666,15 +660,7 @@ MM_EXPORT int mm_relayout_fill(int device, void* stream, const int64_t* indptr, 
     P.cnt = cnt; P.err = err_flag;
     if (sorted_rows) {
         MM_REQUIRE(row_block_ptr && err_flag && n_rows >= 0, "tiled path: row_block_ptr / err_flag / n_rows");
-        cudaStream_t st = (cudaStream_t)stream;
-        const long long* sp = (const long long*)seg_ptr;
-        switch (tile_cfg()) {
-            case 1: return launch_tile_fill<128, 12288, 256, 3>(st, P, row_block_ptr, n_rows, sp, vals_out, rows_out);
-            case 2: return launch_tile_fill<256, 16384, 512, 2>(st, P, row_block_ptr, n_rows, sp, vals_out, rows_out);
-            case 3: return launch_tile_fill<256, 24576, 512, 1>(st, P, row_block_ptr, n_rows, sp, vals_out, rows_out);
-            case 4: return launch_tile_fill<128, 8192, 256, 4>(st, P, row_block_ptr, n_rows, sp, vals_out, rows_out);
-            default: return launch_tile_fill<128, 12288, 384, 3>(st, P, row_block_ptr, n_rows, sp, vals_out, rows_out);
-        }
+        return launch_tile_fill((cudaStream_t)stream, P, row_block_ptr, n_rows, (const long long*)seg_ptr, vals_out, rows_out);
     }
     const int per = kRelayoutThreads / 32;
     relayout_fill_kernel<<<(n_chunks + per - 1) / per, kRelayoutThreads, 0, (cudaStream_t)stream>>>(

@@ -18,7 +18,6 @@ _i32, _i64, _u64, _vp = C.c_int32, C.c_int64, C.c_uint64, C.c_void_p
 SIGNATURES = {
     "mm_csr_row_sums": [_vp, _vp, _vp, _i64, _vp, _vp],
     "mm_seg_moments": [_vp, _vp, _vp, _i64, _i64, _vp, _i64, _vp, _vp, _vp, _vp],
-    "mm_seg_moments_windows": [_vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp, _vp, _i32, _i32, _vp, _vp, _vp, _vp],
     "mm_validate_counts": [_vp, _i64, _vp],
     "mm_upload": [_vp, _vp, _i64, _i32],
     "mm_csr_check_sorted": [_vp, _vp, _i64, _vp],
@@ -56,8 +55,7 @@ SIGNATURES = {
 }
 
 # host-only helpers (no leading device / stream arguments)
-HOST_SIGNATURES = {"mm_poisson_table_size": [_i32, _vp, _vp], "mm_launch_count": [], "mm_reload_tuning": [], "mm_upload_release": [],
-                   "mm_block_debug_counters": [_i32, _vp]}
+HOST_SIGNATURES = {"mm_poisson_table_size": [_i32, _vp, _vp], "mm_launch_count": [], "mm_reload_tuning": [], "mm_upload_release": []}
 
 _lib = None
 
@@ -116,7 +114,7 @@ def launch_count():
 
 
 def reload_tuning():
-    """Re-read the MM_* tuning variables (they are otherwise read once, at library load).  Tests / tuning scripts."""
+    """Re-read the MM_MOMENTS_KERNEL test hook (otherwise read once, at library load; include/memento_b200.h)."""
     load().mm_reload_tuning()
 
 

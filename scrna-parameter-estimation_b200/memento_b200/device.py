@@ -76,7 +76,7 @@ UPLOAD_MIN_BYTES = 32 << 20      # larger pageable arrays go through mm_upload (
 def upload_threads():
     """Host threads of one mm_upload: the cores of the box shared out over the ranks of the node, at most 8."""
     ranks = max(1, int(os.environ.get("LOCAL_WORLD_SIZE", "1")))
-    return int(os.environ.get("MM_UPLOAD_THREADS", max(1, min(8, (os.cpu_count() or 1) // ranks))))
+    return max(1, min(8, (os.cpu_count() or 1) // ranks))
 
 
 def to_device(arr, device, dtype=None, pinned=False):
@@ -135,18 +135,6 @@ class CsrOnDevice:
                   gene_mask, out)
         timer.stop("csr_row_sums", ev)
         return out
-
-
-MOMENTS_KERNEL = "auto"      # "auto" | "windows" | "legacy": which mm_seg_moments* entry SegMatrix.moments calls (A/B switch)
-
-
-def WINDOWS_AUTO(seg, plan):
-    """auto rule of SegMatrix.use_windows beyond the piece-length test.  Measured on B200
-    (profiles/r02_moments_shapes.json): the row-window kernel ties with the span kernel where the 1/sf table does not
-    fit shared memory (1 M cells x 40 groups: 3.60 vs 3.66 TB/s) and loses where it does (25 k cells x 16 groups:
-    1.5 vs 3.3 TB/s) -- the gather's shared-memory wavefronts, not its source, are the cost -- so auto never picks
-    it; it stays reachable through MOMENTS_KERNEL = "windows" for A/B runs."""
-    return False
 
 
 class SegMatrix:
@@ -352,72 +340,9 @@ class SegMatrix:
             self._chunk_seg = idx.clamp_(0, max(self.n_seg - 1, 0)).to(torch.int32)
         return self._chunk_seg
 
-    # ------------------------------------------------------------------ row-window plan (csrc/moments.cu)
-    WINDOW_SMALL_ROWS = 12 * 1024       # a window up to here leaves room for 2+ CTAs per SM (96 KB of table)
-    WINDOW_MAX_ROWS = 28 * 1024         # 224 KB of table: one 768-thread CTA per SM
-    WINDOW_MIN_PIECE = 192              # mean nonzeros of a (gene, window) piece below which a warp per piece is wasteful
-
-    def window_plan(self):
-        """Row windows for mm_seg_moments_windows: every group is one window, or several equal ones when it is larger
-        than the shared-memory budget; the CTAs (two waves of resident CTAs) are shared out by window size.  Built
-        once per matrix.  None when there would be more than 65535 windows."""
-        if getattr(self, "_win", None) is None:
-            gs = self.group_start_host
-            sizes = np.diff(gs)
-            cap = self.WINDOW_SMALL_ROWS if sizes.max() <= self.WINDOW_SMALL_ROWS else self.WINDOW_MAX_ROWS
-            per_group = np.maximum(1, -(-sizes // cap)).astype(np.int64)
-            n_win = int(per_group.sum())
-            if n_win > 65535:
-                self._win = False
-                return None
-            lo, grp = [], []
-            for r, (n, k) in enumerate(zip(sizes, per_group)):
-                edges = gs[r] + (np.arange(k) * n) // k
-                lo.extend(edges.tolist())
-                grp.extend([r] * int(k))
-            lo.append(int(gs[-1]))
-            lo = np.asarray(lo, dtype=np.int64)
-            rows = np.diff(lo)
-            max_rows = int(max(1, rows.max()))
-            resident = int(np.clip((227 * 1024) // max(max_rows * 8 + 1024, 1), 1, 4)) if max_rows * 8 <= 100 * 1024 else 1
-            target = 148 * resident * 2
-            share = rows / max(1, rows.sum()) * target
-            parts = np.maximum(1, np.floor(share)).astype(np.int64)
-            short = target - int(parts.sum())
-            if short > 0:       # largest remainders first
-                parts[np.argsort(-(share - np.floor(share)), kind="stable")[:short]] += 1
-            parts = np.minimum(parts, max(1, self.G))
-            d = lambda a: torch.as_tensor(np.ascontiguousarray(a, dtype=np.int32), device=self.device)  # noqa: E731
-            self._win = {"n_win": n_win, "lo": d(lo), "group": d(grp), "parts": d(parts), "parts_max": int(parts.max()),
-                         "max_rows": max_rows, "group_win_lo": d(np.concatenate([[0], np.cumsum(per_group)])),
-                         "partial": None}
-        return self._win or None
-
-    def use_windows(self):
-        if MOMENTS_KERNEL == "legacy":
-            return False
-        plan = self.window_plan()
-        if plan is None or self.nnz == 0 or self.G == 0:
-            return False
-        if MOMENTS_KERNEL == "windows":
-            return True
-        # auto: long pieces, and either the whole table does not fit shared memory (the span kernel then gathers from
-        # L2) or ... (measured: profiles/r02_moments_shapes.json)
-        return self.nnz / (self.G * plan["n_win"]) >= self.WINDOW_MIN_PIECE and WINDOWS_AUTO(self, plan)
-
     def moments(self, inv_sf, timer=NULL_TIMER):
         """(5, G, R) float64 on the device: sum x, max x, sum x/sf, sum x/sf^2, sum x^2/sf^2."""
         out = torch.empty(5 * self.n_seg, dtype=torch.float64, device=self.device)
-        if self.use_windows():
-            plan = self.window_plan()
-            if plan["n_win"] > self.R and plan["partial"] is None:
-                plan["partial"] = torch.empty(plan["n_win"] * self.G * 5, dtype=torch.float64, device=self.device)
-            ev = timer.start()
-            _lib.call("mm_seg_moments_windows", self.device, self.vals, self.rows, self.seg_ptr, self.G, self.R,
-                      plan["n_win"], plan["lo"], plan["group"], plan["parts"], plan["parts_max"], plan["max_rows"],
-                      plan["group_win_lo"], inv_sf, out, plan["partial"])
-            timer.stop("seg_moments", ev)
-            return out.view(5, self.G, self.R)
         if self._big is None:      # scratch: big-segment list (fallback kernel) and per-tile edge partials
             n_chunks = (self.nnz + self.CHUNK - 1) // self.CHUNK
             self._big = torch.zeros(self.nnz // 4096 + 2, dtype=torch.int32, device=self.device)

@@ -3,7 +3,6 @@ regression + ASL, over tiles of genes.  Everything between the uploads and the r
 runs in our CUDA kernels (csrc/); the only host step per tile is grouping the genes by their
 group-validity mask (a (tile_genes x R) byte matrix) so that the small solves are shared.
 """
-import os
 
 import numpy as np
 import torch
@@ -298,7 +297,7 @@ def bootstrap_tile(seg, design, tab, n_genes, estimator, num_boot, seed, seg_ski
         timer.stop("boot_prepare", ev)
     # block rows of the Poissonised kernel in order of decreasing table length (longest-processing-time first)
     seg_order = None
-    if seg_info is not None and os.environ.get("MM_BOOT_LPT", "1") != "0":
+    if seg_info is not None:
         seg_order = torch.argsort(tab["seg_U"], descending=True, stable=True).to(torch.int32)
     ev = timer.start()
     _lib.call("mm_bootstrap_1d", dev, tab["entries"], seg.seg_ptr, tab["seg_lo"], n_seg, R, tab["seg_U"],
@@ -521,9 +520,8 @@ def ht_2d_tile(seg, design, cell_bin, idx1, idx2, true_corr, covariate, treatmen
     item_id = None
     if pair_id is not None:
         item_id = (pair_id[:, None] * R + torch.arange(R, device=dev)[None, :]).reshape(-1).contiguous()
-    item_order = None
-    if os.environ.get("MM_BOOT_LPT", "1") != "0":       # longest tables first (see bootstrap_tile)
-        item_order = torch.argsort(tab["item_U"], descending=True, stable=True).to(torch.int32)
+    # longest tables first (see bootstrap_tile)
+    item_order = torch.argsort(tab["item_U"], descending=True, stable=True).to(torch.int32)
     ev = timer.start()
     _lib.call("mm_pair_bootstrap", dev, tab["entries"], tab["item_ptr"], n_items, R, info, design.n_cells, tc,
               tab_pool, acc_pool, num_boot, seed, item_id, boot, good, item_order)

@@ -59,20 +59,28 @@ def test_block_cross_vs_numpy(sizes, n_genes, na, nb):
         assert (err <= 5e-6 * scale + 1e-12).all(), (r, float((err / (scale + 1e-300)).max()))
 
 
-def test_block_gemm_cluster_variant_equals_the_default(tuning):
-    """The 2 x 2 cluster kernel (TMA-multicast operand halves, MM_BLOCK_CLUSTER=2) performs the same MMAs in the same
-    order as the single-CTA kernel: equal bits, on tile counts that are odd / even / one each way (padding tiles of an
-    incomplete 2 x 2 group must load and multicast but store nothing)."""
-    for sizes, n_genes, na, nb in [([300, 517, 90], 700, 129, 700), ([200, 64], 400, 400, 390), ([150, 70], 300, 128, 300)]:
-        seg, dense, sf, gs = _random_matrix(sizes, n_genes, seed=7, density=0.2)
-        inv_sf = torch.as_tensor(1.0 / sf, device=seg.device)
-        sums = seg.moments(inv_sf)
-        idx_a, idx_b = np.arange(na), np.arange(n_genes - nb, n_genes)
-        tuning(MM_BLOCK_CLUSTER="1")
-        base = seg.block_cross(idx_a, idx_b, inv_sf, sums).clone()
-        tuning(MM_BLOCK_CLUSTER="2")
-        clus = seg.block_cross(idx_a, idx_b, inv_sf, sums)
-        assert torch.equal(base, clus), (sizes, na, nb)
+def test_block_gemm_cluster_variant_equals_the_default():
+    """The two epilogue store paths of mm_block_gemm give equal bits: TMA tensor stores (16-byte aligned output rows,
+    the path block_cross takes) and 8-byte stores (odd leading dimension), on grids of 2 x 6, 4 x 4 and 1 x 3 output
+    tiles with partial edge tiles.  Neither path writes past column n of a row."""
+    from memento_b200 import _lib
+    d = torch.device("cuda", 0)
+    g = torch.Generator().manual_seed(7)
+    for m, n, k_pad in [(129, 700, 640), (400, 390, 256), (128, 300, 192)]:
+        a = torch.randn(2, m, k_pad, generator=g).to(torch.float16).to(d)
+        b = torch.randn(2, n, k_pad, generator=g).to(torch.float16).to(d)
+        sa = (torch.rand(m, generator=g, dtype=torch.float64) + 0.5).to(d)
+        sb = (torch.rand(n, generator=g, dtype=torch.float64) + 0.5).to(d)
+        outs = []
+        for ldo in ((n + 7) // 8 * 8 + 8, n + 1 + n % 2):          # aligned rows / odd leading dimension
+            out = torch.full((m, ldo), -3.0, dtype=torch.float64, device=d)
+            _lib.call("mm_block_gemm", d, a[0], a[1], m, b[0], b[1], n, k_pad, sa, sb, out, ldo)
+            assert bool((out[:, n:] == -3.0).all()), (m, n, ldo)
+            outs.append(out[:, :n])
+        assert torch.equal(outs[0], outs[1]), (m, n)
+        want = ((a[0].double() + a[1].double() / 2048) @ (b[0].double() + b[1].double() / 2048).T) * sa[:, None] * sb[None, :]
+        scale = ((a[0].double().abs() @ b[0].double().abs().T) * sa[:, None] * sb[None, :])
+        assert bool(((outs[0] - want).abs() <= 1e-5 * scale + 1e-9).all()), (m, n)
 
 
 def test_compute_2d_moments_dense_block_vs_pair_path(monkeypatch):

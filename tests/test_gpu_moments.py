@@ -90,23 +90,48 @@ def test_seg_moments_every_kernel(kernel, name, tuning):
     _run(CASES[name], seed=5)
 
 
+def _tile_pieces(lens):
+    """Pieces per 4096-nonzero tile as seg_moments_tile_kernel counts them (segments from the one holding the tile's
+    first nonzero to the one holding the next tile's first nonzero)."""
+    seg_ptr = np.concatenate([[0], np.cumsum(lens)])
+    n_seg = len(lens)
+    first = np.clip(np.searchsorted(seg_ptr, np.arange(0, max(int(seg_ptr[-1]), 1), 4096), side="right") - 1, 0, n_seg - 1)
+    first[0] = 0
+    return np.append(first[1:], n_seg - 1) - first + 1
+
+
+# the tile kernel picks its regime per tile: the span regime up to 32 pieces, the group / lane regimes above
+TILE_REGIME_CASES = {"0": ("exact_tile_edges", "multi_tile_segments", "one_long_piece_per_tile", "mixed"),
+                     "1": ("many_small", "more_than_staged_boundaries", "window_of_31")}
+
+
 @pytest.mark.parametrize("regime", ["0", "1"])
 def test_seg_moments_tile_regimes(regime, tuning):
-    tuning(MM_MOMENTS_KERNEL="tile", MM_MOMENTS_REGIME=regime)
-    for name in ("mixed", "exact_tile_edges", "multi_tile_segments", "many_small"):
+    """The tile kernel on structures whose every tile takes the span regime ("0") or the group / lane regimes ("1")."""
+    tuning(MM_MOMENTS_KERNEL="tile")
+    for name in TILE_REGIME_CASES[regime]:
+        pieces = _tile_pieces(CASES[name])
+        assert (pieces.max() <= 32) if regime == "0" else (pieces.min() > 32), (name, pieces)
         _run(CASES[name], seed=6)
 
 
 @pytest.mark.parametrize("name", ["exact_span_edges", "window_of_31", "multi_tile_segments", "ragged_end3", "mixed"])
 def test_seg_moments_stream_single_span_chunks(name, tuning):
-    tuning(MM_MOMENTS_KERNEL="stream", MM_MOMENTS_CHUNK=1)
-    _run(CASES[name], seed=8)
+    """Span-edge structures through the stream kernel: with the 1/sf table in shared memory and with the gather from
+    global memory it is the same summation, so both give bit-identical sums."""
+    got = {}
+    for kern in ("stream", "stream_l1"):
+        tuning(MM_MOMENTS_KERNEL=kern)
+        got[kern] = _run(CASES[name], seed=8)
+    np.testing.assert_array_equal(got["stream"], got["stream_l1"])
 
 
 @pytest.mark.parametrize("name", ["exact_span_edges", "exact_chunk_edges", "window_of_31", "ragged_end3", "mixed"])
 def test_seg_moments_stream_short_spans(name, tuning):
-    tuning(MM_MOMENTS_KERNEL="stream", MM_MOMENTS_CHUNK=8, MM_MOMENTS_THREADS=896)
-    _run(CASES[name], seed=9)
+    """Span- and chunk-edge structures through the stream kernel when the 1/sf table (40 000 cells, 320 KB) does not
+    fit shared memory, so that the launch itself falls back to the gather from global memory."""
+    tuning(MM_MOMENTS_KERNEL="stream")
+    _run(CASES[name], n_cells=40000, seed=9)
 
 
 def test_seg_moments_table_too_large_for_smem(tuning):
@@ -114,10 +139,16 @@ def test_seg_moments_table_too_large_for_smem(tuning):
     _run(CASES["mixed"], n_cells=40000, seed=7)
 
 
+# W lanes per segment of the fallback kernel, chosen from the mean segment length (< 48 -> 8, < 1024 -> 16, else 32)
+LANE_WIDTH_CASES = {"8": "many_small", "16": "mixed", "32": "multi_tile_segments"}
+
+
 @pytest.mark.parametrize("w", ["8", "16", "32"])
-def test_seg_moments_lane_widths(w, tuning):
-    tuning(MM_MOMENTS_W=w)
-    _run(CASES["mixed"], seed=5, use_tiles=False)
+def test_seg_moments_lane_widths(w):
+    lens = CASES[LANE_WIDTH_CASES[w]]
+    mean = sum(lens) // len(lens)
+    assert (8 if mean < 48 else 16 if mean < 1024 else 32) == int(w), mean
+    _run(lens, seed=5, use_tiles=False)
 
 
 def test_seg_moments_empty_matrix():
@@ -125,7 +156,7 @@ def test_seg_moments_empty_matrix():
     assert not got.any()
 
 
-# ----------------------------------------------------------------------------- row-window kernel
+# ----------------------------------------------------------------------------- grouped matrices
 def _grouped_case(n_cells, n_genes, sizes, density, seed):
     """A group-sorted matrix with the given group sizes: rows of segment (g, r) lie in the group's row range."""
     rng = np.random.default_rng(seed)
@@ -152,15 +183,15 @@ def _grouped_case(n_cells, n_genes, sizes, density, seed):
 
 @pytest.mark.parametrize("case", [
     dict(n_cells=3000, n_genes=40, sizes=[1000, 0, 1500, 500], density=0.3),          # an empty group
-    dict(n_cells=20000, n_genes=25, sizes=[20000], density=0.2),                      # one group, one large window
-    dict(n_cells=70001, n_genes=12, sizes=[70001], density=0.1),                      # one group cut into 3 windows
-    dict(n_cells=65000, n_genes=10, sizes=[30000, 5, 34995], density=0.15),           # cut groups next to a tiny one
+    dict(n_cells=20000, n_genes=25, sizes=[20000], density=0.2),                      # one large group
+    dict(n_cells=70001, n_genes=12, sizes=[70001], density=0.1),                      # one group, table beyond shared memory
+    dict(n_cells=65000, n_genes=10, sizes=[30000, 5, 34995], density=0.15),           # large groups next to a tiny one
     dict(n_cells=5000, n_genes=300, sizes=[313] * 15 + [305], density=0.25),          # C2-like: many genes, 16 groups
     dict(n_cells=64, n_genes=3, sizes=[1, 63], density=0.9),
 ])
-def test_seg_moments_window_kernel(case):
-    """mm_seg_moments_windows (a group's 1/sf slice in shared memory, one warp per (gene, window) piece) against the
-    numpy restatement and against the span / tile kernels (same sums, another order)."""
+def test_seg_moments_grouped(case):
+    """SegMatrix.moments on group-sorted matrices (several groups, empty and full segments) against the numpy
+    restatement; deterministic."""
     vals, rows, seg_ptr, inv_sf, gs = _grouped_case(seed=11, **case)
     d = torch.device("cuda", 0)
     R = len(case["sizes"])
@@ -168,18 +199,9 @@ def test_seg_moments_window_kernel(case):
                             torch.as_tensor(seg_ptr, device=d), case["n_genes"], R, case["n_cells"], gs)
     w = torch.as_tensor(inv_sf, device=d)
     want = _reference(vals, rows, seg_ptr, inv_sf)
-    got = {}
-    for kern in ("windows", "legacy"):
-        dev_mod.MOMENTS_KERNEL = kern
-        try:
-            a = seg.moments(w).cpu().numpy().reshape(5, -1)
-            b = seg.moments(w).cpu().numpy().reshape(5, -1)
-        finally:
-            dev_mod.MOMENTS_KERNEL = "auto"
-        np.testing.assert_array_equal(a, b)                  # deterministic
-        np.testing.assert_array_equal(a[0], want[0])
-        np.testing.assert_array_equal(a[1], want[1])
-        np.testing.assert_allclose(a[2:], want[2:], rtol=1e-12, atol=0)
-        got[kern] = a
-    plan = seg.window_plan()
-    assert plan["n_win"] >= R and plan["max_rows"] <= dev_mod.SegMatrix.WINDOW_MAX_ROWS
+    a = seg.moments(w).cpu().numpy().reshape(5, -1)
+    b = seg.moments(w).cpu().numpy().reshape(5, -1)
+    np.testing.assert_array_equal(a, b)                  # deterministic
+    np.testing.assert_array_equal(a[0], want[0])
+    np.testing.assert_array_equal(a[1], want[1])
+    np.testing.assert_allclose(a[2:], want[2:], rtol=1e-12, atol=0)
