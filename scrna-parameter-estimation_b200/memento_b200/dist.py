@@ -12,8 +12,15 @@ SAME cells and runs the whole pipeline on it.  The only exchanges are tiny and s
                                                   all-gathers one G-length vector
   * results                                    -> one all-gather of 7 doubles per test (ht_1d_moments); gene names and
                                                   per-rank sizes are exchanged once per gene set
+  * 2D (compute_2d_moments, ht_2d_moments)     -> a pair is computed by the rank holding its SECOND gene; the columns of
+                                                  the first genes held elsewhere are imported once per pair set (one
+                                                  variable-length device buffer per source rank); per-group variances,
+                                                  covariances and test results are all-gathered so that every rank ends
+                                                  with the full-length arrays in the caller's pair order
 
-No collective is inside a hot kernel, so there is nothing to fuse with one.
+No collective is inside a hot kernel, so there is nothing to fuse with one.  With a gloo group the tensors of the
+device-side exchanges are staged through the host and come back on the device they came from, so that two ranks can
+share one GPU.
 """
 import numpy as np
 import torch
@@ -39,12 +46,46 @@ class DistContext:
         return t.to(self.device) if self.device is not None else t.cpu()
 
     def all_reduce_sum(self, a):
-        """Element-wise sum over ranks.  Accepts a numpy array or a tensor; returns the same kind."""
+        """Element-wise sum over ranks.  Accepts a numpy array or a tensor; returns the same kind (a tensor on the
+        device of ``a``)."""
         was_np = not isinstance(a, torch.Tensor)
         t = self._t(a, torch.float64).contiguous().clone()
         tdist.all_reduce(t, op=tdist.ReduceOp.SUM, group=self.group)
         self.bytes_reduced += t.numel() * 8
-        return t.cpu().numpy() if was_np else t
+        return t.cpu().numpy() if was_np else t.to(a.device)
+
+    def all_gather_tensors(self, t, sizes):
+        """Per-rank 1-D tensors whose lengths (``sizes``, one per rank) every rank already knows, as a list in rank
+        order of views of one buffer on the device of ``t``: ONE all-gather of padded blocks, straight between device
+        buffers under NCCL (through the host under gloo)."""
+        n_max = max(1, max(sizes))
+        block = torch.zeros(n_max, dtype=t.dtype, device=t.device if self.device is not None else "cpu")
+        block[:t.numel()] = t.reshape(-1)
+        out = torch.empty(self.world * n_max, dtype=t.dtype, device=block.device)
+        if self.device is not None:
+            tdist.all_gather_into_tensor(out, block, group=self.group)
+        else:
+            tdist.all_gather(list(out.view(self.world, n_max).unbind(0)), block, group=self.group)
+        self.bytes_gathered += out.numel() * out.element_size()
+        out = out.to(t.device)
+        return [out[r * n_max:r * n_max + n] for r, n in enumerate(sizes)]
+
+    def exchange_from_each(self, t):
+        """Variable-length exchange: every rank's 1-D uint8 tensor ``t`` to every rank.  The lengths are all-gathered
+        first, then each source rank broadcasts its buffer (device to device under NCCL).  Returns the list of the
+        ranks' buffers in rank order, on the device of ``t`` (this rank's entry is ``t`` itself)."""
+        sizes, _ = self.all_gather_concat(np.array([t.numel()], dtype=np.int64))
+        outs = []
+        for src, n in enumerate(sizes.tolist()):
+            if src == self.rank:
+                buf = t if self.device is not None else t.cpu()
+            else:
+                buf = torch.empty(int(n), dtype=torch.uint8, device=t.device if self.device is not None else "cpu")
+            if n:
+                tdist.broadcast(buf, src=src, group=self.group)
+                self.bytes_gathered += int(n)
+            outs.append(t if src == self.rank else buf.to(t.device))
+        return outs
 
     def all_gather_concat(self, a, axis=0):
         """Concatenate per-rank numpy arrays (different lengths along ``axis`` allowed) in rank order."""
@@ -90,9 +131,13 @@ class DistContext:
 
     def all_gather_names(self, names):
         """Concatenate per-rank lists of strings (gene names) in rank order."""
+        return [n for part in self.all_gather_objects(list(names)) for n in part]
+
+    def all_gather_objects(self, obj):
+        """Every rank's picklable ``obj``, as a list in rank order."""
         outs = [None] * self.world
-        tdist.all_gather_object(outs, list(names), group=self.group)
-        return [n for part in outs for n in part]
+        tdist.all_gather_object(outs, obj, group=self.group)
+        return outs
 
     def barrier(self):
         tdist.barrier(group=self.group)

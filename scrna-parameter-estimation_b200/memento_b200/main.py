@@ -8,6 +8,7 @@ per-(gene, group) moments, compression, bootstrap, regression, ASL) runs in the 
 ``np.quantile`` / ``np.polyfit`` / ``binned_statistic`` semantics are part of the contract.
 There is no CPU fallback: without a CUDA device or the built library every call raises.
 """
+import hashlib
 import os
 import time
 
@@ -54,6 +55,8 @@ class DeviceState:
         self.dist = None         # DistContext when the genes are sharded over ranks
         self.host_profile = None # {section: seconds} when profiling (setup_memento(profile=True))
         self.gene_offset = 0     # global index of this rank's first gene column
+        self.gene_map = None     # gene-sharded runs: all ranks' genes (_gene_map)
+        self.seg2d = None        # gene-sharded runs: this rank's genes + the imported partner genes (_seg_2d)
 
     def __deepcopy__(self, memo):
         new = DeviceState(self.device)
@@ -390,6 +393,7 @@ def create_groups(adata, label_columns, label_delimiter="^", inplace=True):
         st.seg = base.regroup(to_device(codes, st.device, np.int32), R, to_device(rank, st.device, np.int32))
     st.csr = None
     st.design = None            # group sizes / q / trend belong to the previous grouping
+    st.gene_map = st.seg2d = None
     for key in ("size_factor", "approx_size_factor", "all_approx_size_factor", "1d_moments", "mv_regressor"):
         mem.pop(key, None)      # per-group state of the previous grouping
     X = adata.X
@@ -474,6 +478,7 @@ def compute_1d_moments(adata, inplace=True, min_perc_group=0.7, filter_genes=Tru
         mem["group_cells"] = {g: mem["group_cells"][g].with_genes(st.x_cols) for g in groups}
         adata._inplace_subset_var(overall)
     mem["gene_rv_filter"] = {g: rv_filter[:, r].copy() for r, g in enumerate(groups)}
+    st.gene_map = st.seg2d = None
 
     # pooled mean-variance trend over the groups' (mean, var), concatenated in group order (:232-245)
     if st.host_profile is not None:
@@ -695,26 +700,21 @@ def _gather_1d_ht(adata, t_gene):
     contiguous gene ranges), as ``uns['memento']['1d_ht_all']`` = {"gene": names, "n_tests": per-gene test counts,
     the six flat arrays of ``1d_ht``}.  One variable-length all-gather of (tests of the rank) x 7 doubles over
     NCCL / NVLink: the six statistics plus the gene's position in the gathered name list; the names themselves are
-    exchanged once per gene set (they change only when compute_1d_moments filters).  The rank's own ``1d_ht`` keeps
-    matching its ``adata.var``."""
+    exchanged once per gene set (_gene_map).  The rank's own ``1d_ht`` keeps matching its ``adata.var``."""
     mem = adata.uns["memento"]
     st = _state(adata)
     ht = mem["1d_ht"]
-    names_local = adata.var.index
+    gm = _gene_map(st, adata.var.index)
     n_local = int(t_gene.sum())
-    key = (len(names_local), n_local, hash(tuple(names_local[:: max(1, len(names_local) // 64)])))
-    if getattr(st, "all_names_key", None) != key:       # once per gene set / treatment_for_gene: names and sizes
-        counts, _ = st.dist.all_gather_concat(np.array([len(names_local), n_local], dtype=np.int64))
-        counts = counts.reshape(-1, 2)
-        st.all_names = st.dist.all_gather_names(names_local.tolist())
-        st.all_names_lo = int(counts[:st.dist.rank, 0].sum())
-        st.all_tests = [int(c) for c in counts[:, 1]]
-        st.all_names_key = key
-    gene_pos = np.repeat(st.all_names_lo + np.arange(t_gene.size), t_gene).astype(np.float64)
+    all_tests = gm["tests"].get(n_local)
+    if all_tests is None:           # once per gene set / treatment_for_gene: the ranks' test counts
+        counts, _ = st.dist.all_gather_concat(np.array([n_local], dtype=np.int64))
+        all_tests = gm["tests"][n_local] = [int(c) for c in counts]
+    gene_pos = np.repeat(gm["lo"] + np.arange(t_gene.size), t_gene).astype(np.float64)
     packed = np.stack([ht[k][:n_local] for k in _HT_KEYS] + [gene_pos], axis=1)     # (tests, 7)
-    allv = st.dist.all_gather_known(packed, st.all_tests)
+    allv = st.dist.all_gather_known(packed, all_tests)
     pos = np.rint(allv[:, 6]).astype(np.int64)
-    res = {"gene": st.all_names, "n_tests": np.bincount(pos, minlength=len(st.all_names)).astype(np.int64)}
+    res = {"gene": gm["names"], "n_tests": np.bincount(pos, minlength=len(gm["names"])).astype(np.int64)}
     for j, k in enumerate(_HT_KEYS):
         res[k] = np.ascontiguousarray(allv[:, j])
     mem["1d_ht_all"] = res
@@ -731,6 +731,9 @@ def compute_2d_moments(adata, gene_pairs, inplace=True):
         with _Section(st, "compute_1d_moments: bin size factors"):
             _bin_size_factor(adata)
     groups = mem["groups"]
+    if st.dist is not None:
+        mem["2d_moments"] = _compute_2d_sharded(adata, gene_pairs)
+        return adata if not inplace else None
     idx1, idx2 = _pair_indices(adata.var.index, gene_pairs)
     out = {"gene_pairs": gene_pairs, "gene_idx_1": idx1, "gene_idx_2": idx2}
     n_cells = np.diff(st.group_start).astype(np.float64)
@@ -761,16 +764,8 @@ def compute_2d_moments(adata, gene_pairs, inplace=True):
                 cov_d = cov_d[pos_d]
             corr_same = (1 - q) * s3_d[i1_d, r] / n_cells[r]                               # estimator.py:229-230
             cov_d = torch.where(same_d, cov_d - corr_same, cov_d)
-            var_g = to_device(mem["1d_moments"][g][1], dev, np.float64)
-            var_g = torch.where(var_g > 0, var_g, torch.full_like(var_g, float("nan")))      # _corr_from_cov, :281-292
-            denom = torch.sqrt(var_g[i1_d] * var_g[i2_d])
-            corr_d = torch.where(torch.isfinite(denom), cov_d / denom, torch.full_like(cov_d, 5.0))
-            corr_d = corr_d.clamp(-1.0, 1.0)
-            # clamp maps NaN to NaN; the reference leaves cov / denom = NaN only where cov is NaN (never here)
-            var_h = var_g.cpu().numpy()
-            out[g] = LazyArrays({"cov": (lambda t=cov_d: t.cpu().numpy()), "corr": (lambda t=corr_d: t.cpu().numpy()),
-                                 "var_1": (lambda v=var_h: v[idx1]), "var_2": (lambda v=var_h: v[idx2])},
-                                dev={"cov": cov_d, "corr": corr_d})
+            out[g] = _block_group_arrays(cov_d, to_device(mem["1d_moments"][g][1], dev, np.float64), idx1, idx2,
+                                         i1_d, i2_d)
     else:
         for r, g in enumerate(groups):
             q = mem["group_q"][g]
@@ -783,6 +778,21 @@ def compute_2d_moments(adata, gene_pairs, inplace=True):
     mem["2d_moments"] = out
     if not inplace:
         return adata
+
+
+def _block_group_arrays(cov_d, var_g, idx1, idx2, i1_d, i2_d):
+    """One group's ``2d_moments`` record of the dense-block path: correlation from the device covariances ``cov_d`` (pair
+    order) and the group's variance vector ``var_g`` (device, indexed by ``i1_d`` / ``i2_d``); the arrays stay on the
+    device until read."""
+    var_g = torch.where(var_g > 0, var_g, torch.full_like(var_g, float("nan")))      # _corr_from_cov, :281-292
+    denom = torch.sqrt(var_g[i1_d] * var_g[i2_d])
+    corr_d = torch.where(torch.isfinite(denom), cov_d / denom, torch.full_like(cov_d, 5.0))
+    corr_d = corr_d.clamp(-1.0, 1.0)
+    # clamp maps NaN to NaN; the reference leaves cov / denom = NaN only where cov is NaN (never here)
+    var_h = var_g.cpu().numpy()
+    return LazyArrays({"cov": (lambda t=cov_d: t.cpu().numpy()), "corr": (lambda t=corr_d: t.cpu().numpy()),
+                       "var_1": (lambda v=var_h: v[idx1]), "var_2": (lambda v=var_h: v[idx2])},
+                      dev={"cov": cov_d, "corr": corr_d})
 
 
 def _pair_indices(names, gene_pairs):
@@ -1004,6 +1014,15 @@ def ht_2d_moments(adata, covariate, treatment, treatment_for_gene=None, inplace=
     n_all = idx1.shape[0]
     if bootstrap not in ("pair", "shared"):
         raise ValueError("bootstrap must be 'pair' or 'shared'")
+    if st.dist is not None:
+        _check_same_on_all_ranks(st, "ht_2d_moments", [
+            idx1, idx2, cov, tr, list(covariate.columns), list(treatment.columns), list(covariate.index),
+            list(treatment.index), num_boot, seed, approx, resample_rep, bootstrap])
+        out = _ht_2d_sharded(adata, cov, tr, num_boot, seed, approx, one_sample, resample_rep, workspace_bytes,
+                             bootstrap)
+        mem["2d_ht"] = {"treatment": treatment, "covariate": covariate, "corr_coef": out["coef"],
+                        "corr_se": out["se"], "corr_asl": out["asl"]}
+        return adata if not inplace else None
     block = _as_dense_block(idx1, idx2) if bootstrap == "shared" else None
     # unordered de-duplication, first occurrence computes (main.py:467-482)
     owner, uniq = _first_unordered(idx1, idx2) if block is None else _first_unordered_block(*block)
@@ -1062,3 +1081,345 @@ def ht_2d_moments(adata, covariate, treatment, treatment_for_gene=None, inplace=
                     "corr_se": out["se"], "corr_asl": out["asl"]}
     if not inplace:
         return adata
+
+
+# --------------------------------------------------------------------------- 2D in a gene-sharded run
+# compute_2d_moments and ht_2d_moments are collective calls there: every rank passes the same pairs (global gene names)
+# and arguments and ends with the same full-length arrays, in the caller's pair order, that the unsharded run produces.
+# A pair is computed by the rank holding its SECOND gene; the columns of the first genes that live on other ranks are
+# imported once per pair set (_seg_2d).  Global position of a gene = its index in the rank blocks concatenated (the
+# unsharded run's adata.var order); global id = its original column plus the rank's gene_offset (the RNG stream id).
+
+def _gene_map(st, names_local):
+    """The genes of all ranks, from one all-gather per gene set (create_groups and compute_1d_moments drop it):
+    "names" (global order), "index" (pd.Index of them), "bounds" (int64 [world + 1]: rank r holds the global positions
+    bounds[r] .. bounds[r + 1] - 1), "lo" (this rank's first position), "gid" (global id of every position, None when
+    the state has no gene index) and "tests" (test counts per rank of ht_1d_moments, by this rank's count)."""
+    gm = getattr(st, "gene_map", None)
+    if gm is None:
+        gid = getattr(st, "gene_index", None)
+        gid = None if gid is None else np.asarray(gid, dtype=np.int64) + st.gene_offset
+        parts = st.dist.all_gather_objects((list(names_local), gid))
+        names = [n for p, _ in parts for n in p]
+        bounds = np.concatenate([[0], np.cumsum([len(p) for p, _ in parts])]).astype(np.int64)
+        gm = st.gene_map = {"names": names, "index": pd.Index(names), "bounds": bounds,
+                            "lo": int(bounds[st.dist.rank]), "tests": {},
+                            "gid": None if gid is None else np.concatenate([g for _, g in parts])}
+    return gm
+
+
+def _check_same_on_all_ranks(st, what, parts, error=None):
+    """Collective argument check: every rank all-gathers a digest of ``parts`` (arrays or reprs) before any other
+    collective of the call, so that ranks passed different arguments raise on EVERY rank instead of hanging in a later
+    collective.  ``error``: this rank's own failure (raised here, after the exchange)."""
+    h = hashlib.blake2b(digest_size=16)
+    for p in parts:
+        h.update(np.ascontiguousarray(p).tobytes() if isinstance(p, np.ndarray) else repr(p).encode())
+    got = st.dist.all_gather_objects((h.hexdigest(), error is not None))
+    if error is not None:
+        raise error
+    if any(failed for _, failed in got):
+        raise ValueError("%s: the call failed on rank(s) %s" % (what, [r for r, (_, f) in enumerate(got) if f]))
+    if len({d for d, _ in got}) != 1:
+        raise ValueError("%s is a collective call in a gene-sharded run: every rank must pass the same gene pairs, "
+                         "covariate / treatment frames and keyword arguments (digests differ: %s)"
+                         % (what, [d[:8] for d, _ in got]))
+
+
+def plan_sharded_pairs(gpos1, gpos2, bounds, dedup=True):
+    """Work split of a pair list over the ranks of a gene-sharded run; pure numpy, identical on every rank.
+    ``gpos1`` / ``gpos2``: global positions of the two genes of every pair; ``bounds``: int64 [world + 1], rank r
+    holds the positions bounds[r] .. bounds[r + 1] - 1.  Returns
+      "rank":    the rank that computes every pair (the holder of its second gene),
+      "pairs":   per rank, the (ascending) indices of its pairs,
+      "imports": per rank, the sorted global positions of the first genes of its pairs that other ranks hold,
+    and with ``dedup`` the unordered de-duplication of :func:`_first_unordered` ("owner", "uniq") and
+    "tests": per rank, its pairs among "uniq" (the ones ht_2d_moments tests)."""
+    gpos1, gpos2 = np.asarray(gpos1, dtype=np.int64), np.asarray(gpos2, dtype=np.int64)
+    bounds = np.asarray(bounds, dtype=np.int64)
+    world = bounds.size - 1
+    rank = np.searchsorted(bounds, gpos2, side="right") - 1
+    order = np.argsort(rank, kind="stable")
+    cuts = np.searchsorted(rank[order], np.arange(world + 1))
+    pairs = [order[cuts[r]:cuts[r + 1]] for r in range(world)]
+    imports = []
+    for r in range(world):
+        need = np.zeros(int(bounds[-1]), dtype=bool)
+        need[gpos1[pairs[r]]] = True
+        need[bounds[r]:bounds[r + 1]] = False
+        imports.append(np.flatnonzero(need))
+    plan = {"rank": rank, "pairs": pairs, "imports": imports}
+    if dedup:
+        owner, uniq = _first_unordered(gpos1, gpos2)
+        plan.update(owner=owner, uniq=uniq, tests=[uniq[rank[uniq] == r] for r in range(world)])
+    return plan
+
+
+def _block_share(genes_a, genes_b, bounds):
+    """:func:`plan_sharded_pairs` for a full block A x B (sorted unique global positions), without touching the
+    |A| |B| pairs: rank r computes A x genes_b[jb[r]:jb[r + 1]] (B is sorted, so its genes on one rank are a slice)
+    and imports the genes of A that it does not hold, when it computes anything.  Returns (jb, imports)."""
+    jb = np.searchsorted(genes_b, bounds)
+    imports = [genes_a[(genes_a < bounds[r]) | (genes_a >= bounds[r + 1])] if jb[r + 1] > jb[r]
+               else np.zeros(0, dtype=np.int64) for r in range(bounds.size - 1)]
+    return jb, imports
+
+
+def _concat_seg(parts, n_cells, group_start):
+    """Genes of several group-sorted matrices (same cells, same groups) one after the other: [(vals, rows, seg_ptr)]."""
+    vals = torch.cat([p[0] for p in parts])
+    rows = torch.cat([p[1] for p in parts])
+    ptrs, base = [parts[0][2][:1]], 0
+    for p in parts:
+        ptrs.append(p[2][1:] - p[2][0] + base)
+        base += int(p[0].numel())
+    n_seg = sum(int(p[2].numel()) - 1 for p in parts)
+    R = group_start.size - 1
+    return SegMatrix(vals, rows, torch.cat(ptrs), n_seg // R, R, n_cells, group_start)
+
+
+def _seg_2d(st, gm, imports):
+    """This rank's 2D matrix: its own genes followed by the genes ``imports[st.dist.rank]`` held by other ranks
+    (``imports``: sorted global positions, one list per rank, identical on every rank).  Collective: every rank sends
+    the genes any other rank imports from it as one device buffer [R segment lengths per gene (int64) | vals (float32)
+    | rows (int32)]; a gene's R segments are one contiguous range of the group-sorted CSC.  Cached on the state
+    (create_groups and compute_1d_moments drop it).  Returns {"seg", "row" (row of every global position, -1 when
+    absent), "sums" (device moment sums of the matrix), "import_bytes", "import_ms"}."""
+    dist, me = st.dist, st.dist.rank
+    key = (id(st.seg), tuple(hashlib.blake2b(np.ascontiguousarray(i).tobytes()).hexdigest() for i in imports))
+    if st.seg2d is not None and st.seg2d["key"] == key:
+        return st.seg2d
+    bounds, lo = gm["bounds"], gm["lo"]
+    seg, R = st.seg, st.seg.R
+    world = bounds.size - 1
+    G = int(bounds[-1])
+    row = np.full(G, -1, dtype=np.int64)
+    row[lo:lo + seg.G] = np.arange(seg.G)
+    row[imports[me]] = seg.G + np.arange(imports[me].size)
+    t0 = time.perf_counter()
+    nbytes = 0
+    if not any(i.size for i in imports):
+        mat = seg
+    else:
+        # the cells must be renumbered identically on every rank (create_groups is deterministic on the same obs)
+        starts = dist.all_gather_objects(np.asarray(st.group_start))
+        if not all(np.array_equal(s, starts[0]) for s in starts):
+            raise RuntimeError("gene-sharded 2D: the ranks' cell groupings differ (create_groups on different obs?)")
+        wanted = [np.zeros(G, dtype=bool) for _ in range(world)]       # what any other rank imports from rank s
+        for r, imp in enumerate(imports):
+            for s in range(world):
+                if s != r:
+                    wanted[s][imp[(imp >= bounds[s]) & (imp < bounds[s + 1])]] = True
+        sent = [np.flatnonzero(w) for w in wanted]
+        if sent[me].size:
+            sub = seg.select_genes(sent[me] - lo)
+            lens = (sub.seg_ptr[1:] - sub.seg_ptr[:-1]).contiguous()
+            buf = torch.cat([lens.view(torch.uint8), sub.vals.view(torch.uint8), sub.rows.view(torch.uint8)])
+        else:
+            buf = torch.zeros(0, dtype=torch.uint8, device=seg.device)
+        bufs = dist.exchange_from_each(buf)
+        parts = [(seg.vals, seg.rows, seg.seg_ptr)]
+        for s in range(world):
+            take = imports[me][(imports[me] >= bounds[s]) & (imports[me] < bounds[s + 1])]
+            if s == me or take.size == 0:
+                continue
+            n = sent[s].size
+            b = bufs[s]
+            nbytes += int(b.numel())
+            lens = b[:n * R * 8].view(torch.int64)
+            ptr = torch.zeros(n * R + 1, dtype=torch.int64, device=seg.device)
+            torch.cumsum(lens, 0, out=ptr[1:])
+            nnz = int(ptr[-1].item())
+            off = n * R * 8
+            vals = b[off:off + 4 * nnz].view(torch.float32)
+            rows = b[off + 4 * nnz:off + 8 * nnz].view(torch.int32)
+            got = SegMatrix(vals, rows, ptr, n, R, seg.n_cells, seg.group_start_host)
+            got = got.select_genes(np.searchsorted(sent[s], take))
+            parts.append((got.vals, got.rows, got.seg_ptr))
+        mat = seg if len(parts) == 1 else _concat_seg(parts, seg.n_cells, seg.group_start_host)
+    sums = mat.moments(st.inv_sf_sorted, st.timer)
+    torch.cuda.synchronize(st.device)
+    st.seg2d = {"key": key, "seg": mat, "row": row, "sums": sums, "import_bytes": nbytes,
+                "import_ms": (time.perf_counter() - t0) * 1e3}
+    return st.seg2d
+
+
+def _gathered_var(st, gm, mem, groups):
+    """(G_global, R) per-group variances (``1d_moments``) of all ranks' genes, all-gathered once per gene set."""
+    if gm.get("var") is None:
+        local = np.stack([mem["1d_moments"][g][1] for g in groups], axis=1)
+        gm["var"] = st.dist.all_gather_concat(local)[0]
+    return gm["var"]
+
+
+def _compute_2d_sharded(adata, gene_pairs):
+    """compute_2d_moments in a gene-sharded run (see the section comment)."""
+    mem = adata.uns["memento"]
+    st = _state(adata)
+    dist, me = st.dist, st.dist.rank
+    groups = mem["groups"]
+    R = len(groups)
+    dev = st.device
+    gm = _gene_map(st, adata.var.index)
+    error = None
+    try:
+        idx1, idx2 = _pair_indices(gm["index"], gene_pairs)
+    except KeyError as exc:
+        error, idx1, idx2 = exc, np.zeros(0, dtype=int), np.zeros(0, dtype=int)
+    _check_same_on_all_ranks(st, "compute_2d_moments", [idx1, idx2], error)
+    out = {"gene_pairs": gene_pairs, "gene_idx_1": idx1, "gene_idx_2": idx2}
+    var_all = _gathered_var(st, gm, mem, groups)
+    bounds = gm["bounds"]
+    n_cells = np.diff(st.group_start).astype(np.float64)
+    q = [mem["group_q"][g] for g in groups]
+    block = _as_dense_block(idx1, idx2)
+    if block is not None:
+        # this rank's share is A x (B on this rank): one tensor-core GEMM per group on the 2D matrix
+        genes_a, genes_b, pos = block
+        na, nb = genes_a.size, genes_b.size
+        jb, imports = _block_share(genes_a, genes_b, bounds)
+        m = _seg_2d(st, gm, imports)
+        own_b = genes_b[jb[me]:jb[me + 1]]
+        part = torch.zeros(0, dtype=torch.float64, device=dev)
+        if own_b.size:
+            ra = m["row"][genes_a]
+            cross = m["seg"].block_cross(ra, m["row"][own_b], st.inv_sf_sorted, m["sums"], timer=st.timer)
+            same_d = to_device(genes_a[:, None] == own_b[None, :], dev)
+            s3_d = m["sums"][3][to_device(ra, dev, np.int64)]                                # (|A|, R)
+            part = torch.empty((R, na, own_b.size), dtype=torch.float64, device=dev)
+            for r in range(R):
+                c = cross[r] / n_cells[r]
+                corr_same = ((1 - q[r]) * s3_d[:, r] / n_cells[r])[:, None]               # estimator.py:229-230
+                part[r] = torch.where(same_d, c - corr_same, c)
+        sizes = [R * na * int(jb[r + 1] - jb[r]) for r in range(dist.world)]
+        pieces = dist.all_gather_tensors(part.reshape(-1), sizes)
+        cov_blk = torch.empty((R, na, nb), dtype=torch.float64, device=dev)
+        for r, p in enumerate(pieces):
+            cov_blk[:, :, jb[r]:jb[r + 1]] = p.view(R, na, int(jb[r + 1] - jb[r]))
+        cov_all = cov_blk.view(R, na * nb)
+        if pos is not None:
+            cov_all = cov_all[:, to_device(pos, dev, np.int64)]
+        i1_d, i2_d = to_device(idx1, dev, np.int64), to_device(idx2, dev, np.int64)
+        var_d = to_device(var_all, dev, np.float64)
+        for r, g in enumerate(groups):
+            out[g] = _block_group_arrays(cov_all[r], var_d[:, r].contiguous(), idx1, idx2, i1_d, i2_d)
+        st.last_2d_plan = {"imports": [int(i.size) for i in imports], "import_bytes": m["import_bytes"],
+                           "import_ms": m["import_ms"]}
+        return out
+    plan = plan_sharded_pairs(idx1, idx2, bounds, dedup=False)
+    m = _seg_2d(st, gm, plan["imports"])
+    mine = plan["pairs"][me]
+    a, b = m["row"][idx1[mine]], m["row"][idx2[mine]]
+    cov_mine = np.empty((mine.size, R))
+    if mine.size:
+        prod = m["seg"].pair_products(to_device(a, dev, np.int32), to_device(b, dev, np.int32), st.inv_sf_sorted,
+                                      st.timer).cpu().numpy()                                # (pairs, R)
+        sums = m["sums"].cpu().numpy()
+        same = a == b
+        for r in range(R):                      # as the unsharded per-pair path
+            p = prod[:, r] / n_cells[r]
+            p[same] = p[same] - (1 - q[r]) * sums[3][a[same], r] / n_cells[r]             # estimator.py:229-230
+            cov_mine[:, r] = p - (sums[2][a, r] / n_cells[r]) * (sums[2][b, r] / n_cells[r])  # :231
+    gathered = dist.all_gather_known(cov_mine, [p.size for p in plan["pairs"]])
+    cov_all = np.empty((idx1.size, R))
+    cov_all[np.concatenate(plan["pairs"])] = gathered
+    for r, g in enumerate(groups):
+        cov = np.ascontiguousarray(cov_all[:, r])
+        var_1, var_2 = var_all[idx1, r], var_all[idx2, r]
+        out[g] = {"cov": cov, "corr": _corr_from_cov(cov, var_1, var_2), "var_1": var_1, "var_2": var_2}
+    st.last_2d_plan = {"imports": [int(i.size) for i in plan["imports"]], "import_bytes": m["import_bytes"],
+                       "import_ms": m["import_ms"]}
+    return out
+
+
+def _ht_2d_sharded(adata, cov, tr, num_boot, seed, approx, one_sample, resample_rep, workspace_bytes, bootstrap):
+    """ht_2d_moments in a gene-sharded run (see the section comment): every rank tests the unique pairs whose second
+    gene it holds; the results are all-gathered and fanned out to the duplicates on every rank."""
+    mem = adata.uns["memento"]
+    st = _state(adata)
+    dist, me = st.dist, st.dist.rank
+    groups = mem["groups"]
+    R = len(groups)
+    dev = st.device
+    gm = _gene_map(st, adata.var.index)
+    bounds = gm["bounds"]
+    idx1, idx2 = mem["2d_moments"]["gene_idx_1"], mem["2d_moments"]["gene_idx_2"]
+    n_all = idx1.shape[0]
+    block = _as_dense_block(idx1, idx2) if bootstrap == "shared" else None
+    if bootstrap == "shared":
+        if resample_rep:
+            raise NotImplementedError("bootstrap='shared' does not combine with resample_rep")
+        if block is None:
+            raise ValueError("bootstrap='shared' needs gene_pairs that form a full block A x B of at least %d pairs"
+                             % DENSE_BLOCK_MIN_PAIRS)
+        owner, uniq = _first_unordered_block(*block)
+        jb, imports = _block_share(block[0], block[1], bounds)
+    else:
+        plan = plan_sharded_pairs(idx1, idx2, bounds)
+        owner, uniq, imports = plan["owner"], plan["uniq"], plan["imports"]
+    m = _seg_2d(st, gm, imports)
+    q = [mem["group_q"][g] for g in groups]
+    shared_done = None
+    if bootstrap == "shared":
+        genes_a, genes_b, pos = block
+        na, nb = genes_a.size, genes_b.size
+        own_b = genes_b[jb[me]:jb[me + 1]]
+        tc_all = _stacked_corr(mem, groups, dev)                                             # (n_all, R)
+        pos_blk = np.arange(n_all) if pos is None else pos
+        if pos is None:
+            tc_blk = tc_all
+        else:
+            tc_blk = torch.empty_like(tc_all)
+            tc_blk[to_device(pos_blk, dev, np.int64)] = tc_all
+        part = torch.zeros(0, dtype=torch.float64, device=dev)
+        if own_b.size:
+            tc_own = tc_blk.reshape(na, nb, R)[:, jb[me]:jb[me + 1], :].contiguous()
+            res = engine.ht_2d_shared_block(m["seg"], m["row"][genes_a], m["row"][own_b], st.inv_sf_sorted, m["sums"],
+                                            q, tc_own, cov, tr, num_boot, seed, approx, one_sample, timer=st.timer)
+            usable = torch.as_tensor(res["usable"], dtype=torch.float64, device=dev)
+            part = torch.stack([res["coef"], res["se"], res["asl"], usable])
+        sizes = [4 * na * int(jb[r + 1] - jb[r]) for r in range(dist.world)]
+        pieces = dist.all_gather_tensors(part.reshape(-1), sizes)
+        blk = torch.empty((4, na, nb), dtype=torch.float64, device=dev)
+        for r, p in enumerate(pieces):
+            blk[:, :, jb[r]:jb[r + 1]] = p.view(4, na, int(jb[r + 1] - jb[r]))
+        flat = blk.reshape(4, -1).cpu().numpy()[:, pos_blk]
+        shared_done = {"coef": flat[0], "se": flat[1], "asl": flat[2]}
+        shared_ok = flat[3] != 0
+        uniq = uniq[~shared_ok[uniq]]           # the per-pair path below only sees the pairs the block path could not take
+    holder = np.searchsorted(bounds, idx2[uniq], side="right") - 1
+    tests = [uniq[holder == r] for r in range(dist.world)]
+    mine = tests[me]
+    true_corr_d = _stacked_corr(mem, groups, dev)                                          # (n_all, R)
+    res_mine = np.full((mine.size, 3), np.nan)
+    per_item = 8 * (num_boot + 1) * (3 if not approx else 2)
+    pairs_per_tile = int(max(1, min(65535 // R, workspace_bytes // (per_item * R))))
+    stats_acc = {}
+    gid = gm["gid"]
+    for lo in range(0, mine.size, pairs_per_tile):
+        sel = mine[lo:lo + pairs_per_tile]
+        ga, gb = gid[idx1[sel]], gid[idx2[sel]]
+        pid = np.minimum(ga, gb) * (1 << 31) + np.maximum(ga, gb)                        # order-free stream id
+        true_corr = true_corr_d[to_device(sel, dev, np.int64)].cpu().numpy()
+        res = engine.ht_2d_tile(m["seg"], st.design, st.cell_bin, m["row"][idx1[sel]], m["row"][idx2[sel]], true_corr,
+                                cov, tr, num_boot, seed, approx, one_sample, want_coef_rows=not approx,
+                                pair_id=to_device(pid, dev, np.int64), timer=st.timer, stats=stats_acc,
+                                resample_rep=resample_rep)
+        if not approx:
+            gev.refine_tail_asl(res, dev, st.timer, stats_acc)
+        for j, k in enumerate(("coef", "se", "asl")):
+            res_mine[lo:lo + sel.size, j] = res[k].cpu().numpy()[:, 0, 0]
+    gev.count_tail_tests(stats_acc)
+    gathered = dist.all_gather_known(res_mine, [t.size for t in tests])
+    out = {k: np.full(n_all, np.nan) for k in ("coef", "se", "asl")}
+    order = np.concatenate(tests)
+    for j, k in enumerate(("coef", "se", "asl")):
+        out[k][order] = gathered[:, j]
+    dup = owner >= 0
+    for k in out:
+        out[k][dup] = out[k][owner[dup]]
+    if shared_done is not None:
+        for k in out:
+            out[k][shared_ok] = shared_done[k][shared_ok]
+    st.last_stats = stats_acc
+    return out
