@@ -143,6 +143,25 @@ class DistContext:
         tdist.barrier(group=self.group)
 
 
+class OneRank:
+    """The context of an unsharded run, which is the one-rank case of a gene-sharded one: the 2D calls run their
+    sharded code with it (main.compute_2d_moments, main.ht_2d_moments), and every gather returns its input without
+    torch.distributed."""
+    rank, world = 0, 1
+
+    def all_gather_concat(self, a, axis=0):
+        return a, [np.shape(a)[axis]]
+
+    def all_gather_known(self, a, sizes):
+        return a
+
+    def all_gather_objects(self, obj):
+        return [obj]
+
+
+ONE_RANK = OneRank()
+
+
 def shard_plan(work_per_gene, world):
     """Contiguous gene blocks with balanced work: boundaries at the world-quantiles of the cumulative
     work.  Returns int64 array of world + 1 offsets."""

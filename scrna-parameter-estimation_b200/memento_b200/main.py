@@ -20,6 +20,7 @@ import torch
 
 from . import _lib, engine, gev
 from .device import NULL_TIMER, CsrOnDevice, SegMatrix, StageTimer, require_cuda, to_device
+from .dist import ONE_RANK
 
 ESTIMATORS = {"hyper_relative": 0, "mean_only": 1}
 _UNDEFINED_IN_REFERENCE = ("hyper_absolute", "poi_absolute", "poi_relative")  # NameError there too
@@ -55,8 +56,8 @@ class DeviceState:
         self.dist = None         # DistContext when the genes are sharded over ranks
         self.host_profile = None # {section: seconds} when profiling (setup_memento(profile=True))
         self.gene_offset = 0     # global index of this rank's first gene column
-        self.gene_map = None     # gene-sharded runs: all ranks' genes (_gene_map)
-        self.seg2d = None        # gene-sharded runs: this rank's genes + the imported partner genes (_seg_2d)
+        self.gene_map = None     # all ranks' genes (_gene_map; one rank when unsharded)
+        self.seg2d = None        # 2D matrix: this rank's genes + imported partner genes (_seg_2d; seg when unsharded)
 
     def __deepcopy__(self, memo):
         new = DeviceState(self.device)
@@ -69,7 +70,7 @@ class DeviceState:
         if self.host is None:   # the matrix is immutable: stage it once
             self.host = {"seg": self.seg.to_host_pinned(), "cell_bin": self.cell_bin.cpu().pin_memory(),
                          "inv_sf": self.inv_sf_sorted.cpu().pin_memory()}
-        self.seg = self.cell_bin = self.inv_sf_sorted = self.design = self.seg_all = None
+        self.seg = self.cell_bin = self.inv_sf_sorted = self.design = self.seg_all = self.seg2d = None
         self.pending_tail = self.tail_event = None
         self.h2d_bytes = 0
 
@@ -730,51 +731,76 @@ def compute_2d_moments(adata, gene_pairs, inplace=True):
     if "size_factor" not in mem:
         with _Section(st, "compute_1d_moments: bin size factors"):
             _bin_size_factor(adata)
+    dist = st.dist or ONE_RANK
+    me = dist.rank
     groups = mem["groups"]
+    R = len(groups)
+    dev = st.device
+    gm = _gene_map(st, adata.var.index)
+    error = None
+    try:
+        idx1, idx2 = _pair_indices(gm["index"], gene_pairs)
+    except KeyError as exc:
+        if st.dist is None:
+            raise
+        error, idx1, idx2 = exc, np.zeros(0, dtype=int), np.zeros(0, dtype=int)
     if st.dist is not None:
-        mem["2d_moments"] = _compute_2d_sharded(adata, gene_pairs)
-        return adata if not inplace else None
-    idx1, idx2 = _pair_indices(adata.var.index, gene_pairs)
+        _check_same_on_all_ranks(st, "compute_2d_moments", [idx1, idx2], error)
     out = {"gene_pairs": gene_pairs, "gene_idx_1": idx1, "gene_idx_2": idx2}
+    var_all = _gathered_var(st, gm, mem, groups)
     n_cells = np.diff(st.group_start).astype(np.float64)
-    sums_d = st.seg.moments(st.inv_sf_sorted, st.timer)                                     # (5, G, R) on the device
-    sums = sums_d.cpu().numpy()
-    same = idx1 == idx2
+    q = [mem["group_q"][g] for g in groups]
     block = _as_dense_block(idx1, idx2)
     if block is not None:
-        # gene_pairs is a full A x B block: one tensor-core GEMM per group instead of a merge join per pair
+        # gene_pairs is a full A x B block: one tensor-core GEMM per group instead of a merge join per pair; this rank's
+        # share is A x (B on this rank)
         genes_a, genes_b, pos = block
-        cross = st.seg.block_cross(genes_a, genes_b, st.inv_sf_sorted, sums_d, timer=st.timer)    # (R, |A|, |B|) view
-        pos_d = None if pos is None else to_device(pos, st.device, np.int64)
-    else:
-        i1_d = to_device(idx1, st.device, np.int32)
-        i2_d = to_device(idx2, st.device, np.int32)
-        prod = st.seg.pair_products(i1_d, i2_d, st.inv_sf_sorted, st.timer).cpu().numpy()  # (n_pairs, R)
-    if block is not None:
+        jb, imports = _block_share(genes_a, genes_b, gm["bounds"])
+        m = _seg_2d(st, gm, imports)
+        own_b = genes_b[jb[me]:jb[me + 1]]
+        part = [torch.zeros((genes_a.size, 0), dtype=torch.float64, device=dev)] * R
+        if own_b.size:
+            ra = m["row"][genes_a]
+            sums_d = m["seg"].moments(st.inv_sf_sorted, st.timer)                            # (5, G, R) on the device
+            cross = m["seg"].block_cross(ra, m["row"][own_b], st.inv_sf_sorted, sums_d, timer=st.timer)
+            same_d = to_device(genes_a[:, None] == own_b[None, :], dev)
+            s3_d = sums_d[3][to_device(ra, dev, np.int64)]                                  # (|A|, R)
+            for r in range(R):
+                c = cross[r] / n_cells[r]                                         # centred: :226-231 in one step
+                corr_same = ((1 - q[r]) * s3_d[:, r] / n_cells[r])[:, None]               # estimator.py:229-230
+                part[r] = torch.where(same_d, c - corr_same, c)
+            del cross
         # covariance, correlation and the two variance vectors of every group on the device (element-wise glue over
         # R x n_pairs values: 16 x 11 M for the configs[2] block), one read-back per array
-        dev = st.device
-        same_d = to_device(same, dev)
+        cov_blk = _gather_block(dist, part, jb, dev)
+        pos_d = None if pos is None else to_device(pos, dev, np.int64)
         i1_d, i2_d = to_device(idx1, dev, np.int64), to_device(idx2, dev, np.int64)
-        s3_d = sums_d[3]
         for r, g in enumerate(groups):
-            q = mem["group_q"][g]
-            cov_d = (cross[r] / n_cells[r]).reshape(-1)                                    # centred: :226-231 in one step
-            if pos_d is not None:
-                cov_d = cov_d[pos_d]
-            corr_same = (1 - q) * s3_d[i1_d, r] / n_cells[r]                               # estimator.py:229-230
-            cov_d = torch.where(same_d, cov_d - corr_same, cov_d)
-            out[g] = _block_group_arrays(cov_d, to_device(mem["1d_moments"][g][1], dev, np.float64), idx1, idx2,
-                                         i1_d, i2_d)
+            cov_d = cov_blk[r].reshape(-1) if pos_d is None else cov_blk[r].reshape(-1)[pos_d]
+            out[g] = _block_group_arrays(cov_d, to_device(var_all[:, r], dev, np.float64), idx1, idx2, i1_d, i2_d)
     else:
+        plan = plan_sharded_pairs(idx1, idx2, gm["bounds"], dedup=False)
+        imports = plan["imports"]
+        m = _seg_2d(st, gm, imports)
+        mine = plan["pairs"][me]
+        a, b = m["row"][idx1[mine]], m["row"][idx2[mine]]
+        cov_mine = np.empty((mine.size, R))
+        if mine.size:
+            sums = m["seg"].moments(st.inv_sf_sorted, st.timer).cpu().numpy()
+            prod = m["seg"].pair_products(to_device(a, dev, np.int32), to_device(b, dev, np.int32), st.inv_sf_sorted,
+                                          st.timer).cpu().numpy()                                # (pairs, R)
+            same = a == b
+            for r in range(R):
+                p = prod[:, r] / n_cells[r]
+                p[same] = p[same] - (1 - q[r]) * sums[3][a[same], r] / n_cells[r]         # estimator.py:229-230
+                cov_mine[:, r] = p - (sums[2][a, r] / n_cells[r]) * (sums[2][b, r] / n_cells[r])  # :231
+        cov_all = _gather_pairs(dist, cov_mine, plan["pairs"], idx1.size)
         for r, g in enumerate(groups):
-            q = mem["group_q"][g]
-            p = prod[:, r] / n_cells[r]
-            p[same] = p[same] - (1 - q) * sums[3][idx1[same], r] / n_cells[r]             # estimator.py:229-230
-            cov = p - (sums[2][idx1, r] / n_cells[r]) * (sums[2][idx2, r] / n_cells[r])    # :231
-            var_1 = mem["1d_moments"][g][1][idx1]
-            var_2 = mem["1d_moments"][g][1][idx2]
+            cov = np.ascontiguousarray(cov_all[:, r])
+            var_1, var_2 = var_all[idx1, r], var_all[idx2, r]
             out[g] = {"cov": cov, "corr": _corr_from_cov(cov, var_1, var_2), "var_1": var_1, "var_2": var_2}
+    st.last_2d_plan = {"imports": [int(i.size) for i in imports], "import_bytes": m["import_bytes"],
+                       "import_ms": m["import_ms"]}
     mem["2d_moments"] = out
     if not inplace:
         return adata
@@ -1014,62 +1040,78 @@ def ht_2d_moments(adata, covariate, treatment, treatment_for_gene=None, inplace=
     n_all = idx1.shape[0]
     if bootstrap not in ("pair", "shared"):
         raise ValueError("bootstrap must be 'pair' or 'shared'")
+    dist = st.dist or ONE_RANK
+    me = dist.rank
     if st.dist is not None:
         _check_same_on_all_ranks(st, "ht_2d_moments", [
             idx1, idx2, cov, tr, list(covariate.columns), list(treatment.columns), list(covariate.index),
             list(treatment.index), num_boot, seed, approx, resample_rep, bootstrap])
-        out = _ht_2d_sharded(adata, cov, tr, num_boot, seed, approx, one_sample, resample_rep, workspace_bytes,
-                             bootstrap)
-        mem["2d_ht"] = {"treatment": treatment, "covariate": covariate, "corr_coef": out["coef"],
-                        "corr_se": out["se"], "corr_asl": out["asl"]}
-        return adata if not inplace else None
+    dev = st.device
+    gm = _gene_map(st, adata.var.index)
+    # every rank tests the unique pairs whose second gene it holds; unordered de-duplication, first occurrence computes
+    # (main.py:467-482)
     block = _as_dense_block(idx1, idx2) if bootstrap == "shared" else None
-    # unordered de-duplication, first occurrence computes (main.py:467-482)
-    owner, uniq = _first_unordered(idx1, idx2) if block is None else _first_unordered_block(*block)
-    shared_done = None
     if bootstrap == "shared":
         if resample_rep:
             raise NotImplementedError("bootstrap='shared' does not combine with resample_rep")
         if block is None:
             raise ValueError("bootstrap='shared' needs gene_pairs that form a full block A x B of at least %d pairs"
                              % DENSE_BLOCK_MIN_PAIRS)
+        owner, uniq = _first_unordered_block(*block)
+        jb, imports = _block_share(block[0], block[1], gm["bounds"])
+    else:
+        plan = plan_sharded_pairs(idx1, idx2, gm["bounds"])
+        owner, uniq, imports = plan["owner"], plan["uniq"], plan["imports"]
+    m = _seg_2d(st, gm, imports)
+    q = [mem["group_q"][g] for g in groups]
+    true_corr_d = _stacked_corr(mem, groups, dev)                                          # (n_all, R) on the device
+    shared_done = None
+    if bootstrap == "shared":
         genes_a, genes_b, pos = block
-        tc_all = _stacked_corr(mem, groups, st.device)                                   # (n_all, R) on the device
+        na, nb = genes_a.size, genes_b.size
+        own_b = genes_b[jb[me]:jb[me + 1]]
         pos_blk = np.arange(n_all) if pos is None else pos
         if pos is None:
-            tc_blk = tc_all
+            tc_blk = true_corr_d
         else:
-            tc_blk = torch.empty_like(tc_all)
-            tc_blk[to_device(pos_blk, st.device, np.int64)] = tc_all
-        sums_d = st.seg.moments(st.inv_sf_sorted, st.timer)
-        res = engine.ht_2d_shared_block(st.seg, genes_a, genes_b, st.inv_sf_sorted, sums_d,
-                                        [mem["group_q"][g] for g in groups],
-                                        tc_blk.reshape(genes_a.size, genes_b.size, R), cov, tr, num_boot, seed, approx,
-                                        one_sample, timer=st.timer)
-        shared_done = {k: res[k].reshape(-1).cpu().numpy()[pos_blk] for k in ("coef", "se", "asl")}
-        shared_ok = res["usable"].reshape(-1)[pos_blk]
-        # the per-pair path below only sees the pairs the block path could not take
-        uniq = uniq[~shared_ok[uniq]]
-    true_corr_d = _stacked_corr(mem, groups, st.device)                                  # (n_all, R) on the device
-    out = {k: np.full(n_all, np.nan) for k in ("coef", "se", "asl")}
+            tc_blk = torch.empty_like(true_corr_d)
+            tc_blk[to_device(pos_blk, dev, np.int64)] = true_corr_d
+        part = [torch.zeros((na, 0), dtype=torch.float64, device=dev)] * 4
+        if own_b.size:
+            tc_own = tc_blk.reshape(na, nb, R)[:, jb[me]:jb[me + 1], :].contiguous()
+            sums_d = m["seg"].moments(st.inv_sf_sorted, st.timer)
+            res = engine.ht_2d_shared_block(m["seg"], m["row"][genes_a], m["row"][own_b], st.inv_sf_sorted, sums_d,
+                                            q, tc_own, cov, tr, num_boot, seed, approx, one_sample, timer=st.timer)
+            part = [res["coef"], res["se"], res["asl"], res["usable"]]
+        flat = [(t.cpu().numpy() if torch.is_tensor(t) else t).reshape(-1)[pos_blk]
+                for t in _gather_block(dist, part, jb, dev)]
+        shared_done = dict(zip(("coef", "se", "asl"), flat))
+        shared_ok = flat[3] != 0
+        uniq = uniq[~shared_ok[uniq]]       # the per-pair path below only sees the pairs the block path could not take
+    holder = np.searchsorted(gm["bounds"], idx2[uniq], side="right") - 1
+    tests = [uniq[holder == r] for r in range(dist.world)]
+    mine = tests[me]
+    res_mine = np.full((mine.size, 3), np.nan)
     per_item = 8 * (num_boot + 1) * (3 if not approx else 2)
     pairs_per_tile = int(max(1, min(65535 // R, workspace_bytes // (per_item * R))))
     stats_acc = {}
-    G = adata.shape[1]
-    for lo in range(0, uniq.shape[0], pairs_per_tile):
-        sel = uniq[lo:lo + pairs_per_tile]
-        a, b = idx1[sel].astype(np.int64), idx2[sel].astype(np.int64)
-        ga, gb = st.gene_index[a] + st.gene_offset, st.gene_index[b] + st.gene_offset
+    gid = gm["gid"]
+    for lo in range(0, mine.size, pairs_per_tile):
+        sel = mine[lo:lo + pairs_per_tile]
+        ga, gb = gid[idx1[sel]], gid[idx2[sel]]
         pid = np.minimum(ga, gb) * (1 << 31) + np.maximum(ga, gb)                        # order-free stream id
-        pair_id = to_device(pid, st.device, np.int64)
-        true_corr = true_corr_d[to_device(sel, st.device, np.int64)].cpu().numpy()
-        res = engine.ht_2d_tile(st.seg, st.design, st.cell_bin, a, b, true_corr, cov, tr, num_boot, seed, approx,
-                                one_sample, want_coef_rows=not approx, pair_id=pair_id, timer=st.timer,
-                                stats=stats_acc, resample_rep=resample_rep)
+        true_corr = true_corr_d[to_device(sel, dev, np.int64)].cpu().numpy()
+        res = engine.ht_2d_tile(m["seg"], st.design, st.cell_bin, m["row"][idx1[sel]], m["row"][idx2[sel]], true_corr,
+                                cov, tr, num_boot, seed, approx, one_sample, want_coef_rows=not approx,
+                                pair_id=to_device(pid, dev, np.int64), timer=st.timer, stats=stats_acc,
+                                resample_rep=resample_rep)
         if not approx:
-            gev.refine_tail_asl(res, st.device, st.timer, stats_acc)
-        for k in out:
-            out[k][sel] = res[k].cpu().numpy()[:, 0, 0]
+            gev.refine_tail_asl(res, dev, st.timer, stats_acc)
+        for j, k in enumerate(("coef", "se", "asl")):
+            res_mine[lo:lo + sel.size, j] = res[k].cpu().numpy()[:, 0, 0]
+    gev.count_tail_tests(stats_acc)
+    res_all = _gather_pairs(dist, res_mine, tests, n_all)
+    out = {k: np.ascontiguousarray(res_all[:, j]) for j, k in enumerate(("coef", "se", "asl"))}
     dup = owner >= 0
     for k in out:
         out[k][dup] = out[k][owner[dup]]
@@ -1083,12 +1125,14 @@ def ht_2d_moments(adata, covariate, treatment, treatment_for_gene=None, inplace=
         return adata
 
 
-# --------------------------------------------------------------------------- 2D in a gene-sharded run
-# compute_2d_moments and ht_2d_moments are collective calls there: every rank passes the same pairs (global gene names)
-# and arguments and ends with the same full-length arrays, in the caller's pair order, that the unsharded run produces.
-# A pair is computed by the rank holding its SECOND gene; the columns of the first genes that live on other ranks are
-# imported once per pair set (_seg_2d).  Global position of a gene = its index in the rank blocks concatenated (the
-# unsharded run's adata.var order); global id = its original column plus the rank's gene_offset (the RNG stream id).
+# --------------------------------------------------------------------------- 2D and gene sharding
+# compute_2d_moments and ht_2d_moments are collective calls in a gene-sharded run: every rank passes the same pairs
+# (global gene names) and arguments and ends with the same full-length arrays, in the caller's pair order, that the
+# unsharded run produces.  A pair is computed by the rank holding its SECOND gene; the columns of the first genes that
+# live on other ranks are imported once per pair set (_seg_2d).  Global position of a gene = its index in the rank
+# blocks concatenated (the unsharded run's adata.var order); global id = its original column plus the rank's
+# gene_offset (the RNG stream id).  An unsharded run is the one-rank case (dist.ONE_RANK): rank 0 holds every gene,
+# computes every pair and imports nothing, and its gathers return their input.
 
 def _gene_map(st, names_local):
     """The genes of all ranks, from one all-gather per gene set (create_groups and compute_1d_moments drop it):
@@ -1099,11 +1143,13 @@ def _gene_map(st, names_local):
     if gm is None:
         gid = getattr(st, "gene_index", None)
         gid = None if gid is None else np.asarray(gid, dtype=np.int64) + st.gene_offset
-        parts = st.dist.all_gather_objects((list(names_local), gid))
-        names = [n for p, _ in parts for n in p]
+        dist = st.dist or ONE_RANK
+        # pd.Index objects, not lists: element-wise iteration of a string index costs ms per 10k genes
+        parts = dist.all_gather_objects((pd.Index(names_local), gid))
+        index = parts[0][0].append([p for p, _ in parts[1:]])
         bounds = np.concatenate([[0], np.cumsum([len(p) for p, _ in parts])]).astype(np.int64)
-        gm = st.gene_map = {"names": names, "index": pd.Index(names), "bounds": bounds,
-                            "lo": int(bounds[st.dist.rank]), "tests": {},
+        gm = st.gene_map = {"names": index.tolist(), "index": index, "bounds": bounds,
+                            "lo": int(bounds[dist.rank]), "tests": {},
                             "gid": None if gid is None else np.concatenate([g for _, g in parts])}
     return gm
 
@@ -1179,13 +1225,14 @@ def _concat_seg(parts, n_cells, group_start):
 
 
 def _seg_2d(st, gm, imports):
-    """This rank's 2D matrix: its own genes followed by the genes ``imports[st.dist.rank]`` held by other ranks
-    (``imports``: sorted global positions, one list per rank, identical on every rank).  Collective: every rank sends
-    the genes any other rank imports from it as one device buffer [R segment lengths per gene (int64) | vals (float32)
-    | rows (int32)]; a gene's R segments are one contiguous range of the group-sorted CSC.  Cached on the state
-    (create_groups and compute_1d_moments drop it).  Returns {"seg", "row" (row of every global position, -1 when
-    absent), "sums" (device moment sums of the matrix), "import_bytes", "import_ms"}."""
-    dist, me = st.dist, st.dist.rank
+    """This rank's 2D matrix: its own genes followed by the genes ``imports[rank]`` held by other ranks (``imports``:
+    sorted global positions, one list per rank, identical on every rank).  Collective unless nothing is imported (one
+    rank: the matrix is ``st.seg``): every rank sends the genes any other rank imports from it as one device buffer
+    [R segment lengths per gene (int64) | vals (float32) | rows (int32)]; a gene's R segments are one contiguous range
+    of the group-sorted CSC.  Cached on the state (create_groups, compute_1d_moments and offload drop it).  Returns
+    {"seg", "row" (row of every global position, -1 when absent), "import_bytes", "import_ms"}."""
+    dist = st.dist or ONE_RANK
+    me = dist.rank
     key = (id(st.seg), tuple(hashlib.blake2b(np.ascontiguousarray(i).tobytes()).hexdigest() for i in imports))
     if st.seg2d is not None and st.seg2d["key"] == key:
         return st.seg2d
@@ -1237,9 +1284,8 @@ def _seg_2d(st, gm, imports):
             got = got.select_genes(np.searchsorted(sent[s], take))
             parts.append((got.vals, got.rows, got.seg_ptr))
         mat = seg if len(parts) == 1 else _concat_seg(parts, seg.n_cells, seg.group_start_host)
-    sums = mat.moments(st.inv_sf_sorted, st.timer)
-    torch.cuda.synchronize(st.device)
-    st.seg2d = {"key": key, "seg": mat, "row": row, "sums": sums, "import_bytes": nbytes,
+        torch.cuda.synchronize(st.device)
+    st.seg2d = {"key": key, "seg": mat, "row": row, "import_bytes": nbytes,
                 "import_ms": (time.perf_counter() - t0) * 1e3}
     return st.seg2d
 
@@ -1248,178 +1294,29 @@ def _gathered_var(st, gm, mem, groups):
     """(G_global, R) per-group variances (``1d_moments``) of all ranks' genes, all-gathered once per gene set."""
     if gm.get("var") is None:
         local = np.stack([mem["1d_moments"][g][1] for g in groups], axis=1)
-        gm["var"] = st.dist.all_gather_concat(local)[0]
+        gm["var"] = (st.dist or ONE_RANK).all_gather_concat(local)[0]
     return gm["var"]
 
 
-def _compute_2d_sharded(adata, gene_pairs):
-    """compute_2d_moments in a gene-sharded run (see the section comment)."""
-    mem = adata.uns["memento"]
-    st = _state(adata)
-    dist, me = st.dist, st.dist.rank
-    groups = mem["groups"]
-    R = len(groups)
-    dev = st.device
-    gm = _gene_map(st, adata.var.index)
-    error = None
-    try:
-        idx1, idx2 = _pair_indices(gm["index"], gene_pairs)
-    except KeyError as exc:
-        error, idx1, idx2 = exc, np.zeros(0, dtype=int), np.zeros(0, dtype=int)
-    _check_same_on_all_ranks(st, "compute_2d_moments", [idx1, idx2], error)
-    out = {"gene_pairs": gene_pairs, "gene_idx_1": idx1, "gene_idx_2": idx2}
-    var_all = _gathered_var(st, gm, mem, groups)
-    bounds = gm["bounds"]
-    n_cells = np.diff(st.group_start).astype(np.float64)
-    q = [mem["group_q"][g] for g in groups]
-    block = _as_dense_block(idx1, idx2)
-    if block is not None:
-        # this rank's share is A x (B on this rank): one tensor-core GEMM per group on the 2D matrix
-        genes_a, genes_b, pos = block
-        na, nb = genes_a.size, genes_b.size
-        jb, imports = _block_share(genes_a, genes_b, bounds)
-        m = _seg_2d(st, gm, imports)
-        own_b = genes_b[jb[me]:jb[me + 1]]
-        part = torch.zeros(0, dtype=torch.float64, device=dev)
-        if own_b.size:
-            ra = m["row"][genes_a]
-            cross = m["seg"].block_cross(ra, m["row"][own_b], st.inv_sf_sorted, m["sums"], timer=st.timer)
-            same_d = to_device(genes_a[:, None] == own_b[None, :], dev)
-            s3_d = m["sums"][3][to_device(ra, dev, np.int64)]                                # (|A|, R)
-            part = torch.empty((R, na, own_b.size), dtype=torch.float64, device=dev)
-            for r in range(R):
-                c = cross[r] / n_cells[r]
-                corr_same = ((1 - q[r]) * s3_d[:, r] / n_cells[r])[:, None]               # estimator.py:229-230
-                part[r] = torch.where(same_d, c - corr_same, c)
-        sizes = [R * na * int(jb[r + 1] - jb[r]) for r in range(dist.world)]
-        pieces = dist.all_gather_tensors(part.reshape(-1), sizes)
-        cov_blk = torch.empty((R, na, nb), dtype=torch.float64, device=dev)
-        for r, p in enumerate(pieces):
-            cov_blk[:, :, jb[r]:jb[r + 1]] = p.view(R, na, int(jb[r + 1] - jb[r]))
-        cov_all = cov_blk.view(R, na * nb)
-        if pos is not None:
-            cov_all = cov_all[:, to_device(pos, dev, np.int64)]
-        i1_d, i2_d = to_device(idx1, dev, np.int64), to_device(idx2, dev, np.int64)
-        var_d = to_device(var_all, dev, np.float64)
-        for r, g in enumerate(groups):
-            out[g] = _block_group_arrays(cov_all[r], var_d[:, r].contiguous(), idx1, idx2, i1_d, i2_d)
-        st.last_2d_plan = {"imports": [int(i.size) for i in imports], "import_bytes": m["import_bytes"],
-                           "import_ms": m["import_ms"]}
-        return out
-    plan = plan_sharded_pairs(idx1, idx2, bounds, dedup=False)
-    m = _seg_2d(st, gm, plan["imports"])
-    mine = plan["pairs"][me]
-    a, b = m["row"][idx1[mine]], m["row"][idx2[mine]]
-    cov_mine = np.empty((mine.size, R))
-    if mine.size:
-        prod = m["seg"].pair_products(to_device(a, dev, np.int32), to_device(b, dev, np.int32), st.inv_sf_sorted,
-                                      st.timer).cpu().numpy()                                # (pairs, R)
-        sums = m["sums"].cpu().numpy()
-        same = a == b
-        for r in range(R):                      # as the unsharded per-pair path
-            p = prod[:, r] / n_cells[r]
-            p[same] = p[same] - (1 - q[r]) * sums[3][a[same], r] / n_cells[r]             # estimator.py:229-230
-            cov_mine[:, r] = p - (sums[2][a, r] / n_cells[r]) * (sums[2][b, r] / n_cells[r])  # :231
-    gathered = dist.all_gather_known(cov_mine, [p.size for p in plan["pairs"]])
-    cov_all = np.empty((idx1.size, R))
-    cov_all[np.concatenate(plan["pairs"])] = gathered
-    for r, g in enumerate(groups):
-        cov = np.ascontiguousarray(cov_all[:, r])
-        var_1, var_2 = var_all[idx1, r], var_all[idx2, r]
-        out[g] = {"cov": cov, "corr": _corr_from_cov(cov, var_1, var_2), "var_1": var_1, "var_2": var_2}
-    st.last_2d_plan = {"imports": [int(i.size) for i in plan["imports"]], "import_bytes": m["import_bytes"],
-                       "import_ms": m["import_ms"]}
-    return out
+def _gather_block(dist, parts, jb, device):
+    """K blocks A x B from every rank's columns A x genes_b[jb[r]:jb[r + 1]] of them (_block_share).  ``parts``: this
+    rank's columns of the K blocks, (|A|, jb[rank + 1] - jb[rank]) device tensors or numpy arrays.  Returns the
+    (K, |A|, |B|) float64 device tensor of the full blocks, from ONE all-gather.  With one rank the columns are the
+    blocks, and ``parts`` comes back as it is: nothing is copied."""
+    if dist.world == 1:
+        return parts
+    K, na = len(parts), parts[0].shape[0]
+    part = torch.stack([torch.as_tensor(p, dtype=torch.float64, device=device) for p in parts])
+    pieces = dist.all_gather_tensors(part.reshape(-1), [K * na * int(jb[r + 1] - jb[r]) for r in range(dist.world)])
+    blk = torch.empty((K, na, int(jb[-1])), dtype=torch.float64, device=device)
+    for r, p in enumerate(pieces):
+        blk[:, :, jb[r]:jb[r + 1]] = p.view(K, na, int(jb[r + 1] - jb[r]))
+    return blk
 
 
-def _ht_2d_sharded(adata, cov, tr, num_boot, seed, approx, one_sample, resample_rep, workspace_bytes, bootstrap):
-    """ht_2d_moments in a gene-sharded run (see the section comment): every rank tests the unique pairs whose second
-    gene it holds; the results are all-gathered and fanned out to the duplicates on every rank."""
-    mem = adata.uns["memento"]
-    st = _state(adata)
-    dist, me = st.dist, st.dist.rank
-    groups = mem["groups"]
-    R = len(groups)
-    dev = st.device
-    gm = _gene_map(st, adata.var.index)
-    bounds = gm["bounds"]
-    idx1, idx2 = mem["2d_moments"]["gene_idx_1"], mem["2d_moments"]["gene_idx_2"]
-    n_all = idx1.shape[0]
-    block = _as_dense_block(idx1, idx2) if bootstrap == "shared" else None
-    if bootstrap == "shared":
-        if resample_rep:
-            raise NotImplementedError("bootstrap='shared' does not combine with resample_rep")
-        if block is None:
-            raise ValueError("bootstrap='shared' needs gene_pairs that form a full block A x B of at least %d pairs"
-                             % DENSE_BLOCK_MIN_PAIRS)
-        owner, uniq = _first_unordered_block(*block)
-        jb, imports = _block_share(block[0], block[1], bounds)
-    else:
-        plan = plan_sharded_pairs(idx1, idx2, bounds)
-        owner, uniq, imports = plan["owner"], plan["uniq"], plan["imports"]
-    m = _seg_2d(st, gm, imports)
-    q = [mem["group_q"][g] for g in groups]
-    shared_done = None
-    if bootstrap == "shared":
-        genes_a, genes_b, pos = block
-        na, nb = genes_a.size, genes_b.size
-        own_b = genes_b[jb[me]:jb[me + 1]]
-        tc_all = _stacked_corr(mem, groups, dev)                                             # (n_all, R)
-        pos_blk = np.arange(n_all) if pos is None else pos
-        if pos is None:
-            tc_blk = tc_all
-        else:
-            tc_blk = torch.empty_like(tc_all)
-            tc_blk[to_device(pos_blk, dev, np.int64)] = tc_all
-        part = torch.zeros(0, dtype=torch.float64, device=dev)
-        if own_b.size:
-            tc_own = tc_blk.reshape(na, nb, R)[:, jb[me]:jb[me + 1], :].contiguous()
-            res = engine.ht_2d_shared_block(m["seg"], m["row"][genes_a], m["row"][own_b], st.inv_sf_sorted, m["sums"],
-                                            q, tc_own, cov, tr, num_boot, seed, approx, one_sample, timer=st.timer)
-            usable = torch.as_tensor(res["usable"], dtype=torch.float64, device=dev)
-            part = torch.stack([res["coef"], res["se"], res["asl"], usable])
-        sizes = [4 * na * int(jb[r + 1] - jb[r]) for r in range(dist.world)]
-        pieces = dist.all_gather_tensors(part.reshape(-1), sizes)
-        blk = torch.empty((4, na, nb), dtype=torch.float64, device=dev)
-        for r, p in enumerate(pieces):
-            blk[:, :, jb[r]:jb[r + 1]] = p.view(4, na, int(jb[r + 1] - jb[r]))
-        flat = blk.reshape(4, -1).cpu().numpy()[:, pos_blk]
-        shared_done = {"coef": flat[0], "se": flat[1], "asl": flat[2]}
-        shared_ok = flat[3] != 0
-        uniq = uniq[~shared_ok[uniq]]           # the per-pair path below only sees the pairs the block path could not take
-    holder = np.searchsorted(bounds, idx2[uniq], side="right") - 1
-    tests = [uniq[holder == r] for r in range(dist.world)]
-    mine = tests[me]
-    true_corr_d = _stacked_corr(mem, groups, dev)                                          # (n_all, R)
-    res_mine = np.full((mine.size, 3), np.nan)
-    per_item = 8 * (num_boot + 1) * (3 if not approx else 2)
-    pairs_per_tile = int(max(1, min(65535 // R, workspace_bytes // (per_item * R))))
-    stats_acc = {}
-    gid = gm["gid"]
-    for lo in range(0, mine.size, pairs_per_tile):
-        sel = mine[lo:lo + pairs_per_tile]
-        ga, gb = gid[idx1[sel]], gid[idx2[sel]]
-        pid = np.minimum(ga, gb) * (1 << 31) + np.maximum(ga, gb)                        # order-free stream id
-        true_corr = true_corr_d[to_device(sel, dev, np.int64)].cpu().numpy()
-        res = engine.ht_2d_tile(m["seg"], st.design, st.cell_bin, m["row"][idx1[sel]], m["row"][idx2[sel]], true_corr,
-                                cov, tr, num_boot, seed, approx, one_sample, want_coef_rows=not approx,
-                                pair_id=to_device(pid, dev, np.int64), timer=st.timer, stats=stats_acc,
-                                resample_rep=resample_rep)
-        if not approx:
-            gev.refine_tail_asl(res, dev, st.timer, stats_acc)
-        for j, k in enumerate(("coef", "se", "asl")):
-            res_mine[lo:lo + sel.size, j] = res[k].cpu().numpy()[:, 0, 0]
-    gev.count_tail_tests(stats_acc)
-    gathered = dist.all_gather_known(res_mine, [t.size for t in tests])
-    out = {k: np.full(n_all, np.nan) for k in ("coef", "se", "asl")}
-    order = np.concatenate(tests)
-    for j, k in enumerate(("coef", "se", "asl")):
-        out[k][order] = gathered[:, j]
-    dup = owner >= 0
-    for k in out:
-        out[k][dup] = out[k][owner[dup]]
-    if shared_done is not None:
-        for k in out:
-            out[k][shared_ok] = shared_done[k][shared_ok]
-    st.last_stats = stats_acc
+def _gather_pairs(dist, local, pairs, n):
+    """(n, ...) float64 array of every rank's per-pair results in pair order, NaN for the pairs no rank computed.
+    ``pairs``: the pair indices of every rank; ``local``: this rank's results, one row per pair of ``pairs[rank]``."""
+    out = np.full((n,) + local.shape[1:], np.nan)
+    out[np.concatenate(pairs)] = dist.all_gather_known(local, [p.size for p in pairs])
     return out

@@ -1,9 +1,12 @@
 """Host logic of the gene-sharded 2D path (no GPU): the pair-ownership plan of main.plan_sharded_pairs and its block
-form, and the two exchanges it adds to DistContext, run over gloo with CPU tensors."""
+form, the one-rank context of unsharded runs, and the two exchanges it adds to DistContext, run over gloo with CPU
+tensors."""
 import os
 import socket
+from types import SimpleNamespace
 
 import numpy as np
+import pandas as pd
 import pytest
 import torch
 import torch.distributed as tdist
@@ -68,6 +71,46 @@ def test_block_share_equals_the_plan_of_the_block(world):
             assert np.array_equal(imports[r], plan["imports"][r])
             blk = np.arange(A.size)[:, None] * B.size + np.arange(jb[r], jb[r + 1])[None, :]
             assert np.array_equal(np.sort(blk.reshape(-1)), plan["pairs"][r])
+
+
+def test_one_rank_context_runs_the_world_1_plan_without_exchanges():
+    """An unsharded run is the one-rank case: rank 0 holds every gene, computes every pair, imports nothing, and each
+    gather of mdist.ONE_RANK returns its input (there is no process group here, so a collective would raise)."""
+    ctx = mdist.ONE_RANK
+    assert (ctx.rank, ctx.world) == (0, 1) and not tdist.is_initialized()
+    rng = np.random.default_rng(0)
+    G, n, R = 30, 50, 4
+    st = mmain.DeviceState("cpu")
+    st.gene_index, st.seg = np.arange(G) + 7, SimpleNamespace(G=G, R=R)
+    names = ["g%d" % i for i in range(G)]
+    gm = mmain._gene_map(st, pd.Index(names))
+    assert gm["names"] == names and gm["bounds"].tolist() == [0, G] and gm["lo"] == 0
+    assert np.array_equal(gm["gid"], st.gene_index)
+    mem = {"1d_moments": {g: [None, rng.random(G), None] for g in "abcd"}}
+    var, sizes = ctx.all_gather_concat(np.stack([mem["1d_moments"][g][1] for g in "abcd"], axis=1))
+    assert sizes == [G] and np.array_equal(mmain._gathered_var(st, gm, mem, list("abcd")), var)
+    obj = (names, st.gene_index)
+    assert ctx.all_gather_objects(obj)[0] is obj
+
+    g1, g2 = rng.integers(0, G, n), rng.integers(0, G, n)
+    plan = mmain.plan_sharded_pairs(g1, g2, gm["bounds"])
+    assert np.array_equal(plan["pairs"][0], np.arange(n)) and np.array_equal(plan["tests"][0], plan["uniq"])
+    assert plan["imports"][0].size == 0
+    m = mmain._seg_2d(st, gm, plan["imports"])
+    assert m["seg"] is st.seg and np.array_equal(m["row"], np.arange(G)) and m["import_bytes"] == 0
+    local = rng.random((n, R))
+    assert ctx.all_gather_known(local, [n]) is local
+    assert np.array_equal(mmain._gather_pairs(ctx, local, plan["pairs"], n), local)
+    tests = plan["tests"][0]
+    got = mmain._gather_pairs(ctx, local[:tests.size], plan["tests"], n)
+    assert np.array_equal(got[tests], local[:tests.size]) and np.isnan(np.delete(got, tests, axis=0)).all()
+
+    A, B = np.sort(rng.choice(G, 6, replace=False)), np.arange(G)
+    jb, imports = mmain._block_share(A, B, gm["bounds"])
+    assert jb.tolist() == [0, G] and imports[0].size == 0
+    assert mmain._seg_2d(st, gm, imports) is m          # the same (empty) imports: the cached matrix
+    parts = [torch.ones(A.size, G), np.zeros((A.size, G), dtype=bool)]
+    assert mmain._gather_block(ctx, parts, jb, "cpu") is parts
 
 
 # ----------------------------------------------------------------------------- exchanges over gloo (CPU tensors)

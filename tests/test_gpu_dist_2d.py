@@ -2,7 +2,8 @@
 
 Two configurations: gloo with both ranks on cuda:0 (any single-GPU box) and NCCL on cuda:0 / cuda:1 (skipped with fewer
 than 2 GPUs).  Each rank holds a block of the gene columns; every rank must end with the same full-length arrays, in the
-caller's pair order, that the single run produces."""
+caller's pair order, that the single run produces.  The single run itself is the one-rank case of the same code, and
+must run without torch.distributed."""
 import itertools
 import os
 import socket
@@ -81,9 +82,7 @@ def _run_cases(ad, cases, save):
                                   **kw)
             for k in ("corr_coef", "corr_se", "corr_asl"):
                 save("%s|ht%d|%s" % (name, j, k), np.asarray(mem["2d_ht"][k]))
-            stats = mem["_b200"].last_stats
-            n_gev = stats.get("gev_tests", sum(int((s >= 0).sum().item()) for s in stats.get("_gev_status", [])))
-            save("%s|ht%d|gev_tests" % (name, j), np.asarray(n_gev))
+            save("%s|ht%d|gev_tests" % (name, j), np.asarray(mem["_b200"].last_stats["gev_tests"]))
 
 
 def _cell_weights(st, R):
@@ -219,3 +218,45 @@ def test_sharded_2d_equals_single_gpu(tmp_path, monkeypatch, backend):
         key = "%s|ht%d|gev_tests" % (name, j)
         assert int(single[key]) > 0 or name == "small", key
         assert int(parts[0][key]) + int(parts[1][key]) == int(single[key]), key
+
+
+def test_unsharded_2d_is_the_one_rank_case(monkeypatch):
+    """Without torch.distributed the 2D calls run as one rank: no argument digest and no collective, the 2D matrix is
+    the device matrix itself, and offload() releases it with the other device copies."""
+    import gc
+    import torch.distributed as tdist
+    import memento_b200 as memento
+    from memento_b200 import main as mm_main, synth
+
+    def no_digest(*args, **kwargs):
+        raise AssertionError("argument digest in an unsharded run")
+
+    assert not tdist.is_initialized()
+    monkeypatch.setattr(mm_main, "_check_same_on_all_ranks", no_digest)
+    monkeypatch.setattr(mm_main, "DENSE_BLOCK_MIN_PAIRS", 64)
+    ad = _data()
+    memento.setup_memento(ad, "q")
+    memento.create_groups(ad, ["stim", "cell"])
+    memento.compute_1d_moments(ad, min_perc_group=0.9)
+    names = ad.var.index.tolist()
+    cases = {name: pairs for name, pairs, _ in _cases([names[:len(names) // 2], names[len(names) // 2:]])}
+    mem = ad.uns["memento"]
+    st = mem["_b200"]
+    cov, tr = synth.design_from_groups(mem["groups"], ["stim", "cell"])
+    for name, boots in (("small", ["pair"]), ("block", ["pair", "shared"])):
+        memento.compute_2d_moments(ad, cases[name])
+        assert st.seg2d["seg"] is st.seg and st.last_2d_plan["import_bytes"] == 0, name
+        for boot in boots:
+            memento.ht_2d_moments(ad, cov, tr, num_boot=NUM_BOOT, resampling="bootstrap", seed=SEED, bootstrap=boot,
+                                  approx=boot == "shared")
+            assert np.isfinite(mem["2d_ht"]["corr_asl"]).any(), (name, boot)
+            assert "gev_tests" in st.last_stats, (name, boot)
+    seg = st.seg
+    n_bytes = sum(t.numel() * t.element_size() for t in (seg.vals, seg.rows, seg.seg_ptr))
+    del seg
+    torch.cuda.synchronize()
+    before = torch.cuda.memory_allocated()
+    st.offload()
+    gc.collect()
+    assert st.seg2d is None
+    assert before - torch.cuda.memory_allocated() >= n_bytes
