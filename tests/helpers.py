@@ -44,6 +44,38 @@ def assert_close(a, b, rtol, atol=0.0, what=""):
                                a[ok][np.argmax(err)], b[ok][np.argmax(err)])
 
 
+_MASK32 = np.uint64(0xFFFFFFFF)
+
+
+def philox4x32(c0, c1, c2, c3, seed, rounds):
+    """numpy restatement of Philox4x32 as csrc/common.cuh Philox::rounds (counter words c0..c3, key = the 64-bit
+    seed split into its low / high words).  Arguments broadcast; returns the four output words as uint64 arrays."""
+    M0, M1, W0, W1 = np.uint64(0xD2511F53), np.uint64(0xCD9E8D57), 0x9E3779B9, 0xBB67AE85
+    c = [np.asarray(v, dtype=np.uint64) & _MASK32 for v in (c0, c1, c2, c3)]
+    c = list(np.broadcast_arrays(*c))
+    k0, k1 = int(seed) & 0xFFFFFFFF, (int(seed) >> 32) & 0xFFFFFFFF
+    for _ in range(rounds):
+        p0, p1 = M0 * c[0], M1 * c[2]
+        c = [(p1 >> np.uint64(32)) ^ c[1] ^ np.uint64(k0), p1 & _MASK32,
+             (p0 >> np.uint64(32)) ^ c[3] ^ np.uint64(k1), p0 & _MASK32]
+        k0, k1 = (k0 + W0) & 0xFFFFFFFF, (k1 + W1) & 0xFFFFFFFF
+    return c
+
+
+def cell_weights_host(group_start, seed, replicate):
+    """Host replay of mm_cell_weights (csrc/sharedboot.cu): draw i picks cell g0 + umul64hi(x << 32 | y, n) of its
+    group, (x, y) the first two words of Philox4x32-10 at counter (i lo, i hi, replicate, 0x5B007).  Returns the int64
+    weight vector."""
+    gs = np.asarray(group_start, dtype=np.int64)
+    i = np.arange(gs[-1], dtype=np.int64)
+    grp = np.searchsorted(gs, i, side="right") - 1
+    n = (gs[grp + 1] - gs[grp]).astype(np.uint64)
+    iu = i.astype(np.uint64)
+    x, y, _, _ = philox4x32(iu, iu >> np.uint64(32), replicate, 0x5B007, seed, 10)
+    idx = (x * n + ((y * n) >> np.uint64(32))) >> np.uint64(32)      # high word of the 96-bit (x 2^32 + y) n
+    return np.bincount(gs[grp] + idx.astype(np.int64), minlength=int(gs[-1]))
+
+
 def gev_battery_vector(i):
     """Coefficient row i of the GEV battery (tests/golden/gev_battery.npz): x[0] = statistic, x[1:] = bootstrap
     values around it.  Normal / Student-t(5) / skewed (centred gamma) nulls of 1000-10000 replicates with effects of
