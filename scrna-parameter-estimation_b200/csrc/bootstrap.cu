@@ -469,24 +469,31 @@ bootstrap_1d_poisson_kernel(BootParams P) {
     // dense gene's block runs 10 x the average) start first instead of leaving a tail of a few busy SMs
     const long long seg_rel = P.seg_order ? P.seg_order[blockIdx.y] : blockIdx.y;
     if (P.seg_skip && P.seg_skip[seg_rel]) return;
-    const SegInfo si = P.info[seg_rel];
-    if (si.mode != 1) return;
+    if (P.info[seg_rel].mode != 1) return;
+    // per-segment constants of the acceptance step and the epilogue live in shared memory, not in registers: the
+    // register peak is the draw loop, and everything kept live across it costs resident warps
+    __shared__ SegInfo s_si;
+    __shared__ double s_inv_n;
+    __shared__ long long s_seg_rel;
+    __shared__ int s_r;
+    __shared__ int s_next;
+    __shared__ double2 s_log[128];
     const long long seg = P.seg_lo + seg_rel;
     const int r = (int)(seg % P.R);
     const int U = P.seg_U[seg_rel];
     const BootEntry* tab = P.entries + (P.seg_ptr[seg] - P.seg_ptr[P.seg_lo]);
-    const int N = P.group_ncells[r];
     const long long sid = P.gene_id ? P.gene_id[seg_rel / P.R] * P.R + r : seg;
-    const uint32_t* acc = P.acc_pool + si.acc_off;
-    const double* fit = P.mv_fit + 3 * r;
     const int b_end = min(P.B, (int)(blockIdx.x + 1) * P.reps_per_block);
-    __shared__ int s_next;
-    __shared__ double2 s_log[128];
     static_assert(kBootThreads >= 128, "one log-table entry per thread");
     if (threadIdx.x < 128) log_tab_fill(s_log, threadIdx.x);
-    if (threadIdx.x == 0) s_next = blockIdx.x * P.reps_per_block + kBootSlots * kBootThreads;
+    if (threadIdx.x == 0) {
+        s_si = P.info[seg_rel];
+        s_inv_n = 1.0 / (double)P.group_ncells[r];
+        s_seg_rel = seg_rel;
+        s_r = r;
+        s_next = blockIdx.x * P.reps_per_block + kBootSlots * kBootThreads;
+    }
     __syncthreads();
-    const double inv_n = 1.0 / (double)N;
     // Philox counter = (replicate, segment lo, block number, segment hi ^ tag); the block number runs on over the
     // attempts of one replicate and restarts with a new replicate
     const uint32_t key0 = (uint32_t)P.seed, key1 = (uint32_t)(P.seed >> 32);
@@ -519,17 +526,20 @@ bootstrap_1d_poisson_kernel(BootParams P) {
         };
         int u = 0;
         for (; u + 4 <= U; u += 4) {        // four categories per Philox block
-            int4 lo4[4], hi4[4];
+            uint4 r4[kBootSlots];
 #pragma unroll
-            for (int c = 0; c < 4; ++c) {
-                lo4[c] = __ldg(reinterpret_cast<const int4*>(tab + u + c));
-                hi4[c] = __ldg(reinterpret_cast<const int4*>(tab + u + c) + 1);
-            }
+            for (int j = 0; j < kBootSlots; ++j) r4[j] = fresh4(j);
 #pragma unroll
-            for (int j = 0; j < kBootSlots; ++j) {
-                const uint4 r4 = fresh4(j);
-                draw(j, lo4[0], hi4[0], r4.x); draw(j, lo4[1], hi4[1], r4.y);
-                draw(j, lo4[2], hi4[2], r4.z); draw(j, lo4[3], hi4[3], r4.w);
+            for (int c = 0; c < 4; c += 2) {    // two category records at a time: 14 registers instead of 28
+                const int4 lo0 = __ldg(reinterpret_cast<const int4*>(tab + u + c));
+                const int4 hi0 = __ldg(reinterpret_cast<const int4*>(tab + u + c) + 1);
+                const int4 lo1 = __ldg(reinterpret_cast<const int4*>(tab + u + c + 1));
+                const int4 hi1 = __ldg(reinterpret_cast<const int4*>(tab + u + c + 1) + 1);
+#pragma unroll
+                for (int j = 0; j < kBootSlots; ++j) {
+                    draw(j, lo0, hi0, c == 0 ? r4[j].x : r4[j].z);
+                    draw(j, lo1, hi1, c == 0 ? r4[j].y : r4[j].w);
+                }
             }
         }
         uint4 r4[kBootSlots];
@@ -550,22 +560,27 @@ bootstrap_1d_poisson_kernel(BootParams P) {
 #pragma unroll
             for (int j = 0; j < kBootSlots; ++j) draw(j, lo4, hi4, r4[j].z);
         }
-        if (si.zero_off >= 0) {
+        const int zero_off = s_si.zero_off;
+        if (zero_off >= 0) {
+            const int zero_kl = s_si.zero_kl;
 #pragma unroll
             for (int j = 0; j < kBootSlots; ++j)
-                S[j] += alias_draw(P.tab_pool, (unsigned)si.zero_off, (unsigned)(si.zero_kl & 0xFFFF),
-                                   (si.zero_kl >> 16) - si.zero_off, r4[j].w);
+                S[j] += alias_draw(P.tab_pool, (unsigned)zero_off, (unsigned)(zero_kl & 0xFFFF),
+                                   (zero_kl >> 16) - zero_off, r4[j].w);
         }
 #pragma unroll
         for (int j = 0; j < kBootSlots; ++j) {
             const uint4 ra = fresh4(j);
-            const int i = S[j] - si.s_lo;
-            bool ok = (i >= 0) && (i < si.acc_len) && (b[j] < b_end);
-            if (ok) ok = ra.x < __ldg(acc + i);
+            const int i = S[j] - s_si.s_lo;
+            bool ok = (i >= 0) && (i < s_si.acc_len) && (b[j] < b_end);
+            if (ok) ok = ra.x < __ldg(P.acc_pool + s_si.acc_off + i);
             if (ok) {
+                const long long sr = s_seg_rel;
+                const int rr = s_r;
+                const int N = P.group_ncells[rr];
                 const double w = (double)(N - S[j]);            // the remainder category takes the rest
-                const double m1 = fma(si.rem_a, w, M1[j]), m2 = fma(si.rem_b, w, M2[j]);
-                emit_replicate(P, seg_rel, b[j], m1, m2, N, inv_n, fit, s_log);
+                const double m1 = fma(s_si.rem_a, w, M1[j]), m2 = fma(s_si.rem_b, w, M2[j]);
+                emit_replicate(P, sr, b[j], m1, m2, N, s_inv_n, P.mv_fit + 3 * rr, s_log);
                 b[j] = atomicAdd(&s_next, 1);                // results depend on (seed, replicate) only, not on the lane
                 blk[j] = 0;
             }
