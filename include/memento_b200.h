@@ -387,6 +387,17 @@ int mm_pair_bootstrap_replay(int device, void* stream, const double* x, const do
                              const int32_t* n_cells, const double* q, int32_t n_tab, int32_t num_boot,
                              double* out_cov, double* out_var1, double* out_var2, double* out_corr);
 
+/* Negative-binomial quantiles of normal draws, the count step of the Gaussian-copula transcriptome generator
+ * (csrc/simulate.cu): z is a row-major (n_rows, n_genes) float64 chunk; out[i * n_genes + j] = the smallest k >= 0
+ * with F_j(k) >= Phi(z) in float64, F_j the cdf of scipy's nbinom(r[j], p[j]) (r > 0, 0 < p <= 1).  Where Phi(z)
+ * rounds to 1 (z > 8.29; the reference returns inf there) the count is the finite upper-tail quantile
+ * nbinom.isf(norm.sf(z)).  An element whose bounded search fails is written as -1 and added to *n_failed (device
+ * int32, zero-initialised by the caller; it accumulates over calls).
+ * Replaces: memento/simulate.py:69-88 (stats.norm.cdf + stats.nbinom.ppf on the draws of
+ * stats.multivariate_normal.rvs). */
+int mm_nb_quantile(int device, void* stream, const double* z, int64_t n_rows, int32_t n_genes, const double* r,
+                   const double* p, int64_t* out, int32_t* n_failed);
+
 #ifdef __cplusplus
 }
 #endif

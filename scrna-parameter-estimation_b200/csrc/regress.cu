@@ -383,6 +383,8 @@ regress_asl_kernel(RegParams P) {
             P.out_coef[obase + i] = nan(""); P.out_se[obase + i] = nan(""); P.out_asl[obase + i] = nan("");
             P.out_extreme[obase + i] = -1; P.out_nnull[obase + i] = 0;
         }
+        if (P.coef_ws && blockIdx.y == 0)   // the gene's coefficient rows are NaN too, not left unwritten
+            for (long long i = tid; i < (long long)NS * T * B1; i += kRegThreads) P.coef_ws[obase * B1 + i] = nan("");
         return;
     }
 

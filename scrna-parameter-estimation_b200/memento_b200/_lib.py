@@ -52,6 +52,7 @@ SIGNATURES = {
     "mm_gev_tail_asl": [_vp, _vp, _i32, _i32, _vp, _vp, _vp, _i32],
     "mm_regress_asl": [_vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp,
                        _vp],
+    "mm_nb_quantile": [_vp, _i64, _i32, _vp, _vp, _vp, _vp],
 }
 
 # host-only helpers (no leading device / stream arguments)

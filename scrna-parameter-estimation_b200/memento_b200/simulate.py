@@ -8,7 +8,11 @@ Poisson(q * count).  The reference does the hypergeometric draw in a Python loop
 sampler, which cannot produce a 1 M-cell data set; here every molecule gets a uniform random key and the
 ``n_sample`` smallest keys of a cell are the captured molecules -- the same distribution, as a sort, a k-th value and a
 segmented count in torch (any device; the bench uses the GPU).  This is data generation, not the hot path: plain
-torch, no hand-written kernels.  The copula form (a covariance matrix as ``norm_cov``) is not provided.
+torch, no hand-written kernels, except for the Gaussian-copula form of ``simulate_transcriptomes`` (a covariance matrix
+as ``norm_cov``, :69-88), which needs a CUDA device: the matrix is factored once (``copula_factor``), every chunk of
+cells draws ``E @ F^T`` in float64 with cuBLAS and the library's ``mm_nb_quantile`` turns the normal draws into NB
+counts (scipy's ``nbinom.ppf(norm.cdf(z))``, for which torch has no counterpart).  The dense copula costs O(n G^2) in
+that product.
 """
 import numpy as np
 import torch
@@ -33,13 +37,81 @@ def _gen(device, seed):
     return g
 
 
+def copula_factor(norm_cov, device=None):
+    """``F`` (G, G) float64 on ``device`` with ``F F^T = norm_cov``, from ``torch.linalg.eigh``: ``V diag(sqrt(lam))``
+    over the eigenvalues above scipy's cut-off ``1e6 * eps * max|lam|`` (``stats.multivariate_normal`` drops the same
+    ones, so a rank-deficient matrix is factored as there).  Raises ValueError when the matrix is not positive
+    semidefinite by scipy's rule, ``min lam >= -cut-off``."""
+    m = torch.as_tensor(np.asarray(norm_cov, dtype=np.float64), device=device)
+    lam, vec = torch.linalg.eigh(m)
+    cut = 1e6 * np.finfo(np.float64).eps * float(lam.abs().max()) if lam.numel() else 0.0
+    if lam.numel() and float(lam.min()) < -cut:
+        raise ValueError("norm_cov must be positive semidefinite (smallest eigenvalue %.3g)" % float(lam.min()))
+    return vec * torch.where(lam > cut, lam, torch.zeros_like(lam)).sqrt()[None, :]
+
+
+def _nb_params(means, variances):
+    """(r, p) of scipy's nbinom for the per-gene means / variances, the dispersion floored as simulate.py:60-61."""
+    means = np.asarray(means, dtype=np.float64)
+    with np.errstate(divide="ignore", invalid="ignore"):
+        disp = (np.asarray(variances, dtype=np.float64) - means) / means ** 2
+        disp[disp < 0] = 1e-5
+        return convert_params_nb(means, 1.0 / disp)
+
+
+def _copula_transcriptomes(n_cells, means, variances, norm_cov, dev, seed, chunk):
+    """reference simulate.py:69-88 with one draw of N(0, norm_cov) per cell (the matrix used as given)."""
+    means, variances = np.asarray(means, dtype=np.float64), np.asarray(variances, dtype=np.float64)
+    G = means.shape[0]
+    if means.ndim != 1 or variances.shape != means.shape:
+        raise ValueError("means and variances must be vectors of the same length")
+    cov = np.asarray(norm_cov, dtype=np.float64)
+    if cov.shape != (G, G):
+        raise ValueError("norm_cov must be a (%d, %d) matrix, got shape %s" % (G, G, cov.shape))
+    if not np.isfinite(cov).all():
+        raise ValueError("norm_cov must be finite")
+    if np.abs(cov - cov.T).max(initial=0.0) > 1e-10 * np.abs(cov).max(initial=0.0):
+        raise ValueError("norm_cov must be symmetric")
+    r, p = _nb_params(means, variances)
+    if not (np.isfinite(r).all() and np.isfinite(p).all() and (r > 0).all() and (p > 0).all() and (p <= 1).all()):
+        raise ValueError("every gene needs finite NB parameters r > 0, 0 < p <= 1 (means > 0, variances finite)")
+    # the positive-semidefinite check uses the eigenvalues of the factorisation itself: one O(G^3) pass, no draw yet
+    factor = copula_factor(cov, dev)
+    if dev.type != "cuda":
+        raise NotImplementedError("the Gaussian-copula form of simulate_transcriptomes needs a CUDA device (its NB "
+                                  "quantile step is a kernel of the library); got device %s" % dev)
+    if dev.index is None:
+        dev = torch.device("cuda", torch.cuda.current_device())
+    from . import _lib
+    g = _gen(dev, seed)
+    r_d = torch.as_tensor(r, dtype=torch.float64, device=dev)
+    p_d = torch.as_tensor(p, dtype=torch.float64, device=dev)
+    out = torch.empty((n_cells, G), dtype=torch.int64, device=dev)
+    n_failed = torch.zeros(1, dtype=torch.int32, device=dev)
+    for lo in range(0, n_cells, chunk):
+        hi = min(n_cells, lo + chunk)
+        z = torch.randn((hi - lo, G), generator=g, dtype=torch.float64, device=dev) @ factor.T
+        _lib.call("mm_nb_quantile", dev, z, hi - lo, G, r_d, p_d, out[lo:hi], n_failed)
+    if int(n_failed.item()):
+        raise RuntimeError("mm_nb_quantile: the quantile search failed for %d elements" % int(n_failed.item()))
+    return out
+
+
 def simulate_transcriptomes(n_cells, means, variances, Nc=None, norm_cov="indep", device=None, seed=0, chunk=8192):
     """(n_cells, n_genes) int64 transcript counts, NB with the given per-gene means / variances (dispersions
-    ``(v - m) / m^2``, floored at 1e-5 as the reference does).  reference simulate.py:52-67.  ``Nc`` is unused in this
-    form there too.  Returns a torch tensor on ``device``."""
-    if not isinstance(norm_cov, str):
-        raise NotImplementedError("the Gaussian-copula form (simulate.py:69-88) is not provided on the device")
+    ``(v - m) / m^2``, floored at 1e-5 as the reference does).  reference simulate.py:52-88.  ``Nc`` is unused, as
+    there.  Returns a torch tensor on ``device``.
+
+    ``norm_cov`` a string: independent genes (:52-67), on any device.  ``norm_cov`` a (G, G) matrix: the Gaussian
+    copula (:69-88), on a CUDA device only: every cell draws ``z ~ N(0, norm_cov)`` (the matrix used as given, not
+    rescaled to a correlation matrix) and gene j's count is ``nbinom.ppf(norm.cdf(z_j), r_j, p_j)``.  Where
+    ``norm.cdf(z_j)`` rounds to 1 (z_j > 8.29) the reference returns inf; here the count is the finite
+    ``nbinom.isf(norm.sf(z_j))``.  The matrix must be symmetric and positive semidefinite (scipy's rule; rank-deficient
+    is fine) and every gene's (r, p) valid, else ValueError before anything is drawn.  The same seed gives the same
+    counts; different ``chunk`` sizes draw differently.  The cost is O(n_cells G^2) in the float64 product."""
     dev = torch.device(device) if device is not None else torch.device("cpu")
+    if not isinstance(norm_cov, str):
+        return _copula_transcriptomes(n_cells, means, variances, norm_cov, dev, seed, chunk)
     means = np.asarray(means, dtype=np.float64)
     disp = (np.asarray(variances, dtype=np.float64) - means) / means ** 2
     disp[disp < 0] = 1e-5
