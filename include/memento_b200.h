@@ -132,7 +132,14 @@ int mm_block_panels(int device, void* stream, const float* vals, const int32_t* 
  *                           a NaN correlation in some group is dropped for that pair.  Running sums of d = coef - stat:
  *                           sum, sumsq, n_ext (|d| > |stat|), n_ok.  coef_out (nullable): this replicate's coefficients.
  *   mm_block_boot_finish  : se = std of d (ddof 0); asl = two-sided normal tail (approx != 0, hypothesis_test.py:77-83)
- *                           or (n_ext + 1) / (n_ok + 1) (:85-92, without the GEV refinement).
+ *                           or the counting estimate (n_ext + 1) / (n_ok + 1) (:85-92).  The GEV refinement of :94-141
+ *                           for pairs with n_ext <= 10 is a second pass that replays their replicates:
+ *   mm_block_boot_rows    : for one replicate (0 <= replicate < num_boot) and the sub-block cross [R][na][ld_cross]
+ *                           with its shift_* / isd_* that holds the candidate pairs (cand_a / cand_b [n_cand]:
+ *                           positions inside the sub-block), rows[i * (num_boot + 1) + 1 + replicate] = candidate i's
+ *                           coefficient, computed as in mm_block_boot_update (the same bits), NaN where that update
+ *                           drops the replicate.  The caller puts the observed coefficient in column 0: the layout
+ *                           mm_gev_tail_asl reads.
  * Replaces: memento/bootstrap.py:119-157 + hypothesis_test.py:303-414 for gene_pairs = A x B. */
 int mm_cell_weights(int device, void* stream, const int64_t* group_start, int32_t R, int64_t n_cells, uint64_t seed,
                     uint32_t replicate, int32_t* w);
@@ -147,6 +154,10 @@ int mm_block_boot_update(int device, void* stream, const double* cross, const do
 int mm_block_boot_finish(int device, void* stream, const double* stat, const double* sum, const double* sumsq,
                          const int32_t* n_ext, const int32_t* n_ok, int64_t n_pairs, int32_t approx, double* se,
                          double* asl);
+int mm_block_boot_rows(int device, void* stream, const double* cross, const double* shift_a, const double* isd_a,
+                       const double* shift_b, const double* isd_b, const double* group_n, const double* cfun,
+                       int32_t R, int32_t na, int32_t nb, int64_t ld_cross, const int32_t* cand_a,
+                       const int32_t* cand_b, int32_t n_cand, int32_t replicate, int32_t num_boot, double* rows);
 
 /* Dense gene block, step 2: out[a * ldo + b] = scale_a[a] * scale_b[b] * sum_k z_a[k] z_b[k] for a < m, b < n, with
  * z = z_hi + 2^-11 z_lo, as three fp16 tcgen05.mma products (hi hi, hi lo, lo hi) accumulated in fp32 in tensor

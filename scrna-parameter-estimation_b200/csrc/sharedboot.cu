@@ -13,6 +13,8 @@
 //   mm_block_boot_update   per pair: correlation per group -> regression coefficient across groups -> running sums
 //                          of (coef - stat), its square and the extreme count (hypothesis_test.py:367-414, :57-92)
 //   mm_block_boot_finish   SE and ASL per pair from the running sums
+//   mm_block_boot_rows     one replicate's coefficients of listed candidate pairs, written into their null rows (the
+//                          replay pass that gives those pairs the GEV tail ASL of hypothesis_test.py:94-141)
 #include "common.cuh"
 
 namespace mm {
@@ -70,6 +72,28 @@ seg_weighted_stats_kernel(const float* __restrict__ vals, const int* __restrict_
     }
 }
 
+// The replicate's regression coefficient of pair (a, b) of a block: per group the correlation from the weighted cross
+// product and the weighted shifts / inverse deviations ([na][R] and [nb][R]), clipped to [-1, 1] (estimator.py:289-290),
+// folded with the functional cfun.  ok = false when some group's correlation is NaN: the replicate is dropped for the
+// pair.  The running-sum update and the replay of candidate rows both call this, so their coefficients are the same bits.
+__device__ __forceinline__ double replicate_coef(const double* __restrict__ cross, long long ld, int na,
+                                                 const double* __restrict__ shift_a, const double* __restrict__ isd_a,
+                                                 const double* __restrict__ shift_b, const double* __restrict__ isd_b,
+                                                 const double* __restrict__ group_n, const double* __restrict__ cfun,
+                                                 int R, int a, int b, bool& ok) {
+    double coef = 0.0;
+    ok = true;
+    for (int r = 0; r < R; ++r) {
+        const double n = group_n[r];
+        const double cov = cross[((long long)r * na + a) * ld + b] / n - shift_a[(long long)a * R + r] * shift_b[(long long)b * R + r];
+        double corr = cov * isd_a[(long long)a * R + r] * isd_b[(long long)b * R + r];
+        ok = ok && (corr == corr);
+        corr = fmin(1.0, fmax(-1.0, corr));                  // estimator.py:289-290
+        coef = fma(cfun[r], corr, coef);
+    }
+    return coef;
+}
+
 struct BootUpdate {
     const double* cross;        // [R][na][ld] weighted centred cross products of the replicate (ld >= nb: padded rows)
     long long ld;
@@ -92,16 +116,9 @@ block_boot_update_kernel(BootUpdate P) {
     const int a = (int)(k / P.nb), b = (int)(k % P.nb);
     const double stat = P.stat[k];
     if (!(stat == stat)) { if (P.coef_out) P.coef_out[k] = nan(""); return; }
-    double coef = 0.0;
-    bool ok = true;
-    for (int r = 0; r < P.R; ++r) {
-        const double n = P.group_n[r];
-        const double cov = P.cross[((long long)r * P.na + a) * P.ld + b] / n - P.shift_a[(long long)a * P.R + r] * P.shift_b[(long long)b * P.R + r];
-        double corr = cov * P.isd_a[(long long)a * P.R + r] * P.isd_b[(long long)b * P.R + r];
-        ok = ok && (corr == corr);
-        corr = fmin(1.0, fmax(-1.0, corr));                  // estimator.py:289-290
-        coef = fma(P.cfun[r], corr, coef);
-    }
+    bool ok;
+    const double coef = replicate_coef(P.cross, P.ld, P.na, P.shift_a, P.isd_a, P.shift_b, P.isd_b, P.group_n, P.cfun,
+                                       P.R, a, b, ok);
     if (P.coef_out) P.coef_out[k] = ok ? coef : nan("");
     if (!ok) return;                                         // a replicate without a valid correlation in some group is dropped
     const double d = coef - stat;
@@ -109,6 +126,31 @@ block_boot_update_kernel(BootUpdate P) {
     P.sumsq[k] = fma(d, d, P.sumsq[k]);
     P.n_ext[k] += fabs(d) > fabs(stat) ? 1 : 0;
     P.n_ok[k] += 1;
+}
+
+struct BootRows {
+    const double* cross;        // [R][na][ld] as in BootUpdate, for the sub-block that holds the candidates
+    long long ld;
+    const double* shift_a; const double* isd_a;     // [na][R]
+    const double* shift_b; const double* isd_b;     // [nb][R]
+    const double* group_n; const double* cfun;      // [R]
+    int R, na;
+    const int* cand_a; const int* cand_b;           // [n_cand] positions inside the sub-block
+    int n_cand, col;            // col = 1 + replicate
+    long long ld_rows;          // num_boot + 1
+    double* rows;               // [n_cand][num_boot + 1]
+};
+
+// One thread per candidate; the writes stride by a whole row, but there is one per candidate and replicate against
+// R reads of the cross block, so they are a small part of the traffic.
+__global__ void __launch_bounds__(256)
+block_boot_rows_kernel(BootRows P) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= P.n_cand) return;
+    bool ok;
+    const double coef = replicate_coef(P.cross, P.ld, P.na, P.shift_a, P.isd_a, P.shift_b, P.isd_b, P.group_n, P.cfun,
+                                       P.R, P.cand_a[i], P.cand_b[i], ok);
+    P.rows[(long long)i * P.ld_rows + P.col] = ok ? coef : nan("");
 }
 
 __global__ void block_boot_finish_kernel(const double* __restrict__ stat, const double* __restrict__ sum,
@@ -129,7 +171,7 @@ __global__ void block_boot_finish_kernel(const double* __restrict__ stat, const 
     if (approx) {           // hypothesis_test.py:77-83: normal fit of the null (coef - stat), two-sided tail of |stat|
         const double k2 = 1.0 / (sd * 1.4142135623730951), as = fabs(st);
         asl[k] = 0.5 * erfc((as - mu) * k2) + 0.5 * erfc((as + mu) * k2);
-    } else {                // :85-92 without the GEV refinement of the far tail
+    } else {                // :85-92; the GEV refinement of the far tail is a second pass (mm_block_boot_rows)
         asl[k] = (double)(n_ext[k] + 1) / (double)(n + 1);
     }
 }
@@ -194,4 +236,24 @@ MM_EXPORT int mm_block_boot_finish(int device, void* stream, const double* stat,
     block_boot_finish_kernel<<<(unsigned)((n_pairs + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
         stat, sum, sumsq, n_ext, n_ok, n_pairs, approx, se, asl);
     return check_launch("mm_block_boot_finish");
+}
+
+MM_EXPORT int mm_block_boot_rows(int device, void* stream, const double* cross, const double* shift_a,
+                                 const double* isd_a, const double* shift_b, const double* isd_b,
+                                 const double* group_n, const double* cfun, int32_t R, int32_t na, int32_t nb,
+                                 int64_t ld_cross, const int32_t* cand_a, const int32_t* cand_b, int32_t n_cand,
+                                 int32_t replicate, int32_t num_boot, double* rows) {
+    if (int s = enter(device)) return s;
+    MM_REQUIRE(R > 0 && na >= 0 && nb >= 0 && ld_cross >= nb && n_cand >= 0, "R/na/nb/ld_cross/n_cand");
+    MM_REQUIRE(num_boot > 0 && replicate >= 0 && replicate < num_boot, "replicate/num_boot");
+    if (n_cand == 0) return 0;
+    MM_REQUIRE(na > 0 && nb > 0, "candidates in an empty block");
+    MM_REQUIRE(cross && shift_a && isd_a && shift_b && isd_b && group_n && cfun && cand_a && cand_b && rows,
+               "null pointer");
+    BootRows P;
+    P.cross = cross; P.ld = ld_cross; P.shift_a = shift_a; P.isd_a = isd_a; P.shift_b = shift_b; P.isd_b = isd_b;
+    P.group_n = group_n; P.cfun = cfun; P.R = R; P.na = na; P.cand_a = cand_a; P.cand_b = cand_b; P.n_cand = n_cand;
+    P.col = 1 + replicate; P.ld_rows = (long long)num_boot + 1; P.rows = rows;
+    block_boot_rows_kernel<<<(unsigned)((n_cand + 255) / 256), 256, 0, (cudaStream_t)stream>>>(P);
+    return check_launch("mm_block_boot_rows");
 }

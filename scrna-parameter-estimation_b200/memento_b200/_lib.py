@@ -28,6 +28,7 @@ SIGNATURES = {
     "mm_seg_weighted_stats": [_vp, _vp, _vp, _i32, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     "mm_block_boot_update": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _i64],
     "mm_block_boot_finish": [_vp, _vp, _vp, _vp, _vp, _i64, _i32, _vp, _vp],
+    "mm_block_boot_rows": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i64, _vp, _vp, _i32, _i32, _i32, _vp],
     "mm_block_gemm": [_vp, _vp, _i32, _vp, _vp, _i32, _i32, _vp, _vp, _vp, _i64],
     "mm_block_scaling": [_vp, _i32, _i32, _vp, _vp, _i32, _vp, _i32, _vp, _vp, _vp],
     "mm_block_cross_batch": [_vp, _vp, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp,

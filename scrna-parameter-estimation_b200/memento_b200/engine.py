@@ -7,7 +7,7 @@ group-validity mask (a (tile_genes x R) byte matrix) so that the small solves ar
 import numpy as np
 import torch
 
-from . import _lib
+from . import _lib, gev
 from .device import ENTRY_BYTES, NULL_TIMER
 
 
@@ -536,8 +536,31 @@ def ht_2d_tile(seg, design, cell_bin, idx1, idx2, true_corr, covariate, treatmen
 
 
 # --------------------------------------------------------------------------- shared-weight bootstrap of a dense block
+def plan_tail_chunks(flat, nb, num_boot, budget_bytes):
+    """Chunks of the GEV replay pass of :func:`ht_2d_shared_block`.  ``flat``: ascending flat indices a * nb + b of the
+    candidate pairs in the (na, nb) block (an int64 tensor on any device).  The list is cut into contiguous runs whose
+    null rows (n * (num_boot + 1) float64) fit ``budget_bytes``; a run may start or end inside a row of A.  Because the
+    runs follow the rows, the sub-blocks replayed over all chunks add up to at most one pass over the A rows and B
+    columns that hold candidates.  Returns one dict per run: "lo" / "hi" (the run is flat[lo:hi]), "genes_a" /
+    "genes_b" (the sorted distinct A and B positions of its pairs, int64) and "ia" / "ib" (int32: every pair's
+    position in those lists, so that genes_a[ia] * nb + genes_b[ib] == flat[lo:hi])."""
+    row_bytes = 8 * (num_boot + 1)
+    per = int(budget_bytes) // row_bytes
+    if per < 1:
+        raise ValueError("workspace_bytes = %d holds no null row of %d bytes" % (budget_bytes, row_bytes))
+    chunks = []
+    for lo in range(0, int(flat.numel()), per):
+        f = flat[lo:lo + per]
+        genes_a, ia = torch.unique(torch.div(f, nb, rounding_mode="floor"), sorted=True, return_inverse=True)
+        genes_b, ib = torch.unique(f % nb, sorted=True, return_inverse=True)
+        chunks.append({"lo": lo, "hi": lo + int(f.numel()), "genes_a": genes_a, "genes_b": genes_b,
+                       "ia": ia.to(torch.int32), "ib": ib.to(torch.int32)})
+    return chunks
+
+
 def ht_2d_shared_block(seg, idx_a, idx_b, inv_sf, sums_d, group_q, true_corr, covariate, treatment, num_boot, seed,
-                       approx, one_sample, timer=NULL_TIMER, weights=None, want_coef=False):
+                       approx, one_sample, timer=NULL_TIMER, weights=None, want_coef=False, tail="count",
+                       max_extreme=gev.MAX_EXTREME, workspace_bytes=4 << 30, stats=None, want_rows=False):
     """The "true" cell bootstrap of a dense gene-pair block A x B (csrc/sharedboot.cu; SURVEY.md 8f row 3): per
     replicate one set of per-cell resampling counts shared by all pairs, one weighted tensor-core GEMM per group.
 
@@ -545,8 +568,17 @@ def ht_2d_shared_block(seg, idx_a, idx_b, inv_sf, sums_d, group_q, true_corr, co
     ``true_corr``: (|A|, |B|, R) host array or device tensor (any shape with that many values) of the observed correlations; pairs with a NaN or +-1 correlation in some
     group (reference hypothesis_test.py:325 drops such groups per pair) and i == j pairs are left NaN for the caller's
     per-pair path.  ``weights`` (tests): (num_boot, n_cells) int32 device tensor of resampling counts instead of the
-    Philox draws.  Returns {"coef", "se", "asl"} float64 device tensors (|A|, |B|), "n_ok" and, with ``want_coef``,
-    the last replicate's coefficients."""
+    Philox draws.  Returns {"coef", "se", "asl"} float64 device tensors (|A|, |B|), "n_ext", "n_ok" and, with
+    ``want_coef``, the last replicate's coefficients.
+
+    ``tail="gev"`` (needs ``approx=False``): the pairs whose counting ASL rests on at most ``max_extreme`` extreme
+    replicates get the GEV tail ASL of the reference (hypothesis_test.py:94-141).  Every replicate is a deterministic
+    function of (seed, replicate), so a second pass replays the replicates on the sub-blocks that hold those pairs
+    (chunks of :func:`plan_tail_chunks`, null rows within ``workspace_bytes``), writes their null rows
+    (mm_block_boot_rows) and fits the tails (mm_gev_tail_asl).  ``stats`` (dict) receives "tail_candidates",
+    "tail_chunks", "tail_replayed_pairs" (the pairs of the replayed sub-blocks) and the GEV status vectors for
+    gev.count_tail_tests.  ``want_rows`` (tests): also return the null rows
+    ("rows", (n, num_boot + 1), column 0 = the observed coefficient) and the candidates' flat indices ("tail_index")."""
     dev = seg.device
     R, gs = seg.R, seg.group_start_host
     n_r = np.diff(gs).astype(np.float64)
@@ -575,29 +607,60 @@ def ht_2d_shared_block(seg, idx_a, idx_b, inv_sf, sums_d, group_q, true_corr, co
         e = e.clamp(-200, 200)
         return m.contiguous(), torch.exp2(-e), torch.exp2(e)
 
-    ca, inv_a, sc_a = scaling(ia)                       # (na, R)
-    cb, inv_b, sc_b = scaling(ib)
     BK = seg.BLOCK_K
     k_pad = [max(BK, (int(n) + BK - 1) // BK * BK) for n in n_r]
-    # the plain B panels are the same for every replicate: built once per group and kept
-    panels_b = []
-    for r in range(R):
-        zb = torch.empty((2, nb, k_pad[r]), dtype=torch.float16, device=dev)
-        _lib.call("mm_block_panels", dev, seg.vals, seg.rows, seg.seg_ptr, R, r, int(gs[r]), int(n_r[r]), inv_sf, ib, nb,
-                  cb[:, r].contiguous(), inv_b[:, r].contiguous(), k_pad[r], zb[0], zb[1], None)
-        panels_b.append(zb)
-    # per-group rows for the batched panels + GEMM call: (R, na) / (R, nb), and the host-side group table
-    ca_g, inv_a_g, sc_a_g, sc_b_g = (t.t().contiguous() for t in (ca, inv_a, sc_a, sc_b))
     g_ids = np.arange(R, dtype=np.int32)
     g_row0 = np.ascontiguousarray(gs[:-1], dtype=np.int64)
     g_cells = np.ascontiguousarray(n_r, dtype=np.int32)
-    b_ptrs = np.asarray([p.data_ptr() for p in panels_b], dtype=np.uint64)
-    pa = torch.empty(2 * 2 * na * max(k_pad), dtype=torch.float16, device=dev)      # two buffers of (hi | lo) panels
-    ldc = (nb + 7) // 8 * 8                              # padded rows: aligned TMA tensor stores in the GEMM epilogue
-    cross = torch.empty((R, na, ldc), dtype=torch.float64, device=dev)
-    w = torch.empty(seg.n_cells, dtype=torch.int32, device=dev)
-    shift_a, isd_a = torch.empty((na, R), dtype=torch.float64, device=dev), torch.empty((na, R), dtype=torch.float64, device=dev)
-    shift_b, isd_b = torch.empty((nb, R), dtype=torch.float64, device=dev), torch.empty((nb, R), dtype=torch.float64, device=dev)
+
+    def gene_set(idx, c, inv, sc):
+        """A gene set of one side with its (n, R) centres and scales, their per-group rows (R, n) for the batched panels
+        + GEMM call, and the replicate's weighted shift / inverse deviation buffers."""
+        n = int(idx.numel())
+        return {"idx": idx, "n": n, "c": c.contiguous(), "inv": inv, "sc": sc,
+                "c_g": c.t().contiguous(), "inv_g": inv.t().contiguous(), "sc_g": sc.t().contiguous(),
+                "shift": torch.empty((n, R), dtype=torch.float64, device=dev),
+                "isd": torch.empty((n, R), dtype=torch.float64, device=dev)}
+
+    def b_panels(sb):          # the plain B panels are the same for every replicate: built once per group and kept
+        panels = []
+        for r in range(R):
+            zb = torch.empty((2, sb["n"], k_pad[r]), dtype=torch.float16, device=dev)
+            _lib.call("mm_block_panels", dev, seg.vals, seg.rows, seg.seg_ptr, R, r, int(gs[r]), int(n_r[r]), inv_sf,
+                      sb["idx"], sb["n"], sb["c"][:, r].contiguous(), sb["inv"][:, r].contiguous(), k_pad[r], zb[0],
+                      zb[1], None)
+            panels.append(zb)
+        return panels, np.asarray([p.data_ptr() for p in panels], dtype=np.uint64)
+
+    w_buf = torch.empty(seg.n_cells, dtype=torch.int32, device=dev)
+
+    def replicate(b, sa, sb, b_ptrs, pa, cross, ldc):
+        """Replicate b's cell counts, the weighted shifts / inverse deviations of both gene sets and the weighted cross
+        block of sa x sb: both passes make these launches with these arguments, so a pair's coefficient is the same
+        bits in either."""
+        if weights is None:
+            _lib.call("mm_cell_weights", dev, seg.group_start, R, seg.n_cells, seed, b, w_buf)
+            w = w_buf
+        else:
+            w = weights[b].contiguous()
+        for s in (sa, sb):
+            _lib.call("mm_seg_weighted_stats", dev, seg.vals, seg.rows, seg.seg_ptr, R, s["idx"], s["n"], inv_sf, w,
+                      s["c"], gn, gq, s["shift"], s["isd"])
+        # A panels with the counts folded in + one GEMM per group against the kept B panels, queued by one call
+        _lib.call("mm_block_cross_batch", dev, seg.vals, seg.rows, seg.seg_ptr, R, R, g_ids.ctypes.data,
+                  g_row0.ctypes.data, g_cells.ctypes.data, inv_sf, sa["idx"], sa["n"], sa["c_g"], sa["inv_g"],
+                  sa["sc_g"], None, sb["n"], None, None, sb["sc_g"], pa, None, max(k_pad), 2, b_ptrs.ctypes.data, w,
+                  cross, ldc, sa["n"] * ldc)
+
+    def block_buffers(n_a, n_b):
+        ldc = (n_b + 7) // 8 * 8                         # padded rows: aligned TMA tensor stores in the GEMM epilogue
+        pa = torch.empty(2 * 2 * n_a * max(k_pad), dtype=torch.float16, device=dev)   # two buffers of (hi | lo) panels
+        return pa, torch.empty((R, n_a, ldc), dtype=torch.float64, device=dev), ldc
+
+    A = gene_set(ia, *scaling(ia))
+    B = gene_set(ib, *scaling(ib))
+    panels_b, b_ptrs = b_panels(B)
+    pa, cross, ldc = block_buffers(na, nb)
     acc_sum = torch.zeros((na, nb), dtype=torch.float64, device=dev)
     acc_sq = torch.zeros((na, nb), dtype=torch.float64, device=dev)
     n_ext = torch.zeros((na, nb), dtype=torch.int32, device=dev)
@@ -605,22 +668,58 @@ def ht_2d_shared_block(seg, idx_a, idx_b, inv_sf, sums_d, group_q, true_corr, co
     coef_last = torch.empty((na, nb), dtype=torch.float64, device=dev) if want_coef else None
     ev = timer.start()
     for b in range(num_boot):
-        if weights is None:
-            _lib.call("mm_cell_weights", dev, seg.group_start, R, seg.n_cells, seed, b, w)
-        else:
-            w = weights[b].contiguous()
-        _lib.call("mm_seg_weighted_stats", dev, seg.vals, seg.rows, seg.seg_ptr, R, ia, na, inv_sf, w, ca, gn, gq,
-                  shift_a, isd_a)
-        _lib.call("mm_seg_weighted_stats", dev, seg.vals, seg.rows, seg.seg_ptr, R, ib, nb, inv_sf, w, cb, gn, gq,
-                  shift_b, isd_b)
-        # A panels with the counts folded in + one GEMM per group against the kept B panels, queued by one call
-        _lib.call("mm_block_cross_batch", dev, seg.vals, seg.rows, seg.seg_ptr, R, R, g_ids.ctypes.data, g_row0.ctypes.data,
-                  g_cells.ctypes.data, inv_sf, ia, na, ca_g, inv_a_g, sc_a_g, None, nb, None, None, sc_b_g, pa, None,
-                  max(k_pad), 2, b_ptrs.ctypes.data, w, cross, ldc, na * ldc)
-        _lib.call("mm_block_boot_update", dev, cross, shift_a, isd_a, shift_b, isd_b, gn, cfun, stat, R, na, nb,
-                  acc_sum, acc_sq, n_ext, n_ok, coef_last if (want_coef and b == num_boot - 1) else None, ldc)
+        replicate(b, A, B, b_ptrs, pa, cross, ldc)
+        _lib.call("mm_block_boot_update", dev, cross, A["shift"], A["isd"], B["shift"], B["isd"], gn, cfun, stat, R,
+                  na, nb, acc_sum, acc_sq, n_ext, n_ok, coef_last if (want_coef and b == num_boot - 1) else None, ldc)
     se = torch.empty((na, nb), dtype=torch.float64, device=dev)
     asl = torch.empty((na, nb), dtype=torch.float64, device=dev)
     _lib.call("mm_block_boot_finish", dev, stat, acc_sum, acc_sq, n_ext, n_ok, na * nb, 1 if approx else 0, se, asl)
     timer.stop("shared_block_bootstrap", ev)
-    return {"coef": stat, "se": se, "asl": asl, "n_ok": n_ok, "coef_last": coef_last, "usable": usable}
+    out = {"coef": stat, "se": se, "asl": asl, "n_ext": n_ext, "n_ok": n_ok, "coef_last": coef_last, "usable": usable}
+    if tail != "gev":
+        return out
+    assert not approx, "the GEV tail refines the counting ASL (approx=False)"
+    del pa, cross, panels_b, acc_sum, acc_sq
+    # ---- pass 2: replay the replicates for the pairs with few extreme replicates and fit their tails
+    stat_f, asl_f, ext_f = stat.view(-1), asl.view(-1), n_ext.view(-1)
+    cand = torch.isfinite(stat_f) & (ext_f >= 0) & (ext_f <= max_extreme) & torch.isfinite(asl_f)
+    flat = torch.nonzero(cand).squeeze(1)                # ascending = row-major; the one host read of this pass
+    chunks = plan_tail_chunks(flat, nb, num_boot, workspace_bytes) if flat.numel() else []
+    all_rows = []
+    for ch in chunks:
+        sel_a, sel_b = ch["genes_a"], ch["genes_b"]
+        # slices of pass 1's centres and scales: the chunk's panels are the same bits as pass 1's
+        A_c = gene_set(ia[sel_a], A["c"][sel_a], A["inv"][sel_a], A["sc"][sel_a])
+        B_c = gene_set(ib[sel_b], B["c"][sel_b], B["inv"][sel_b], B["sc"][sel_b])
+        f = flat[ch["lo"]:ch["hi"]]
+        n_c = int(f.numel())
+        rows = torch.empty((n_c, num_boot + 1), dtype=torch.float64, device=dev)
+        rows[:, 0] = stat_f[f]
+        panels_c, b_ptrs_c = b_panels(B_c)
+        pa_c, cross_c, ldc_c = block_buffers(A_c["n"], B_c["n"])
+        ev = timer.start()
+        for b in range(num_boot):
+            replicate(b, A_c, B_c, b_ptrs_c, pa_c, cross_c, ldc_c)
+            _lib.call("mm_block_boot_rows", dev, cross_c, A_c["shift"], A_c["isd"], B_c["shift"], B_c["isd"], gn, cfun,
+                      R, A_c["n"], B_c["n"], ldc_c, ch["ia"], ch["ib"], n_c, b, num_boot, rows)
+        timer.stop("shared_tail_replay", ev)
+        asl_c, ext_c = asl_f[f].contiguous(), ext_f[f].contiguous()
+        status = torch.empty(n_c, dtype=torch.int32, device=dev)
+        ev = timer.start()
+        _lib.call("mm_gev_tail_asl", dev, rows, None, n_c, num_boot, asl_c, status, ext_c, max_extreme)
+        timer.stop("gev_tail_asl", ev)
+        asl_f[f] = asl_c
+        if stats is not None:
+            stats.setdefault("_gev_status", []).append(status)
+            stats["tail_replayed_pairs"] = stats.get("tail_replayed_pairs", 0) + A_c["n"] * B_c["n"]
+        if want_rows:
+            all_rows.append(rows)
+        del panels_c, pa_c, cross_c
+    if stats is not None:
+        stats["tail_candidates"] = stats.get("tail_candidates", 0) + int(flat.numel())
+        stats["tail_chunks"] = stats.get("tail_chunks", 0) + len(chunks)
+    if want_rows:
+        out["rows"] = torch.cat(all_rows) if all_rows else torch.empty((0, num_boot + 1), dtype=torch.float64,
+                                                                        device=dev)
+        out["tail_index"] = flat
+    return out

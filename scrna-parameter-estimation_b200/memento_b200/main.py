@@ -998,7 +998,8 @@ def _corr_from_cov(cov, var_1, var_2):
 
 
 def ht_2d_moments(adata, covariate, treatment, treatment_for_gene=None, inplace=True, num_boot=10000,
-                  verbose=3, num_cpus=1, seed=0, workspace_bytes=4 << 30, bootstrap="pair", **kwargs):
+                  verbose=3, num_cpus=1, seed=0, workspace_bytes=4 << 30, bootstrap="pair", shared_tail="count",
+                  **kwargs):
     """Hypothesis test for the correlation of the gene pairs of ``compute_2d_moments``.
     reference: main.py:418-520.  One value per pair (the reference stores a (T,) array into a scalar
     slot, main.py:509, which only works for one treatment column), unordered duplicates share the
@@ -1007,9 +1008,13 @@ def ht_2d_moments(adata, covariate, treatment, treatment_for_gene=None, inplace=
     Build-only ``bootstrap``: ``"pair"`` (default) is the reference's per-pair compressed bootstrap
     (bootstrap.py:119-157); ``"shared"`` -- for ``gene_pairs`` that are a full block A x B -- is the cell bootstrap that
     scheme approximates, with ONE set of resampling counts per replicate shared by all pairs and one tensor-core GEMM
-    per group and replicate (csrc/sharedboot.cu); its ASL is the normal approximation (``approx=True``) or the
-    counting estimate (c + 1) / (n + 1) without the GEV refinement of the far tail.  Pairs with an unusable
-    correlation in some group fall back to the per-pair path."""
+    per group and replicate (csrc/sharedboot.cu); its ASL is the normal approximation (``approx=True``) or, with
+    ``approx=False``, chosen by the build-only ``shared_tail``: ``"count"`` (default) the counting estimate
+    (c + 1) / (n + 1), which cannot go below 1 / (num_boot + 1); ``"gev"`` the reference's approx=False ASL, where the
+    pairs with at most 10 extreme replicates get GEV tail fits (hypothesis_test.py:94-141) from a second pass that
+    replays their replicates (null rows within ``workspace_bytes`` at a time).  ``shared_tail="gev"`` needs
+    ``bootstrap="shared"`` and ``approx=False``.  Pairs with an unusable correlation in some group fall back to the
+    per-pair path, which refines its tail whenever ``approx=False``."""
     if not inplace:
         adata = adata.copy()
     resampling = kwargs.pop("resampling", "bootstrap")
@@ -1040,12 +1045,19 @@ def ht_2d_moments(adata, covariate, treatment, treatment_for_gene=None, inplace=
     n_all = idx1.shape[0]
     if bootstrap not in ("pair", "shared"):
         raise ValueError("bootstrap must be 'pair' or 'shared'")
+    if shared_tail not in ("count", "gev"):
+        raise ValueError("shared_tail must be 'count' or 'gev'")
+    if shared_tail == "gev" and bootstrap != "shared":
+        raise ValueError("shared_tail='gev' applies to bootstrap='shared' (the per-pair bootstrap always refines its tail "
+                         "when approx=False)")
+    if shared_tail == "gev" and approx:
+        raise ValueError("shared_tail='gev' refines the counting ASL: it needs approx=False")
     dist = st.dist or ONE_RANK
     me = dist.rank
     if st.dist is not None:
         _check_same_on_all_ranks(st, "ht_2d_moments", [
             idx1, idx2, cov, tr, list(covariate.columns), list(treatment.columns), list(covariate.index),
-            list(treatment.index), num_boot, seed, approx, resample_rep, bootstrap])
+            list(treatment.index), num_boot, seed, approx, resample_rep, bootstrap, shared_tail])
     dev = st.device
     gm = _gene_map(st, adata.var.index)
     # every rank tests the unique pairs whose second gene it holds; unordered de-duplication, first occurrence computes
@@ -1066,6 +1078,7 @@ def ht_2d_moments(adata, covariate, treatment, treatment_for_gene=None, inplace=
     q = [mem["group_q"][g] for g in groups]
     true_corr_d = _stacked_corr(mem, groups, dev)                                          # (n_all, R) on the device
     shared_done = None
+    stats_acc = {}
     if bootstrap == "shared":
         genes_a, genes_b, pos = block
         na, nb = genes_a.size, genes_b.size
@@ -1081,7 +1094,8 @@ def ht_2d_moments(adata, covariate, treatment, treatment_for_gene=None, inplace=
             tc_own = tc_blk.reshape(na, nb, R)[:, jb[me]:jb[me + 1], :].contiguous()
             sums_d = m["seg"].moments(st.inv_sf_sorted, st.timer)
             res = engine.ht_2d_shared_block(m["seg"], m["row"][genes_a], m["row"][own_b], st.inv_sf_sorted, sums_d,
-                                            q, tc_own, cov, tr, num_boot, seed, approx, one_sample, timer=st.timer)
+                                            q, tc_own, cov, tr, num_boot, seed, approx, one_sample, timer=st.timer,
+                                            tail=shared_tail, workspace_bytes=workspace_bytes, stats=stats_acc)
             part = [res["coef"], res["se"], res["asl"], res["usable"]]
         flat = [(t.cpu().numpy() if torch.is_tensor(t) else t).reshape(-1)[pos_blk]
                 for t in _gather_block(dist, part, jb, dev)]
@@ -1094,7 +1108,6 @@ def ht_2d_moments(adata, covariate, treatment, treatment_for_gene=None, inplace=
     res_mine = np.full((mine.size, 3), np.nan)
     per_item = 8 * (num_boot + 1) * (3 if not approx else 2)
     pairs_per_tile = int(max(1, min(65535 // R, workspace_bytes // (per_item * R))))
-    stats_acc = {}
     gid = gm["gid"]
     for lo in range(0, mine.size, pairs_per_tile):
         sel = mine[lo:lo + pairs_per_tile]
